@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload stage1_vaegan] [--batch GLOBAL_B]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
   python bench.py --impl reference ...     # the CPU arm: the oracle port of the reference step on the host cores
+  python bench.py ... --dump-outputs DIR   # also write the last timed step's outputs as DIR/<name>.npy (seeded inputs)
 
 One step = one full training iteration (forward, minimal backward, gradient all-reduce for N > 1, three RMSprop updates,
 bf16 operand repack) on one synthetic batch. `value` times K steps with inputs resident in HBM; `e2e` times K steps fed
@@ -88,7 +89,14 @@ def parse():
     ap.add_argument("--graph", action="store_true", help="replay the step from a CUDA graph (engine.GraphedStep; RMSprop "
                     "engines on one GPU): for launch-bound batch sizes such as configs[0]'s 64")
     ap.add_argument("--quick", action="store_true", help="device-resident timing only (for runs under ncu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (forward "
+                    "outputs, loss sums, updated parameters and BatchNorm buffers; rank 0) as DIR/<name>.npy, at most 64 MB")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.warmup < 0:
+        ap.error("--warmup must not be negative")
+    return a
 
 
 def peaks():
@@ -140,7 +148,7 @@ def stock_torch_leg(workload, B):
     try:
         r = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "stock_torch_gpu_baseline.py"), "--workload", workload,
                             "--batch", str(B), "--steps", "3", "--warmup", "2", "--modes", "bf16_cl"],
-                           capture_output=True, text=True, timeout=600)
+                           capture_output=True, text=True, timeout=600, env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
         line = json.loads([x for x in r.stdout.splitlines() if x.startswith("{")][-1])
         if "samples_per_s" not in line:
             return dict(error=line.get("error", "failed"))
@@ -277,12 +285,11 @@ def cpu_reference_steps(workload, B, steps, warmup, threads=None):
 
 
 def find_reference_models():
-    """Root of a reference tree that holds models/vae_gan.py: /root/reference (build container) or the git-ignored staging
-    copy baseline/_ref (what travels to a GPU box; __graft_entry__.build() makes it where /root/reference exists)."""
-    for root in (os.environ.get("FMRI_REFERENCE_ROOT"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if root and os.path.exists(os.path.join(root, "models", "vae_gan.py")) and \
-                os.path.exists(os.path.join(root, "configs", "models_config.py")):
-            return root
+    """Root of a checkout of the original project (named by $FMRI_REFERENCE_ROOT) that holds models/vae_gan.py, or None."""
+    root = os.environ.get("FMRI_REFERENCE_ROOT")
+    if root and os.path.exists(os.path.join(root, "models", "vae_gan.py")) and \
+            os.path.exists(os.path.join(root, "configs", "models_config.py")):
+        return root
     return None
 
 
@@ -363,7 +370,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warm = max(1, min(args.steps, 3)), max(1, min(args.warmup, 1))
+    steps, warm = args.steps, args.warmup
     B = args.cpu_batch
     v, ms, cores, kind, how = cpu_arm(args.workload, B, steps, warm)
     sample = f"{steps} timed + {warm} warm-up steps of batch {B} (bounded sample of the workload), fp32, torch CPU; {how}"
@@ -378,6 +385,29 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------ our arm
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor of `arrays` as <path>/<name>.npy: float64 and integer tensors as float64, all others as float32.
+    Every array gets an equal share of DUMP_BYTES; a larger one is replaced by a fixed sample of its flattened elements (the
+    positions depend only on the seed and the element count), so two builds run with the same arguments compare output for
+    output."""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096          # room for the .npy header
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()
+        cap = share // t.element_size()
+        if t.numel() > cap:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), cap, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     import torch
 
@@ -456,19 +486,22 @@ def run_ours(args):
         return (xb, a)
 
     def run_step(xb, a, b2, fb=None):
-        tr.step(*step_inputs(xb, a, b2, fb))
+        return tr.step(*step_inputs(xb, a, b2, fb))
 
     graphed = None
     if args.graph:
         if world > 1:
             raise SystemExit("--graph: one GPU")
         graphed = engine.GraphedStep(tr, *step_inputs(x, n1, n2, fmri))
+    last = {}
 
     def step_dev():
         if graphed is not None:
-            graphed(*step_inputs(x, n1, n2, fmri))
+            out = graphed(*step_inputs(x, n1, n2, fmri))
         else:
-            run_step(x, n1, n2)
+            out = run_step(x, n1, n2)
+        if args.dump_outputs:
+            last["out"] = out   # held only when dumping: the step's outputs are otherwise freed before the next step
 
     def sync_all():
         if world > 1:
@@ -501,6 +534,12 @@ def run_ours(args):
     losses = tr.losses()
     ms_step = ms_total / args.steps
     value = args.batch / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:   # before the e2e and profiling passes below step the trainer further
+        arrays = {k: v for k, v in last["out"].items() if isinstance(v, torch.Tensor)}
+        arrays["loss_sums"] = tr.sc
+        arrays.update(("param." + k, v) for k, v in tr.named_parameters().items())
+        arrays.update(("buffer." + k, v) for k, v in tr.named_buffers().items())
+        dump_outputs(args.dump_outputs, arrays)
 
     if args.quick:
         if rank == 0:
@@ -629,6 +668,7 @@ def run_ours(args):
 
 def main():
     global METRIC
+    sys.dont_write_bytecode = True   # the benchmark leaves the tree as build() left it: no __pycache__ of its imports
     args = parse()
     METRIC = f"{args.workload}_train_samples_per_sec_{args.resolution}x{args.resolution}"
     if args.impl == "reference":

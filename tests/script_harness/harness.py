@@ -1,15 +1,14 @@
 """Runs the reference's UNCHANGED train / inference scripts on top of this repository's models (SURVEY.md 8f-1).
 
     stubs/          stand-ins for the host-side packages this image lacks (matplotlib, skimage, nibabel, h5py)
-    make_tree()     fabricates the dataset tree of /root/reference/configs/data_config.py:5-45 (random JPEGs for the COCO
+    make_tree()     fabricates the dataset tree of the reference's configs/data_config.py:5-45 (random JPEGs for the COCO
                     folders and the BOLD5000 stimuli, random standardised 3620-voxel vectors in the pickles)
     run_script()    python <reference>/<script> ... in a child process with PYTHONPATH = stubs : this repo : reference, so
                     `models.vae_gan` and `configs.models_config` resolve HERE and everything else (configs.gan_config,
                     data_preprocessing, train.train_utils, the script itself) resolves in the untouched reference tree
 
-The reference tree is looked up at $FMRI_REFERENCE_ROOT, /root/reference, or <repo>/baseline/_ref (git-ignored staging copy
-made by __graft_entry__.build() where /root/reference exists; it is what travels to a GPU box, where /root/reference does
-not exist). Test infrastructure only.
+The reference tree is a checkout of the original project named by $FMRI_REFERENCE_ROOT; this repository does not hold its
+scripts, so without it the harness has nothing to run. Test infrastructure only.
 """
 from __future__ import annotations
 
@@ -30,9 +29,9 @@ NEEDED = ("train/train_vgan_stage1.py", "configs/gan_config.py", "data_preproces
 
 
 def find_reference():
-    for root in (os.environ.get("FMRI_REFERENCE_ROOT"), "/root/reference", os.path.join(REPO, "baseline", "_ref")):
-        if root and all(os.path.exists(os.path.join(root, f)) for f in NEEDED):
-            return root
+    root = os.environ.get("FMRI_REFERENCE_ROOT")
+    if root and all(os.path.exists(os.path.join(root, f)) for f in NEEDED):
+        return root
     return None
 
 

@@ -15,8 +15,8 @@ The VAE/GAN scripts interleave `loss.backward(retain_graph=True)` with `optimize
 which stock torch >= 1.5 rejects ON THE REFERENCE'S OWN MODULES (SURVEY.md 0-6); they run here because no Parameter is saved
 for backward.
 
-The reference tree cannot be committed and /root/reference does not exist on a GPU box: __graft_entry__.build() stages a
-git-ignored copy under baseline/_ref/ where /root/reference exists; without any copy these tests skip (and say so).
+The reference's scripts are not part of this repository: these tests run against a checkout of the original project named by
+$FMRI_REFERENCE_ROOT, and skip (and say so) without one.
 """
 import math
 import os
@@ -30,8 +30,8 @@ import harness as H  # noqa: E402
 pytestmark = pytest.mark.gpu
 
 REF = H.find_reference()
-needs_ref = pytest.mark.skipif(REF is None, reason="no reference tree on this machine (/root/reference or baseline/_ref): "
-                               "the unchanged-script harness needs the reference's scripts, which cannot be committed")
+needs_ref = pytest.mark.skipif(REF is None, reason="FMRI_REFERENCE_ROOT names no checkout of the original project: the "
+                               "unchanged-script harness needs the reference's scripts, which are not part of this repository")
 COMMON = ["-b", 8, "-e", 1, "-nw", 0, "-d", "cuda:0"]
 DRY = os.environ.get("FMRI_HARNESS_DRY") == "1"   # CPU dry run of the harness itself on the reference's own models (WAE chain)
 if DRY:

@@ -55,6 +55,33 @@ static inline int grid1d(long long n, int block, int cap = 148 * 16) {
     return (int)std::max<long long>(1, std::min<long long>(g, cap));
 }
 
+// ---- fixed-order reductions: where several CTAs contribute to one output element, each writes its partial into its own
+// slice of a stream-ordered scratch buffer and ordered_add() sums the slices in CTA order onto the output. Atomics made the
+// result depend on which CTA finished first: a last-bit difference that bf16 rounding and the optimizer grow step by step.
+static void* scratch_alloc(size_t bytes, cudaStream_t st) {
+    static bool pool_ready = false;
+    if (!pool_ready) {   // keep freed scratch in the pool: no re-mapping from step to step
+        int dev = 0;
+        cudaMemPool_t pool;
+        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess) {
+            uint64_t keep = UINT64_MAX;
+            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
+        }
+        pool_ready = true;
+    }
+    void* p = nullptr;
+    return cudaMallocAsync(&p, bytes, st) == cudaSuccess ? p : nullptr;
+}
+#define SCRATCH(ptr, type, count, st)                                                                        \
+    type* ptr = reinterpret_cast<type*>(scratch_alloc(sizeof(type) * (size_t)(count), st));                  \
+    if (!ptr) return fail(FMRI_ERR_CUDA, "scratch allocation of %zu bytes", sizeof(type) * (size_t)(count))
+template <typename T>
+static int ordered_add(const T* part, int nparts, long long n, T* dst, cudaStream_t st) {
+    ordered_add_kernel<T><<<grid1d(n, 256), 256, 0, st>>>(part, nparts, n, dst);
+    LAUNCH_OK();
+    return 0;
+}
+
 extern "C" int fmri_tensor_path_available(void) {
     int dev = 0, major = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) {
@@ -551,13 +578,9 @@ static int run_gemm_tn(const void* A, int lda, const void* B, int ldb, int M, in
     p.num_chunks = cdiv(K, KCH);
     p.n_total = N;
     p.n_tiles = N / BN;
-    // split-K: only for fp32 outputs without a nonlinear epilogue
-    int splits = 1;
-    const long long tiles = (long long)p.tiles_x * p.n_tiles;
-    if (c_fp32 && act == ACT_NONE && tiles < 148 && p.num_chunks >= 16) {
-        splits = (int)std::min<long long>(p.num_chunks / 8, std::max<long long>(1, (2 * 148) / tiles));
-        splits = std::max(1, splits);
-    }
+    // no split-K: with one writer per output element the result does not depend on CTA completion order (the linear
+    // layers are a small share of the step)
+    const int splits = 1;
     p.splits = splits;
     p.a_bytes = p.bw * KCH * 2;
     p.out_sn = 0;
@@ -567,13 +590,6 @@ static int run_gemm_tn(const void* A, int lda, const void* B, int ldb, int M, in
     p.out_fp32 = c_fp32;
     p.atomic_out = (splits > 1 || accumulate) ? 1 : 0;
     if (p.atomic_out && !c_fp32) return fail(FMRI_ERR_ARG, "accumulating gemm needs fp32 output");
-    if (splits > 1 && !accumulate) {
-        if (ldc != N) {
-            CUDA_OK(cudaMemset2DAsync(Cout, (size_t)ldc * 4, 0, (size_t)N * 4, M, st));
-        } else {
-            CUDA_OK(cudaMemsetAsync(Cout, 0, (size_t)M * N * 4, st));
-        }
-    }
     p.bias = bias;
     p.act = act;
     return dispatch_ig(p, BN, KCH, 1, st);
@@ -683,8 +699,16 @@ static int run_wgrad_tc(const void* Dn, int N, int PH, int PW, int Cd, const voi
                            : ((NCH == 64 && BN == 128 && num_taps > 1) ? (num_taps + 1) / 2 : num_taps);
     const long long base = (long long)tap_groups * p.m_tiles * p.n_tiles;
     p.splits = wave_splits(base, std::max<long long>(1, pt / 4));
-    p.out = ws;
-    return dispatch_wg(p, BN, NCH, st);
+    const long long n = (long long)num_taps * Cd * Cs;
+    SCRATCH(slices, float, (long long)p.splits * n, st);   // one slice per split
+    CUDA_OK(cudaMemsetAsync(slices, 0, sizeof(float) * (size_t)p.splits * n, st));
+    p.out = slices;
+    p.split_stride = n;
+    rc = dispatch_wg(p, BN, NCH, st);
+    if (rc) return rc;
+    rc = ordered_add(slices, p.splits, n, ws, st);
+    CUDA_OK(cudaFreeAsync(slices, st));
+    return rc;
 }
 
 // ================================================================================================ conv API
@@ -1226,9 +1250,18 @@ static int hwgrad_run(const void* T, const float* i0, const float* i1, const flo
         attr_smem = smem;
     }
     const int total = N * p.tiles_y;
-    hwgrad_kernel<<<std::min(total, 148 * (smem <= 110 * 1024 ? 2 : 1)), HW_THREADS, smem, st>>>(p);
+    const int nb = std::min(total, 148 * (smem <= 110 * 1024 ? 2 : 1));
+    const long long nw = 75LL * C;
+    SCRATCH(part, float, (long long)nb * (nw + C), st);   // one [75][C] (+ [C] bias) slice per persistent CTA
+    CUDA_OK(cudaMemsetAsync(part, 0, sizeof(float) * (size_t)nb * (nw + C), st));
+    p.dwk = part;
+    p.dbias = dbias ? part + nb * nw : nullptr;
+    hwgrad_kernel<<<nb, HW_THREADS, smem, st>>>(p);
     LAUNCH_OK();
-    return 0;
+    int rc = ordered_add(part, nb, nw, dwk, st);
+    if (!rc && dbias) rc = ordered_add(part + nb * nw, nb, C, dbias, st);
+    CUDA_OK(cudaFreeAsync(part, st));
+    return rc;
 }
 
 static int check_edge(const fmri_edge_desc* d, const void* ws, size_t ws_bytes) {
@@ -1551,7 +1584,8 @@ extern "C" int fmri_linear_wgrad(const fmri_linear_desc* d, const void* x, int l
             p.m_tiles = d->N / 128;
             p.n_tiles = d->K / BN;
             const long long base = (long long)p.m_tiles * p.n_tiles;
-            p.splits = wave_splits(base, std::max<long long>(1, p.tiles_x / 2));
+            (void)base;
+            p.splits = 1;   // one writer per dw element (see the linear split-K note above)
             p.out = dw;
             return dispatch_wg(p, BN, NCH, S(stream));
         }
@@ -1765,14 +1799,17 @@ extern "C" int fmri_relu_bitmask(const void* y, int dtype, long long pixels, int
 }
 extern "C" int fmri_colsum(const void* x, int dtype, long long rows, int C, float* out, void* stream) {
     const int rpb = rows_per_block_for(rows);
+    const int nb = cdiv(rows, rpb);
+    SCRATCH(part, float, (long long)nb * C, S(stream));
     if (dtype == FMRI_BF16)
-        colsum_kernel<__nv_bfloat16><<<cdiv(rows, rpb), 256, 0, S(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(x),
-                                                                            rows, C, out, rpb);
+        colsum_kernel<__nv_bfloat16><<<nb, 256, 0, S(stream)>>>(reinterpret_cast<const __nv_bfloat16*>(x), rows, C, part,
+                                                               rpb);
     else
-        colsum_kernel<float><<<cdiv(rows, rpb), 256, 0, S(stream)>>>(reinterpret_cast<const float*>(x), rows, C, out,
-                                                                    rpb);
+        colsum_kernel<float><<<nb, 256, 0, S(stream)>>>(reinterpret_cast<const float*>(x), rows, C, part, rpb);
     LAUNCH_OK();
-    return 0;
+    int rc = ordered_add(part, nb, C, out, S(stream));
+    CUDA_OK(cudaFreeAsync(part, S(stream)));
+    return rc;
 }
 
 template <typename TI, typename TO>
@@ -1974,15 +2011,22 @@ extern "C" int fmri_head_sigmoid_fwd(const void* x, int dtype, const float* w, c
 extern "C" int fmri_head_sigmoid_bwd(const void* x, int dtype, const float* w, const float* p, const float* gp,
                                      void* dx, float* dw, float* db, int rows, int F, void* stream) {
     const int rpb = 16;
+    const int nb = cdiv(rows, rpb);
+    SCRATCH(part, float, (long long)nb * (F + 1), S(stream));   // per-block dw [nb][F], then db [nb]
+    float* pw = dw ? part : nullptr;
+    float* pb = db ? part + (long long)nb * F : nullptr;
     if (dtype == FMRI_BF16)
-        head_sigmoid_bwd_kernel<__nv_bfloat16><<<cdiv(rows, rpb), 256, 0, S(stream)>>>(
-            reinterpret_cast<const __nv_bfloat16*>(x), w, p, gp, reinterpret_cast<__nv_bfloat16*>(dx), dw, db, rows, F,
+        head_sigmoid_bwd_kernel<__nv_bfloat16><<<nb, 256, 0, S(stream)>>>(
+            reinterpret_cast<const __nv_bfloat16*>(x), w, p, gp, reinterpret_cast<__nv_bfloat16*>(dx), pw, pb, rows, F,
             rpb);
     else
-        head_sigmoid_bwd_kernel<float><<<cdiv(rows, rpb), 256, 0, S(stream)>>>(
-            reinterpret_cast<const float*>(x), w, p, gp, reinterpret_cast<float*>(dx), dw, db, rows, F, rpb);
+        head_sigmoid_bwd_kernel<float><<<nb, 256, 0, S(stream)>>>(
+            reinterpret_cast<const float*>(x), w, p, gp, reinterpret_cast<float*>(dx), pw, pb, rows, F, rpb);
     LAUNCH_OK();
-    return 0;
+    int rc = dw ? ordered_add(pw, nb, F, dw, S(stream)) : 0;
+    if (!rc && db) rc = ordered_add(pb, nb, 1, db, S(stream));
+    CUDA_OK(cudaFreeAsync(part, S(stream)));
+    return rc;
 }
 extern "C" int fmri_bce_fwd(const float* p, float* out, int n, int positive, float scale, void* stream) {
     bce_fwd_kernel<<<cdiv(n, 256), 256, 0, S(stream)>>>(p, out, n, positive, scale);
@@ -2069,9 +2113,12 @@ extern "C" int fmri_axpby_tanh_bwd(float a, const float* x, float b, const float
 extern "C" int fmri_chansum_nchw(const float* x, int N, int C, long long HW, float* out, int accumulate, void* stream) {
     if (!accumulate) CUDA_OK(cudaMemsetAsync(out, 0, sizeof(float) * C, S(stream)));
     dim3 grid(C, std::max(1, std::min(N, 148 * 2 / std::max(C, 1))));
-    chansum_nchw_kernel<<<grid, 256, 0, S(stream)>>>(x, N, C, HW, out);
+    SCRATCH(part, float, (long long)grid.y * C, S(stream));
+    chansum_nchw_kernel<<<grid, 256, 0, S(stream)>>>(x, N, C, HW, part);
     LAUNCH_OK();
-    return 0;
+    int rc = ordered_add(part, (int)grid.y, C, out, S(stream));
+    CUDA_OK(cudaFreeAsync(part, S(stream)));
+    return rc;
 }
 extern "C" int fmri_vecsum(const float* x, long long n, float scale, float* out, int accumulate, void* stream) {
     vecsum_kernel<<<1, 256, 0, S(stream)>>>(x, n, scale, out, accumulate);

@@ -198,7 +198,8 @@ __global__ void __launch_bounds__(HW_THREADS) hwgrad_kernel(const __grid_constan
                     if (p.flip) tap = 24 - tap;
 #pragma unroll
                     for (int ci = 0; ci < 3; ++ci)
-                        atomicAdd(p.dwk + (size_t)(ci * 25 + tap) * p.C + c, __uint_as_float(v[h * 8 + ci]));
+                        atomicAdd(p.dwk + (size_t)blockIdx.x * 75 * p.C + (size_t)(ci * 25 + tap) * p.C + c,
+                                  __uint_as_float(v[h * 8 + ci]));
                 }
             }
         }
@@ -206,7 +207,7 @@ __global__ void __launch_bounds__(HW_THREADS) hwgrad_kernel(const __grid_constan
             uint32_t v[16];
             tmem_ld16(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + 240, v);
             tmem_ld_wait();
-            if (valid) atomicAdd(p.dbias + c, __uint_as_float(v[0]));
+            if (valid) atomicAdd(p.dbias + (size_t)blockIdx.x * p.C + c, __uint_as_float(v[0]));
         }
         tc_fence_before();
     }

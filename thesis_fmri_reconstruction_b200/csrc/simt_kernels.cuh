@@ -1058,6 +1058,17 @@ __global__ void relu_bwd_kernel(const T* __restrict__ y, const T* __restrict__ d
         st_f(dx + i, ld_f(y + i) > 0.f ? ld_f(dy + i) : 0.f);
 }
 
+// dst[i] += part[0][i] + part[1][i] + ... + part[nparts-1][i], always in this order: the fixed-order replacement for
+// atomics where several CTAs contribute to one element (the result must not depend on which CTA finishes first)
+template <typename T>
+__global__ void ordered_add_kernel(const T* __restrict__ part, int nparts, long long n, T* __restrict__ dst) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        T s = part[i];
+        for (int b = 1; b < nparts; ++b) s += part[(long long)b * n + i];
+        dst[i] += s;
+    }
+}
+
 // column sums of a [rows, C] matrix into fp32 (bias gradients)
 template <typename T>
 __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ x, long long rows, int C,
@@ -1067,7 +1078,7 @@ __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ x, lo
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
         float s = 0.f;
         for (long long r = r0; r < r1; ++r) s += ld_f(x + r * C + c);
-        atomicAdd(out + c, s);
+        out[(long long)blockIdx.x * C + c] = s;   // this block's partial (summed in block order by ordered_add_kernel)
     }
 }
 
@@ -1262,12 +1273,12 @@ __global__ void __launch_bounds__(256) head_sigmoid_bwd_kernel(const T* __restri
             if (dx) st_f(dx + (long long)r * F + j, dl * wj);
             acc += dl * ld_f(x + (long long)r * F + j);
         }
-        if (dw) atomicAdd(dw + j, acc);
+        if (dw) dw[(long long)blockIdx.x * F + j] = acc;   // per-block partials, see colsum_kernel
     }
     if (db && threadIdx.x == 0) {
         float acc = 0.f;
         for (int r = r0; r < r1; ++r) acc += gp[r] * p[r] * (1.f - p[r]);
-        atomicAdd(db, acc);
+        db[blockIdx.x] = acc;
     }
 }
 // bce[i] = -log(sign>0 ? p+1e-3 : 1-p+1e-3) * scale
@@ -1375,7 +1386,7 @@ __global__ void __launch_bounds__(256) chansum_nchw_kernel(const float* __restri
     if (threadIdx.x < 32) {
         float v = threadIdx.x < 8 ? red[threadIdx.x] : 0.f;
         v = warp_sum(v);
-        if (threadIdx.x == 0) atomicAdd(out + c, v);
+        if (threadIdx.x == 0) out[blockIdx.y * C + c] = v;   // per-block partial, see colsum_kernel
     }
 }
 // out[0] (+)= scale * sum(x[0..n)) in fp64 internally; single block (n is a batch-sized vector of per-sample losses)

@@ -198,7 +198,7 @@ __global__ void __launch_bounds__(192) igemm_kernel(const __grid_constant__ IgPa
         fence_barrier_init();
     }
     if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
-    for (int i = threadIdx.x; i < 2 * BN; i += blockDim.x) s_stat[i] = 0.f;
+    for (int i = threadIdx.x; i < 4 * 2 * BN; i += blockDim.x) s_stat[i] = 0.f;   // one [2][BN] slot per epilogue warp
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -346,8 +346,9 @@ __global__ void __launch_bounds__(192) igemm_kernel(const __grid_constant__ IgPa
                     }
                     const float s1 = warp_colsum32(f, lane);
                     const float s2 = warp_colsum32(g, lane);
-                    atomicAdd(&s_stat[stat_col + lane], s1);
-                    atomicAdd(&s_stat[BN + stat_col + lane], s2);
+                    float* my_stat = s_stat + q * 2 * BN;   // this warp's slot: no order-dependent shared atomics
+                    my_stat[stat_col + lane] += s1;
+                    my_stat[BN + stat_col + lane] += s2;
                 }
             }
         }
@@ -359,8 +360,13 @@ __global__ void __launch_bounds__(192) igemm_kernel(const __grid_constant__ IgPa
         const int ncol = p.merge ? 32 : BN;
         const int cbase = p.merge ? 0 : nt * BN;
         for (int i = threadIdx.x; i < ncol; i += blockDim.x) {
-            atomicAdd(p.stat_sum + cbase + i, (double)s_stat[i]);
-            atomicAdd(p.stat_sq + cbase + i, (double)s_stat[BN + i]);
+            float a = 0.f, b = 0.f;
+            for (int w = 0; w < 4; ++w) {
+                a += s_stat[w * 2 * BN + i];
+                b += s_stat[w * 2 * BN + BN + i];
+            }
+            atomicAdd(p.stat_sum + cbase + i, (double)a);
+            atomicAdd(p.stat_sq + cbase + i, (double)b);
         }
     }
     if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
@@ -1053,6 +1059,7 @@ struct WgParams {
     int rows;  // bw*bh*bn, multiple of 16
     int merge_taps;  // one N = TG*BN MMA per K step when the kernel supports it (A/B switch)
     float* out;
+    long long split_stride;  // elements between the output slices of consecutive splits (0: all splits add into one)
 };
 
 // TG = filter taps handled by one CTA against the SAME dense-operand tile: with a 32-channel shifted side the dense tile
@@ -1201,7 +1208,8 @@ __global__ void __launch_bounds__(192) wgrad_kernel(const __grid_constant__ WgPa
         const bool valid = m < p.m_total;
 #pragma unroll 1
         for (int tg = 0; tg < tg_live; ++tg) {
-            float* orow = p.out + ((long long)(tap0 + tg) * p.m_total + m) * p.n_total + ntile * BN;
+            float* orow = p.out + blockIdx.z * p.split_stride + ((long long)(tap0 + tg) * p.m_total + m) * p.n_total +
+                          ntile * BN;
 #pragma unroll 1
             for (int c0 = 0; c0 < BN; c0 += 32) {
                 uint32_t v[32];
