@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FMRI_ABI_VERSION 2
+#define FMRI_ABI_VERSION 3
 
 typedef enum { FMRI_OK = 0, FMRI_ERR_ARG = -1, FMRI_ERR_UNSUPPORTED = -2, FMRI_ERR_CUDA = -3, FMRI_ERR_WORKSPACE = -4 } fmri_status;
 typedef enum { FMRI_F32 = 0, FMRI_BF16 = 1 } fmri_dtype;
@@ -243,6 +243,14 @@ int fmri_vecsum(const float* x, long long n, float scale, float* out, int accumu
 /* gates[0] = train_dis, gates[1] = train_dec (0.f / 1.f) from sums[0] = sum bce_original, sums[1] = sum bce_predicted
  * over `count` samples (train_vgan_stage1.py:396-404) */
 int fmri_vgan_gate(const float* sums, float count, float margin, float equilibrium, float* gates, void* stream);
+/* The same gate with the pre-gate value of train_dis as an argument: the loss-mix block of train_vgan_stage1.py:359-388
+ * sets train_dis = False in mode 'vae' (:387) before the gate runs, and the gate's "neither -> both" rule (:403-404) can
+ * turn it back on. fmri_vgan_gate is this call with train_dis_in = 1. */
+int fmri_vgan_gate_mix(const float* sums, float count, float margin, float equilibrium, int train_dis_in, float* gates,
+                       void* stream);
+/* x[i] *= s for i < n (fp32, in place). Mode 'vae' (train_vgan_stage1.py:382-387) takes g_dec = lambda_mse * the decoder
+ * weight gradients of d sum(nle) / d decoder, whose data gradient is the encoder's upstream at unit weight. */
+int fmri_scale_f32(float* x, long long n, float s, void* stream);
 /* eval-mode BatchNorm statistics: mean = running_mean, invstd = rsqrt(running_var + eps) */
 int fmri_bn_eval_stats(const float* running_mean, const float* running_var, int C, float eps, float* mean,
                        float* invstd, void* stream);

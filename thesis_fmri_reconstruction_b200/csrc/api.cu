@@ -2125,9 +2125,20 @@ extern "C" int fmri_vecsum(const float* x, long long n, float scale, float* out,
     LAUNCH_OK();
     return 0;
 }
+extern "C" int fmri_vgan_gate_mix(const float* sums, float count, float margin, float equilibrium, int train_dis_in,
+                                  float* gates, void* stream) {
+    vgan_gate_kernel<<<1, 32, 0, S(stream)>>>(sums, count, margin, equilibrium, train_dis_in, gates);
+    LAUNCH_OK();
+    return 0;
+}
 extern "C" int fmri_vgan_gate(const float* sums, float count, float margin, float equilibrium, float* gates,
                               void* stream) {
-    vgan_gate_kernel<<<1, 32, 0, S(stream)>>>(sums, count, margin, equilibrium, gates);
+    return fmri_vgan_gate_mix(sums, count, margin, equilibrium, 1, gates, stream);
+}
+extern "C" int fmri_scale_f32(float* x, long long n, float s, void* stream) {
+    if (!x || n < 0) return fail(FMRI_ERR_ARG, "scale_f32 arguments");
+    if (n == 0) return 0;
+    scale_f32_kernel<<<grid1d(n, 256), 256, 0, S(stream)>>>(x, n, s);
     LAUNCH_OK();
     return 0;
 }

@@ -1404,17 +1404,23 @@ __global__ void __launch_bounds__(256) vecsum_kernel(const float* __restrict__ x
     if (threadIdx.x == 0) out[0] = (accumulate ? out[0] : 0.f) + scale * (float)red[0];
 }
 // equilibrium gate on the device (train_vgan_stage1.py:396-404): sums[0] = sum bce_original, sums[1] = sum bce_predicted
-// over `count` samples (already reduced across ranks); gates[0] = train_dis, gates[1] = train_dec as 0.f / 1.f
+// over `count` samples (already reduced across ranks); gates[0] = train_dis, gates[1] = train_dec as 0.f / 1.f.
+// train_dis_in: the value the loss-mix block leaves in train_dis before the gate (0 in mode 'vae', :387; 1 otherwise)
 __global__ void vgan_gate_kernel(const float* __restrict__ sums, float count, float margin, float equilibrium,
-                                 float* __restrict__ gates) {
+                                 int train_dis_in, float* __restrict__ gates) {
     if (threadIdx.x || blockIdx.x) return;
     const float mo = sums[0] / count, mp = sums[1] / count;
-    bool dis = true, dec = true;
+    bool dis = train_dis_in != 0, dec = true;
     if (mo < equilibrium - margin || mp < equilibrium - margin) dis = false;
     if (mo > equilibrium + margin || mp > equilibrium + margin) dec = false;
     if (!dis && !dec) dis = dec = true;
     gates[0] = dis ? 1.f : 0.f;
     gates[1] = dec ? 1.f : 0.f;
+}
+// x[i] *= s over a flat fp32 buffer (elementwise: keeps the step's fixed-order determinism)
+__global__ void scale_f32_kernel(float* __restrict__ x, long long n, float s) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        x[i] *= s;
 }
 // eval-mode BatchNorm: mean / invstd from the running statistics
 __global__ void bn_eval_stats_kernel(const float* __restrict__ rm, const float* __restrict__ rv, int C, float eps,

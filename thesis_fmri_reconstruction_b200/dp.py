@@ -61,11 +61,12 @@ def allreduce_sum_(tensors, group=None):
         td.all_reduce(t, op=td.ReduceOp.SUM, group=group)
 
 
-def gate_from_sums(sum_bce_o, sum_bce_p, global_batch, margin, equilibrium):
+def gate_from_sums(sum_bce_o, sum_bce_p, global_batch, margin, equilibrium, train_dis_in=True):
     """Host restatement of the gate (train_vgan_stage1.py:396-404) on globally reduced sums; the engine evaluates the same
-    rule on the device (fmri_vgan_gate). Returns (train_dis, train_dec)."""
+    rule on the device (fmri_vgan_gate_mix). train_dis_in: train_dis as the loss-mix block leaves it before the gate (False
+    in mode 'vae', :387). Returns (train_dis, train_dec)."""
     mo, mp = sum_bce_o / global_batch, sum_bce_p / global_batch
-    dis = dec = True
+    dis, dec = bool(train_dis_in), True
     if mo < equilibrium - margin or mp < equilibrium - margin:
         dis = False
     if mo > equilibrium + margin or mp > equilibrium + margin:

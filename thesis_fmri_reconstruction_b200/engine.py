@@ -1,8 +1,8 @@
 """Fused training steps: one forward, the minimal backward, gradient exchange and the optimizer update, all as
 launches of libfmri_b200.so kernels on raw device buffers (no autograd graph, no host round trip inside the step).
 
-VaeGanStage1 follows /root/reference/train/train_vgan_stage1.py:316-432 (mode 'vae-gan') and computes exactly the
-three gradients its optimizers consume -- g_enc = d loss_encoder / d encoder, g_dec = d loss_decoder / d decoder,
+VaeGanStage1 follows the reference's train/train_vgan_stage1.py:316-432 (all four loss mixes of :359-388) and computes
+exactly the three gradients its optimizers consume -- g_enc = d loss_encoder / d encoder, g_dec = d loss_decoder / d decoder,
 g_dis = d loss_discriminator / d discriminator at the pre-step weights (SURVEY.md 0-7) -- with ONE discriminator forward
 (the reference runs it twice on the same inputs, vae_gan.py:284-285; BN running statistics are updated twice to match)
 and no discarded gradient (the reference's three full autograd sweeps execute 2.35x the necessary FLOPs).
@@ -152,14 +152,21 @@ class _TrainerBase:
 
 
 class VaeGanStage1(_TrainerBase):
-    """Stage-I VAE/GAN trainer (image -> image): visual Encoder, Decoder, Discriminator, three RMSprop optimizers."""
+    """Stage-I VAE/GAN trainer (image -> image): visual Encoder, Decoder, Discriminator, three RMSprop optimizers.
+
+    mode: the loss mix of train_vgan_stage1.py:359-388. 'vae-gan' and 'beta-vae' use the discriminator's feature MSE;
+    'dcgan' (:374-380) and 'vae' (:382-387) use the pixel NLE instead and leave bce_p out of loss_discriminator. 'dcgan'
+    trains no encoder; 'vae' drops the discriminator term from loss_decoder and sets train_dis = False before the gate.
+    gate=False applies the mix's own flags without the gate: 'vae' trains the decoder only, every other mix trains both."""
+
+    MODES = ("vae-gan", "beta-vae", "dcgan", "vae")
 
     def __init__(self, params, buffers, cfg, z=128, adt=BF16, hp=None, dist_group=None, gate=True, mode="vae-gan", beta=1.0):
         from .hp import HP_VGAN
 
-        if mode not in ("vae-gan", "beta-vae"):
-            # train_vgan_stage1.py:359-388 also has 'dcgan' and 'vae' (pixel-NLE mixes): served by the module path
-            raise L.FmriError("the fused Stage-I step implements the 'vae-gan' and 'beta-vae' loss mixes")
+        if mode not in self.MODES:
+            raise L.FmriError(f"unknown Stage-I loss mix {mode!r}: the fused step implements {', '.join(self.MODES)} "
+                              "(train_vgan_stage1.py:359-388)")
         self.mode, self.beta, self._klw = mode, float(beta), 1.0
         self.cfg, self.z, self.adt = cfg, z, adt
         self.hp = dict(HP_VGAN if hp is None else hp)
@@ -230,14 +237,16 @@ class VaeGanStage1(_TrainerBase):
         self._allreduce_async([sc[:8]])  # global loss sums: the gate must agree on every rank (SURVEY.md 0-10)
         out = dict(x_tilde=x_tilde, x_p=x_p, disc_layer_nhwc=raw3, disc_class=p, mu=mu, logvar=lv, z=zz, kl=kl, mse=mse,
                    bce=bce, nle=nle)
-        return NN.Ctx(B=B, eps=eps, ce=ce, cd1=cd1, cd2=cd2, cc=cc, raw3=raw3, p=p, mu=mu, lv=lv, out=out)
+        return NN.Ctx(B=B, x=x, eps=eps, ce=ce, cd1=cd1, cd2=cd2, cc=cc, raw3=raw3, p=p, mu=mu, lv=lv, out=out)
 
     def backward(self, st):
         """The three used gradients (SURVEY.md 0-7) from the saved forward state, as four sweeps."""
-        hp, B, z = self.hp, st.B, self.z
+        if self.mode in ("dcgan", "vae"):
+            return self._backward_pixel_nle(st)
+        hp, B = self.hp, st.B
         lam = float(hp["lambda_mse"])
-        be, bd, bc = self.buckets["encoder."], self.buckets["decoder."], self.buckets["discriminator."]
-        ce, cd1, cd2, cc, raw3, p, mu, lv, eps = st.ce, st.cd1, st.cd2, st.cc, st.raw3, st.p, st.mu, st.lv, st.eps
+        bd, bc = self.buckets["decoder."], self.buckets["discriminator."]
+        cd1, cd2, cc, raw3, p = st.cd1, st.cd2, st.cc, st.raw3, st.p
         Fd = raw3[0].numel()
         # (1) discriminator, class-score path: g_dis = d loss_discriminator / d discriminator, plus d loss_dis / d(x_tilde, x_p)
         gp = E(3 * B)
@@ -257,6 +266,49 @@ class VaeGanStage1(_TrainerBase):
         self._ev_dec = self._allreduce_async([bd.flat_g])   # loss sums, discriminator and decoder buckets are reduced here
         # (4) encoder: g_enc = d [sum kl + sum mse] / d encoder; the mse term flows x_tilde -> decoder (data gradient) -> z
         dz = self.dec.backward(bd.P, cd1, 1.0, dimg_mse, 0.0, None, None, False, False, True)
+        dycat = self._encoder_backward(st, dz)
+        st.sweeps = dict(dimg_bce=dimg_bce, dimg_mse=dimg_mse, dz=dz, dycat=dycat)
+
+    def _backward_pixel_nle(self, st):
+        """Modes 'dcgan' (train_vgan_stage1.py:374-380) and 'vae' (:382-387): no feature-tap sweep (2), because the pixel NLE
+        replaces the feature MSE; bce_p is not in loss_discriminator, but train-mode BatchNorm couples the whole 3B batch, so
+        its gradient slot is zero while x_tilde still receives an image gradient from the class path."""
+        hp, B = self.hp, st.B
+        lam = float(hp["lambda_mse"])
+        bd, bc = self.buckets["decoder."], self.buckets["discriminator."]
+        x, x_tilde, p = st.x, st.out["x_tilde"], st.p
+        dcgan = self.mode == "dcgan"
+        # (1) class path: g_dis = d [sum bce_o + sum bce_s] / d discriminator; image gradients only where loss_decoder has
+        # the discriminator term ('dcgan'). 'vae' runs it every step: its gate is decided on the device.
+        gp = E(3 * B)
+        ones = self._ones(3 * B)
+        L.bce_bwd(p[:B], ones, gp[:B], B, True, 1.0)
+        gp[B:2 * B].zero_()
+        L.bce_bwd(p[2 * B:], ones, gp[2 * B:], B, False, 1.0)
+        dimg_bce = self.dis.backward_gan(bc.P, st.cc, gp, bc.G, False, True, (1, 3) if dcgan else None)
+        self._allreduce_async([bc.flat_g])
+        dnle = torch.empty_like(x_tilde)
+        L.rowsqdiff_bwd(x_tilde, x, ones, dnle, None, B, x[0].numel(), 0.5)   # d sum(nle) / d x_tilde = x_tilde - x
+        if dcgan:
+            # (3) g_dec = d [lambda * sum nle - (1 - lambda) * loss_dis] / d decoder over both decoder calls; no encoder
+            self.dec.backward(bd.P, st.cd1, lam, dnle, -(1.0 - lam), dimg_bce[:B], bd.G, False, True, False)
+            self.dec.backward(bd.P, st.cd2, -(1.0 - lam), dimg_bce[B:], 0.0, None, bd.G, True, True, False)
+            self._ev_dec = self._allreduce_async([bd.flat_g])
+            st.sweeps = dict(dimg_bce=dimg_bce, dnle=dnle)
+            return
+        # 'vae': one decoder sweep over call 1 gives d sum(nle) / d decoder and dz; the backward is linear in its upstream,
+        # so g_dec = lambda * those weight gradients and dz is the encoder's upstream at unit weight. x_p gets no gradient.
+        dz = self.dec.backward(bd.P, st.cd1, 1.0, dnle, 0.0, None, bd.G, False, True, True)
+        NN.join_side()
+        L.scale_f32(bd.flat_g, lam)
+        self._ev_dec = self._allreduce_async([bd.flat_g])
+        dycat = self._encoder_backward(st, dz)
+        st.sweeps = dict(dnle=dnle, dz=dz, dycat=dycat)
+
+    def _encoder_backward(self, st, dz):
+        """Reparameterisation / KL backward from dz, then the encoder sweep with its gradient exchange. Returns dycat."""
+        be, B, z = self.buckets["encoder."], st.B, self.z
+        mu, lv, eps = st.mu, st.lv, st.eps
         dycat = E(B, 2 * z, dtype=self.adt)
         # 'beta-vae' (:359-362): loss_encoder = beta / batch_size * sum kl + sum mse, the batch being the global one here
         self._klw = self.beta / float(B * self.world) if self.mode == "beta-vae" else 1.0
@@ -267,13 +319,13 @@ class VaeGanStage1(_TrainerBase):
         # part (4.1 MB) is exchanged after the last kernel
         split = min(off for k, (off, _) in be.offsets.items() if not k.startswith("conv."))
         if self.world > 1 and all(off < split for k, (off, _) in be.offsets.items() if k.startswith("conv.")):
-            self.enc.backward(be.P, ce, dycat, be.G, False, True, True,
+            self.enc.backward(be.P, st.ce, dycat, be.G, False, True, True,
                               after_fc=lambda: self._allreduce_async([be.flat_g[split:]]))
             self._allreduce_async([be.flat_g[:split]])
         else:
-            self.enc.backward(be.P, ce, dycat, be.G, False, True, True)
+            self.enc.backward(be.P, st.ce, dycat, be.G, False, True, True)
             self._allreduce_async([be.flat_g])
-        st.sweeps = dict(dimg_bce=dimg_bce, dimg_mse=dimg_mse, dz=dz, dycat=dycat)
+        return dycat
 
     _enc_bn_updates = 1
 
@@ -301,12 +353,16 @@ class VaeGanStage1(_TrainerBase):
         else:
             self._wait_comm()
         gates = self.sc[8:10]
+        dis_in = self.mode != "vae"   # 'vae' sets train_dis = False before the gate (train_vgan_stage1.py:387)
         if self.gate_on:
-            L.vgan_gate(self.sc, float(B_global), hp["margin"], hp["equilibrium"], gates)
+            L.vgan_gate_mix(self.sc, float(B_global), hp["margin"], hp["equilibrium"], dis_in, gates)
         else:
-            gates.fill_(1.0)
+            gates[0:1].fill_(1.0 if dis_in else 0.0)
+            gates[1:2].fill_(1.0)
         nets = {"encoder.": self.enc, "decoder.": self.dec, "discriminator.": self.dis}
         for pre, g in (("decoder.", gates[1:2]), ("discriminator.", gates[0:1]), ("encoder.", None)):
+            if pre == "encoder." and self.mode == "dcgan":
+                continue   # :374-380 trains no encoder: its parameters, square_avg and operand packs stay as they are
             if pre == "encoder." and staged:
                 self._wait_comm()
             b = self.buckets[pre]
@@ -324,9 +380,16 @@ class VaeGanStage1(_TrainerBase):
         """Host view of the last step's (globally reduced) loss sums, as the reference logs them (stage1 :391-394)."""
         s = self.sc.tolist()
         lam = float(self.hp["lambda_mse"])
-        loss_dis = s[0] + s[1] + s[2]
-        return dict(loss_encoder=getattr(self, "_klw", 1.0) * s[3] + s[4], loss_discriminator=loss_dis,
-                    loss_decoder=lam * s[4] - (1 - lam) * loss_dis,
+        mode = getattr(self, "mode", "vae-gan")
+        if mode in ("dcgan", "vae"):   # train_vgan_stage1.py:374-387 (the 'dcgan' loss_encoder is logged, not trained)
+            loss_dis = s[0] + s[2]
+            loss_enc = s[3] + s[5]
+            loss_dec = lam * s[5] - ((1 - lam) * loss_dis if mode == "dcgan" else 0.0)
+        else:
+            loss_dis = s[0] + s[1] + s[2]
+            loss_enc = getattr(self, "_klw", 1.0) * s[3] + s[4]
+            loss_dec = lam * s[4] - (1 - lam) * loss_dis
+        return dict(loss_encoder=loss_enc, loss_discriminator=loss_dis, loss_decoder=loss_dec,
                     nle=s[5], bce_o=s[0], bce_p=s[1], bce_s=s[2], kl=s[3], mse=s[4], train_dis=s[8] != 0,
                     train_dec=s[9] != 0)
 

@@ -480,6 +480,20 @@ def vgan_gate(sums, count, margin, equilibrium, gates):
     _check(load().fmri_vgan_gate(ptr(sums), _f(count), _f(margin), _f(equilibrium), ptr(gates), stream()))
 
 
+def vgan_gate_mix(sums, count, margin, equilibrium, train_dis_in, gates):
+    """The gate with the loss mix's pre-gate train_dis (False in mode 'vae', train_vgan_stage1.py:387)."""
+    _check(load().fmri_vgan_gate_mix(ptr(sums), _f(count), _f(margin), _f(equilibrium), int(bool(train_dis_in)), ptr(gates),
+                                     stream()))
+
+
+def scale_f32(x, s):
+    """x *= s in place (contiguous fp32 CUDA tensor)."""
+    _require_cuda(x)
+    if x.dtype != torch.float32:
+        raise FmriError("scale_f32 expects a float32 tensor")
+    _check(load().fmri_scale_f32(ptr(x), _ll(x.numel()), _f(s), stream()))
+
+
 def bn_eval_stats(rm, rv, Cc, eps, mean, invstd):
     _check(load().fmri_bn_eval_stats(ptr(rm), ptr(rv), Cc, _f(eps), ptr(mean), ptr(invstd), stream()))
 
