@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FMRI_ABI_VERSION 3
+#define FMRI_ABI_VERSION 4
 
 typedef enum { FMRI_OK = 0, FMRI_ERR_ARG = -1, FMRI_ERR_UNSUPPORTED = -2, FMRI_ERR_CUDA = -3, FMRI_ERR_WORKSPACE = -4 } fmri_status;
 typedef enum { FMRI_F32 = 0, FMRI_BF16 = 1 } fmri_dtype;
@@ -61,24 +61,18 @@ int fmri_conv_pack_weights(const fmri_conv_desc* d, const float* w, void* pack_f
  * path), `pack_f` bf16 pack (used by the bf16 path). */
 int fmri_conv_fprop(const fmri_conv_desc* d, const void* x, const float* w, const void* pack_f, const float* bias,
                     int act, void* y, double* stat_sum, double* stat_sq, void* stream);
-/* Optional fusion for fmri_conv_dgrad: when dx is the upstream gradient of a BatchNorm(+ReLU) layer whose pre-BN input is
- * `x` (same [N,H,W,Cin] layout and dtype as dx), the call also leaves that layer's backward sums in `sums`:
- * sums[c] = sum g, sums[Cin + c] = sum g * xhat, g = dx masked by the forward ReLU. Pass the same buffer as the `ws` of
- * fmri_bn_backward with sums_ready = 1 (the separate reduction pass, 2 of BN-backward's 5 tensor passes, disappears).
- * With mean == NULL the struct instead describes a bias+ReLU layer WITHOUT BatchNorm (Discriminator.conv[0],
- * vae_gan.py:145-147): `x` is that layer's post-ReLU output and the call applies its ReLU backward, dx *= (x > 0), in the
- * data-gradient epilogue (saves the separate read-dy / write-dx pass of fmri_relu_backward); the other fields are unused. */
+/* Optional fusion for fmri_conv_dgrad: when dx is the upstream gradient of a bias+ReLU layer WITHOUT BatchNorm
+ * (Discriminator.conv[0], vae_gan.py:145-147), `y` is that layer's post-ReLU output (same [N,H,W,Cin] layout and dtype as dx)
+ * and the call applies its ReLU backward, dx *= (y > 0), in the data-gradient epilogue (saves the separate read-dy /
+ * write-dx pass of fmri_relu_backward). */
 typedef struct {
-    const void* x;
-    const float *mean, *invstd, *gamma, *beta;
-    int relu;
-    double* sums; /* >= 3 * Cin doubles (fmri_bn_backward workspace) */
-    const unsigned* mask_bits; /* mean == NULL mode, optional: fmri_relu_bitmask() of `x` (32-channel tensors): the epilogue
-                                * then reads 4 bytes per pixel instead of 64 */
-} fmri_bn_fuse;
-/* dx = conv data-gradient of dy (replaces aten::convolution_backward input-grad); fuse nullable */
+    const void* y;
+    const unsigned* bits; /* optional: fmri_relu_bitmask() of `y` (32-channel tensors): the epilogue then reads 4 bytes per
+                           * pixel instead of 64 */
+} fmri_relu_mask;
+/* dx = conv data-gradient of dy (replaces aten::convolution_backward input-grad); relu_mask nullable */
 int fmri_conv_dgrad(const fmri_conv_desc* d, const void* dy, const float* w, const void* pack_d, void* dx,
-                    const fmri_bn_fuse* fuse, void* stream);
+                    const fmri_relu_mask* relu_mask, void* stream);
 /* dw (+)= conv weight-gradient, reference layout fp32. Workspace: fmri_conv_wgrad_workspace() bytes. */
 size_t fmri_conv_wgrad_workspace(const fmri_conv_desc* d);
 int fmri_conv_wgrad(const fmri_conv_desc* d, const void* x, const void* dy, float* dw, int accumulate, void* ws,
@@ -148,7 +142,7 @@ int fmri_bn_apply(const void* x, int x_dtype, void* y, int y_dtype, long long ro
 /* dx, dgamma (+)=, dbeta (+)= ; train=0 treats mean/invstd as constants (eval-mode BN). ws: 3*C doubles. */
 int fmri_bn_backward(const void* x, int x_dtype, const void* dy, void* dx, int g_dtype, long long rows, int C,
                      const float* mean, const float* invstd, const float* gamma, const float* beta, int relu, int train,
-                     float* dgamma, float* dbeta, int accumulate, double* ws, int sums_ready, void* stream);
+                     float* dgamma, float* dbeta, int accumulate, double* ws, void* stream);
 /* The same with dx produced for rows [row0, row0 + nrows) only (dx points at the first of them): train-mode BatchNorm couples
  * all rows through the two sums, so those always run over the whole [rows, C] matrix, but a caller that needs the input
  * gradient of a few samples only (the discriminator's feature-tap sweep feeds ONE of its three image sources,
@@ -156,9 +150,9 @@ int fmri_bn_backward(const void* x, int x_dtype, const void* dy, void* dx, int g
 int fmri_bn_backward_slice(const void* x, int x_dtype, const void* dy, void* dx, int g_dtype, long long rows, long long row0,
                            long long nrows, int C, const float* mean, const float* invstd, const float* gamma,
                            const float* beta, int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws,
-                           int sums_ready, void* stream);
+                           void* stream);
 /* bits[pixel] bit j = (y[pixel][j] > 0): ReLU mask of a channels-last bf16 tensor with exactly 32 channels, 4 B per pixel
- * (consumed by fmri_conv_dgrad through fmri_bn_fuse.mask_bits) */
+ * (consumed by fmri_conv_dgrad through fmri_relu_mask.bits) */
 int fmri_relu_bitmask(const void* y, int dtype, long long pixels, int C, unsigned* bits, void* stream);
 int fmri_relu_backward(const void* y, const void* dy, void* dx, int dtype, long long n, void* stream);
 int fmri_colsum(const void* x, int dtype, long long rows, int C, float* out /* += */, void* stream);

@@ -1,7 +1,7 @@
 """Times the 32-channel implicit-GEMM launches of the batch-4096 step in isolation (CUDA events, 5 repetitions after warm-up).
 With FMRI_IG_SKIP=1|2|4|8 one role of igemm_persistent_kernel is switched off (TMA loads / whole epilogue / MMAs / only the
-epilogue's global stores): the role whose removal shortens the kernel most is the one that bounds it; FMRI_IG_YR=0 selects
-the tap-per-box gather instead of the row-reuse one.  python scripts/igemm_probe.py [B]"""
+epilogue's global stores): the role whose removal shortens the kernel most is the one that bounds it.
+python scripts/igemm_probe.py [B]"""
 import os
 import sys
 
@@ -67,7 +67,7 @@ def main():
     y2 = torch.empty(N3, 16, 16, 256, dtype=BF, device=dev)
     u1, u2 = torch.zeros(256, dtype=F64, device=dev), torch.zeros(256, dtype=F64, device=dev)
     rows.append(("D block 2 fprop 128->256 s2, 3B imgs, BN stats", lambda: L.conv_fprop(d2, y, w2, p2, None, L.ACT_NONE, y2, u1, u2), 2.0 * N3 * 16 * 16 * 256 * 128 * 25))
-    print(f"# FMRI_IG_SKIP={os.environ.get('FMRI_IG_SKIP', '0')} FMRI_IG_YR={os.environ.get('FMRI_IG_YR', '1')} B={B}")
+    print(f"# FMRI_IG_SKIP={os.environ.get('FMRI_IG_SKIP', '0')} B={B}")
     for name, fn, flops in rows:
         ms = timeit(fn)
         print(f"{name:76s} {ms:8.3f} ms {flops / ms / 1e9:8.1f} TFLOP/s")

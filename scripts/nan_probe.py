@@ -39,7 +39,7 @@ for n in dir(lib):
                                                             "profile_end", "launch_count", "conv_desc", "edge_desc",
                                                             "linear_desc", "conv_out_hw", "conv_pack_elems",
                                                             "conv_wgrad_workspace", "edge_workspace", "FmriError", "ConvDesc",
-                                                            "EdgeDesc", "LinearDesc", "BnFuse"):
+                                                            "EdgeDesc", "LinearDesc", "ReluMask"):
         setattr(lib, n, wrap(n, f))
 
 P, S = init.init_vaegan(hp.CFG64, 128, seed=12345)

@@ -158,12 +158,12 @@ static int launch_ig(const IgParams& p, int classes, cudaStream_t st) {
     LAUNCH_OK();
     return 0;
 }
-template <int BN, int KCH, int STAGES, int MT, int EXTRA, bool YR = false>
+template <int BN, int KCH, int STAGES, int MT, bool MASK, bool YR = false>
 static int launch_ig_persistent_x(const IgParams& p, int classes, cudaStream_t st) {
-    using L = IgSmem<BN, KCH, STAGES, MT, YR, EXTRA, true>;
+    using L = IgSmem<BN, KCH, STAGES, MT, YR, true>;
     static bool attr_done = false;
     if (!attr_done) {
-        CUDA_OK(cudaFuncSetAttribute(igemm_persistent_kernel<BN, KCH, STAGES, MT, EXTRA, YR>,
+        CUDA_OK(cudaFuncSetAttribute(igemm_persistent_kernel<BN, KCH, STAGES, MT, MASK, YR>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, L::TOTAL));
         attr_done = true;
     }
@@ -172,33 +172,25 @@ static int launch_ig_persistent_x(const IgParams& p, int classes, cudaStream_t s
     // resident CTAs per SM: TMEM columns, shared memory and registers (asked from the runtime once per instantiation)
     static int occ = 0;
     if (!occ) {
-        CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, igemm_persistent_kernel<BN, KCH, STAGES, MT, EXTRA, YR>,
+        CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, igemm_persistent_kernel<BN, KCH, STAGES, MT, MASK, YR>,
                                                               IGP_THREADS, L::TOTAL));
         occ = std::max(1, occ);
     }
     const int per_sm = std::max(1, std::min<int>(std::min(2, 512 / (2 * MT * BN)), occ));
     const int grid = (int)std::min<long long>(tiles, 148LL * per_sm);
-    igemm_persistent_kernel<BN, KCH, STAGES, MT, EXTRA, YR><<<grid, IGP_THREADS, L::TOTAL, st>>>(p, classes);
+    igemm_persistent_kernel<BN, KCH, STAGES, MT, MASK, YR><<<grid, IGP_THREADS, L::TOTAL, st>>>(p, classes);
     LAUNCH_OK();
     return 0;
 }
 template <int BN, int KCH, int STAGES, int MT, bool YR = false>
 static int launch_ig_persistent(const IgParams& p, int classes, cudaStream_t st) {
-    // the fused BN-backward-sums / ReLU-mask epilogues live in their own instantiation (register pressure of the common case)
-    if (p.bnb_x) return launch_ig_persistent_x<BN, KCH, STAGES, MT, 2, YR>(p, classes, st);
-    if (p.mask_y || p.mask_bits) return launch_ig_persistent_x<BN, KCH, STAGES, MT, 1, YR>(p, classes, st);
-    return launch_ig_persistent_x<BN, KCH, STAGES, MT, 0, YR>(p, classes, st);
+    // the fused ReLU-mask epilogue lives in its own instantiation (register pressure of the common case)
+    if (p.mask_y || p.mask_bits) return launch_ig_persistent_x<BN, KCH, STAGES, MT, true, YR>(p, classes, st);
+    return launch_ig_persistent_x<BN, KCH, STAGES, MT, false, YR>(p, classes, st);
 }
 static bool g_last_ig_was_persistent = false;  // set by dispatch_ig (host-thread confined, like g_launches)
-static int g_ig_persistent = 1;  // FMRI_IGEMM_PERSISTENT=0 selects the one-tile-per-CTA kernel (A/B comparison)
 static int dispatch_ig_persistent(const IgParams& p_in, int BN, int KCH, int classes, cudaStream_t st) {
-    static int legacy = -1;
-    if (legacy < 0) {
-        const char* e = getenv("FMRI_IG_PRODUCER");
-        legacy = (e && atoi(e) == 0) ? 1 : 0;
-    }
     IgParams p = p_in;
-    p.legacy_producer = legacy;
     if (p.stat_sum && p.out_fp32) return fail(FMRI_ERR_UNSUPPORTED, "fused column statistics need a bf16 output");
     static int skip = -1;
     if (skip < 0) {
@@ -206,15 +198,16 @@ static int dispatch_ig_persistent(const IgParams& p_in, int BN, int KCH, int cla
         skip = e ? atoi(e) : 0;
     }
     p.skip = skip;
-    static int pair = -1;
-    if (pair < 0) {
+    static int force_pair = -1;
+    if (force_pair < 0) {
         const char* e = getenv("FMRI_IG_PAIR");
-        pair = e ? atoi(e) : 1;
+        force_pair = (e && atoi(e) == 2) ? 1 : 0;
     }
-    // measured per form (scripts/igemm_probe.py, FMRI_IG_PAIR=0/1): 128-byte-line stores take 11 % off the BN = 128 gathers
-    // (two-pass staging hides behind their short K loop) but cost 5-7 % on the parity-merged scatter and on BN = 256,
-    // where holding two chunks before the first store lengthens the epilogue's critical path; 2 = force everywhere (tests)
-    p.pair = (pair == 2 || (pair && !p.merge && BN == 128)) ? 1 : 0;
+    // measured per form (scripts/igemm_probe.py, with and without pairs): 128-byte-line stores take 11 % off the BN = 128
+    // gathers (two-pass staging hides behind their short K loop) but cost 5-7 % on the parity-merged scatter and on BN = 256,
+    // where holding two chunks before the first store lengthens the epilogue's critical path; FMRI_IG_PAIR=2 forces them
+    // everywhere (tests)
+    p.pair = (force_pair || (!p.merge && BN == 128)) ? 1 : 0;
     if (p.yr) {   // row-reuse gather (run_gather decided; two M sub-tiles = 8 output rows of one image)
         if (KCH == 32 && BN == 128) return launch_ig_persistent<128, 32, 4, 2, true>(p, classes, st);
         if (KCH == 32 && BN == 64) return launch_ig_persistent<64, 32, 3, 2, true>(p, classes, st);
@@ -238,14 +231,13 @@ static int dispatch_ig_persistent(const IgParams& p_in, int BN, int KCH, int cla
     return fail(FMRI_ERR_UNSUPPORTED, "persistent igemm tile BN=%d KCH=%d not instantiated", BN, KCH);
 }
 static bool ig_goes_persistent(const IgParams& p, int classes) {
-    static bool env_done = false;
-    if (!env_done) {
+    static int force = -1;   // FMRI_IGEMM_PERSISTENT=2: the persistent kernel for every launch, however small (tests)
+    if (force < 0) {
         const char* e = getenv("FMRI_IGEMM_PERSISTENT");
-        if (e) g_ig_persistent = atoi(e);
-        env_done = true;
+        force = (e && atoi(e) == 2) ? 1 : 0;
     }
     const long long all = (long long)p.tiles_x * p.tiles_y * p.tiles_n * p.n_tiles * classes;
-    return g_ig_persistent && p.splits == 1 && (all >= 2 * 148 || g_ig_persistent == 2);  // 2: always (tests)
+    return p.splits == 1 && (all >= 2 * 148 || force);
 }
 static int dispatch_ig(const IgParams& p, int BN, int KCH, int classes, cudaStream_t st) {
     {
@@ -299,26 +291,14 @@ static void pick_box_pow2(int X, int Y, int N, int* bw, int* bh, int* bn) {
 
 // Gather-form plan: out[n,oy,ox,:] = sum_taps X[n, oy*s+kh-2, ox*s+kw-2, :] * pack[tap]
 // (Conv2d fprop; ConvTranspose2d dgrad). X: [N,H,W,Ck] bf16, out: [N,OH,OW,Ng].
-struct BnbFuse {  // fused BatchNorm-backward statistics of the layer whose dy this data gradient produces
-    const void* x;
-    const float *mean, *invstd, *gamma, *beta;
-    int relu;
-    const void* mask_y = nullptr;  // instead: ReLU-backward mask of a bias+ReLU layer (no BatchNorm), see fmri_bn_fuse
-    const unsigned* mask_bits = nullptr;  // the same mask as a bit word per 32-channel pixel (fmri_relu_bitmask)
-};
-static void apply_fuse(IgParams& p, const BnbFuse* f) {
-    if (!f) return;
-    if (f->mask_y) {
-        p.mask_y = f->mask_y;
-        p.mask_bits = f->mask_bits;
-        return;
-    }
-    p.bnb_x = f->x; p.bnb_mean = f->mean; p.bnb_invstd = f->invstd; p.bnb_gamma = f->gamma; p.bnb_beta = f->beta;
-    p.bnb_relu = f->relu;
+static void apply_mask(IgParams& p, const fmri_relu_mask* m) {   // ReLU backward in the epilogue, see fmri_relu_mask
+    if (!m) return;
+    p.mask_y = m->y;
+    p.mask_bits = m->bits;
 }
 static int run_gather(const void* X, int N, int H, int W, int Ck, int OH, int OW, int Ng, int stride, const void* pack,
                       const float* bias, int act, void* out, int out_fp32, double* ssum, double* ssq,
-                      cudaStream_t st, const BnbFuse* fuse = nullptr) {
+                      cudaStream_t st, const fmri_relu_mask* mask = nullptr) {
     if (Ck % 32 || Ng % 32) return fail(FMRI_ERR_UNSUPPORTED, "tensor path needs channels %% 32 == 0 (%d,%d)", Ck, Ng);
     const int KCH = (Ck % 64 == 0) ? 64 : 32;
     IgParams p;
@@ -334,12 +314,7 @@ static int run_gather(const void* X, int N, int H, int W, int Ck, int OH, int OW
     // row reuse (IgSmem YR): thin K side, 32-pixel output rows, two vertically adjacent sub-tiles per CTA
     p.n_tiles = Ng / BN;
     p.splits = 1;
-    static int yr_env = -1;
-    if (yr_env < 0) {
-        const char* e = getenv("FMRI_IG_YR");
-        yr_env = (e && atoi(e) == 0) ? 0 : 1;
-    }
-    const bool yr = yr_env && stride == 2 && Ck == 32 && p.bw == 32 && p.bh == 4 && p.bn == 1 && OW == 32 && OH % 8 == 0 &&
+    const bool yr = stride == 2 && Ck == 32 && p.bw == 32 && p.bh == 4 && p.bn == 1 && OW == 32 && OH % 8 == 0 &&
                     (BN == 64 || BN == 128) && ig_goes_persistent(p, 1);
     p.yr = yr ? 1 : 0;
     const int box_h = yr ? 2 * p.bh + 2 : p.bh;
@@ -396,19 +371,20 @@ static int run_gather(const void* X, int N, int H, int W, int Ck, int OH, int OW
     p.act = act;
     p.stat_sum = ssum;
     p.stat_sq = ssq;
-    apply_fuse(p, fuse);
+    apply_mask(p, mask);
     return dispatch_ig(p, BN, KCH, 1, st);
 }
 
 // Scatter-form plan (stride 2): out[n, 2a+ph, 2b+pw, :] = sum_{kh = ph (mod 2), kw = pw (mod 2)} X[n, a+(ph+2-kh)/2, ..] * pack[tap]
 // (ConvTranspose2d fprop; Conv2d dgrad). X: [N,H,W,Ck], out: [N,OH,OW,Ng] with OH in {2H-1, 2H}.
 static int run_scatter_merged(const void* X, int N, int H, int W, int Ck, int OH, int OW, const void* pack, void* out,
-                              double* ssum, double* ssq, cudaStream_t st, const BnbFuse* fuse, const float* bias, int act);
+                              double* ssum, double* ssq, cudaStream_t st, const fmri_relu_mask* mask, const float* bias,
+                              int act);
 static int run_scatter(const void* X, int N, int H, int W, int Ck, int OH, int OW, int Ng, const void* pack, void* out,
-                       double* ssum, double* ssq, cudaStream_t st, const BnbFuse* fuse = nullptr, const float* bias = nullptr,
-                       int act = 0) {
+                       double* ssum, double* ssq, cudaStream_t st, const fmri_relu_mask* mask = nullptr,
+                       const float* bias = nullptr, int act = 0) {
     if (Ck % 32 || Ng % 32) return fail(FMRI_ERR_UNSUPPORTED, "tensor path needs channels %% 32 == 0 (%d,%d)", Ck, Ng);
-    if (Ng == 32) return run_scatter_merged(X, N, H, W, Ck, OH, OW, pack, out, ssum, ssq, st, fuse, bias, act);
+    if (Ng == 32) return run_scatter_merged(X, N, H, W, Ck, OH, OW, pack, out, ssum, ssq, st, mask, bias, act);
     const int KCH = (Ck % 64 == 0) ? 64 : 32;
     IgParams p;
     memset(&p, 0, sizeof(p));
@@ -461,14 +437,15 @@ static int run_scatter(const void* X, int N, int H, int W, int Ck, int OH, int O
     p.stat_sq = ssq;
     p.bias = bias;
     p.act = act;
-    apply_fuse(p, fuse);
+    apply_mask(p, mask);
     return dispatch_ig(p, BN, KCH, 4, st);
 }
 
 // Parity-merged scatter plan for Ng == 32 (IgParams::merge): one gather over the 3x3 coarse neighbourhood, N = 4 x 32.
 // `pack` is the ordinary tap-major pack [25][32][Ck] followed by the merged pack [9][128][Ck] (fmri_conv_pack_elems).
 static int run_scatter_merged(const void* X, int N, int H, int W, int Ck, int OH, int OW, const void* pack, void* out,
-                              double* ssum, double* ssq, cudaStream_t st, const BnbFuse* fuse, const float* bias, int act) {
+                              double* ssum, double* ssq, cudaStream_t st, const fmri_relu_mask* mask, const float* bias,
+                              int act) {
     const int Ng = 32;
     const int KCH = (Ck % 64 == 0) ? 64 : 32;
     IgParams p;
@@ -499,12 +476,7 @@ static int run_scatter_merged(const void* X, int N, int H, int W, int Ck, int OH
     // Coarse taps, the four full ones first (the first MMA of a tile must initialise every accumulator column). A tap with
     // dy = -1 only feeds the ph = 0 classes and one with dx = -1 only the pw = 0 classes; with the column groups ordered
     // (0,1),(0,0),(1,0),(1,1) (merge_pack_kernel) the live columns are contiguous, and the MMA warp skips the zero slabs:
-    // 4 x 128 + 4 x 64 + 1 x 32 = 800 = 25 x 32 columns per K step instead of 9 x 128 (FMRI_MERGE_SKIP=0 issues full N).
-    static int skip = -1;
-    if (skip < 0) {
-        const char* e = getenv("FMRI_MERGE_SKIP");
-        skip = (e && atoi(e) == 0) ? 0 : 1;
-    }
+    // 4 x 128 + 4 x 64 + 1 x 32 = 800 = 25 x 32 columns per K step instead of 9 x 128.
     static const int order[9] = {4, 5, 7, 8, 1, 2, 3, 6, 0};   // t9 = (dy+1)*3 + (dx+1)
     for (int i = 0; i < 9; ++i) {
         const int t9 = order[i], dy = t9 / 3 - 1, dx = t9 % 3 - 1;
@@ -516,7 +488,7 @@ static int run_scatter_merged(const void* X, int N, int H, int W, int Ck, int OH
         if (dy == -1 && dx == -1) { g0 = 1; ng = 1; }
         else if (dy == -1) { g0 = 0; ng = 2; }
         else if (dx == -1) { g0 = 1; ng = 2; }
-        c.taps[i].ncol = (int16_t)((skip && ng < 4) ? ((ng << 8) | g0) : 0);
+        c.taps[i].ncol = (int16_t)(ng < 4 ? ((ng << 8) | g0) : 0);
     }
     p.num_chunks = Ck / KCH;
     p.n_total = 128;
@@ -536,7 +508,7 @@ static int run_scatter_merged(const void* X, int N, int H, int W, int Ck, int OH
     p.merge_oh = OH;
     p.merge_ow = OW;
     p.merge_sy = (long long)OW * Ng;
-    apply_fuse(p, fuse);
+    apply_mask(p, mask);
     return dispatch_ig(p, BN, KCH, 1, st);
 }
 
@@ -626,14 +598,7 @@ static int wave_splits(long long base, long long max_splits) {
     }
     return (int)best;
 }
-static int dispatch_wg(const WgParams& p_in, int BN, int NCH, cudaStream_t st) {
-    static int merge = -1;
-    if (merge < 0) {
-        const char* e = getenv("FMRI_WG_MERGE");
-        merge = (e && atoi(e) == 0) ? 0 : 1;
-    }
-    WgParams p = p_in;
-    p.merge_taps = merge;
+static int dispatch_wg(const WgParams& p, int BN, int NCH, cudaStream_t st) {
     if (NCH == 64 && BN == 128) return p.num_taps > 1 ? launch_wg<128, 64, 2, 2>(p, st) : launch_wg<128, 64, 3, 1>(p, st);
     if (NCH == 64 && BN == 64) return launch_wg<64, 64, 4, 1>(p, st);
     if (NCH == 32 && BN == 32) return p.num_taps % 5 == 0 ? launch_wg<32, 32, 3, 5>(p, st) : launch_wg<32, 32, 4, 1>(p, st);
@@ -826,72 +791,46 @@ extern "C" int fmri_conv_fprop(const fmri_conv_desc* d, const void* x, const flo
     return 0;
 }
 
-static int bn_bwd_sums(const void* x, int x_dtype, const void* dy, int g_dtype, long long rows, int C, const float* mean,
-                       const float* invstd, const float* gamma, const float* beta, int relu, double* ws, cudaStream_t st);
-
 extern "C" int fmri_conv_dgrad(const fmri_conv_desc* d, const void* dy, const float* w, const void* pack_d, void* dx,
-                               const fmri_bn_fuse* fuse, void* stream) {
+                               const fmri_relu_mask* mask, void* stream) {
     int rc = check_conv(d);
     if (rc) return rc;
+    if (mask && !mask->y) return fail(FMRI_ERR_ARG, "conv dgrad: the ReLU mask needs y");
     int OH, OW;
     fmri_conv_out_hw(d, &OH, &OW);
-    const long long rows_in = (long long)d->N * d->H * d->W;
+    const long long n_in = (long long)d->N * d->H * d->W * d->Cin;
     if (d->dtype == FMRI_BF16) {
         if (!pack_d) return fail(FMRI_ERR_ARG, "bf16 conv dgrad needs the packed weights");
-        BnbFuse bf;
-        double *sg = nullptr, *sgx = nullptr;
-        const bool mask_only = fuse && !fuse->mean;   // ReLU mask of a bias+ReLU layer: dx *= (x > 0)
-        if (mask_only) {
-            bf.x = nullptr; bf.mean = bf.invstd = bf.gamma = bf.beta = nullptr; bf.relu = 1;
-            bf.mask_y = fuse->x;
-            bf.mask_bits = d->Cin == 32 ? fuse->mask_bits : nullptr;   // bit words describe 32-channel pixels only
-        } else if (fuse) {
-            if (d->Cin > 256) return fail(FMRI_ERR_UNSUPPORTED, "fused BN-backward statistics need <= 256 channels");
-            bf.x = fuse->x; bf.mean = fuse->mean; bf.invstd = fuse->invstd; bf.gamma = fuse->gamma; bf.beta = fuse->beta;
-            bf.relu = fuse->relu;
-            sg = fuse->sums;
-            sgx = fuse->sums + d->Cin;
-            CUDA_OK(cudaMemsetAsync(fuse->sums, 0, sizeof(double) * 2 * d->Cin, S(stream)));
+        fmri_relu_mask m;
+        if (mask) {
+            m.y = mask->y;
+            m.bits = d->Cin == 32 ? mask->bits : nullptr;   // bit words describe 32-channel pixels only
         }
         if (d->transposed)  // gather over dy at stride 2
-            rc = run_gather(dy, d->N, OH, OW, d->Cout, d->H, d->W, d->Cin, 2, pack_d, nullptr, 0, dx, 0, sg, sgx, S(stream),
-                            fuse ? &bf : nullptr);
+            rc = run_gather(dy, d->N, OH, OW, d->Cout, d->H, d->W, d->Cin, 2, pack_d, nullptr, 0, dx, 0, nullptr, nullptr,
+                            S(stream), mask ? &m : nullptr);
         else if (d->stride == 2)
-            rc = run_scatter(dy, d->N, OH, OW, d->Cout, d->H, d->W, d->Cin, pack_d, dx, sg, sgx, S(stream),
-                             fuse ? &bf : nullptr);
+            rc = run_scatter(dy, d->N, OH, OW, d->Cout, d->H, d->W, d->Cin, pack_d, dx, nullptr, nullptr, S(stream),
+                             mask ? &m : nullptr);
         else
             return fail(FMRI_ERR_UNSUPPORTED, "stride-1 conv dgrad on the tensor path");
         if (rc) return rc;
-        if (mask_only) {
-            if (!g_last_ig_was_persistent) {  // small launch (one tile per CTA kernel, no fused mask): mask dx in place
-                const long long n = rows_in * d->Cin;
-                relu_bwd_kernel<__nv_bfloat16><<<grid1d((n + 7) / 8, 256, 148 * 8), 256, 0, S(stream)>>>(
-                    reinterpret_cast<const __nv_bfloat16*>(fuse->x), reinterpret_cast<const __nv_bfloat16*>(dx),
-                    reinterpret_cast<__nv_bfloat16*>(dx), n);
-                LAUNCH_OK();
-            }
-            return 0;
-        }
-        if (fuse && !g_last_ig_was_persistent) {
-            // small launch (one tile per CTA kernel): that epilogue produced plain sum(dx) / sum(dx^2); redo the sums properly
-            return bn_bwd_sums(fuse->x, FMRI_BF16, dx, FMRI_BF16, rows_in, d->Cin, fuse->mean, fuse->invstd, fuse->gamma,
-                               fuse->beta, fuse->relu, fuse->sums, S(stream));
+        if (mask && !g_last_ig_was_persistent) {  // small launch (one tile per CTA kernel, no fused mask): mask dx in place
+            relu_bwd_kernel<__nv_bfloat16><<<grid1d((n_in + 7) / 8, 256, 148 * 8), 256, 0, S(stream)>>>(
+                reinterpret_cast<const __nv_bfloat16*>(mask->y), reinterpret_cast<const __nv_bfloat16*>(dx),
+                reinterpret_cast<__nv_bfloat16*>(dx), n_in);
+            LAUNCH_OK();
         }
         return 0;
     }
     rc = direct_conv<float>(d, true, reinterpret_cast<const float*>(dy), w, nullptr, 0, reinterpret_cast<float*>(dx),
                             S(stream));
     if (rc) return rc;
-    if (fuse && !fuse->mean) {
-        const long long n = rows_in * d->Cin;
-        relu_bwd_kernel<float><<<grid1d((n + 7) / 8, 256, 148 * 8), 256, 0, S(stream)>>>(
-            reinterpret_cast<const float*>(fuse->x), reinterpret_cast<const float*>(dx), reinterpret_cast<float*>(dx), n);
+    if (mask) {
+        relu_bwd_kernel<float><<<grid1d((n_in + 7) / 8, 256, 148 * 8), 256, 0, S(stream)>>>(
+            reinterpret_cast<const float*>(mask->y), reinterpret_cast<const float*>(dx), reinterpret_cast<float*>(dx), n_in);
         LAUNCH_OK();
-        return 0;
     }
-    if (fuse)
-        return bn_bwd_sums(fuse->x, FMRI_F32, dx, FMRI_F32, rows_in, d->Cin, fuse->mean, fuse->invstd, fuse->gamma, fuse->beta,
-                           fuse->relu, fuse->sums, S(stream));
     return 0;
 }
 
@@ -1076,21 +1015,13 @@ static bool hc_build(HcParams& p, HcPackSpec& spec, int N, int H, int W, int chu
 
 template <int BN>
 static int hc_launch(const HcParams& p_in, cudaStream_t st) {
-    static int issuers = 0;
-    if (!issuers) {
-        const char* e = getenv("FMRI_HC_ISSUERS");
-        issuers = e ? std::max(1, std::min(HC_ISSUERS, atoi(e))) : HC_ISSUERS;
-    }
     HcParams p = p_in;
-    p.issuers_max = issuers;
-    {
-        static int skip = -1;
-        if (skip < 0) {
-            const char* e = getenv("FMRI_HC_SKIP");
-            skip = e ? atoi(e) : 0;
-        }
-        p.skip = skip;
+    static int skip = -1;
+    if (skip < 0) {
+        const char* e = getenv("FMRI_HC_SKIP");
+        skip = e ? atoi(e) : 0;
     }
+    p.skip = skip;
     const int smem = hc_smem_bytes(p, BN);
     static int attr_smem = 0;
     if (smem > attr_smem) {
@@ -1125,12 +1056,7 @@ static int hc_run(HcParams& p, const HcPackSpec& spec, int BN, const float* w, i
 // to give every SM whole images. Returns 1 when the shape does not fit (caller falls back to the halo-tile kernel).
 static int cto3_run(const void* X, int N, int H, int W, int C, const float* w, long long s_co, long long s_c, int flip,
                     const float* bias, int act, float* img, void* ws, cudaStream_t st) {
-    static int enabled = -1;
-    if (enabled < 0) {
-        const char* e = getenv("FMRI_CTO3");
-        enabled = (e && atoi(e) == 0) ? 0 : 1;
-    }
-    if (!enabled || C != 32 || W != C3_W || H < 3 || N < 74) return 1;
+    if (C != 32 || W != C3_W || H < 3 || N < 74) return 1;
     C3Params p;
     memset(&p, 0, sizeof(p));
     __nv_bfloat16* wt = reinterpret_cast<__nv_bfloat16*>(ws);
@@ -1192,16 +1118,10 @@ static int hconv_3_to_c(const float* i0, const float* i1, const float* i2, int n
 // Edge-conv weight gradient on tcgen05 (hwgrad_kernels.cuh), stride 1. T: [N,PH,PW,C] bf16 NHWC; the 3-channel side comes as
 // up to three fp32 NCHW sources and is repacked to NHWC-8 in the workspace. dwk: fp32 [75][C] (zeroed by the caller).
 // Returns 1 when the shape does not fit (caller falls back to the CUDA-core kernel).
-static int g_hw_variant = -1;
 // plane < 0: stride-1 convolution (images packed here). plane = ph * 2 + pw: one stride-parity plane of a stride-2 convolution --
 // (IH, IW) is the image, (PH, PW) the T grid = the conv output; see HwParams::plane.
 static int hwgrad_run(const void* T, const float* i0, const float* i1, const float* i2, int nps, int N, int PH, int PW, int C,
                       float* dwk, float* dbias, int flip, void* ws, cudaStream_t st, int plane = -1, int IH = 0, int IW = 0) {
-    if (g_hw_variant < 0) {
-        const char* e = getenv("FMRI_HWGRAD");   // -1/unset: default variant 0; 0/1: descriptor variant; 2: disable
-        g_hw_variant = e ? atoi(e) : 0;
-    }
-    if (g_hw_variant == 2) return 1;
     if (C != 32 && C != 64) return 1;
     HwParams p;
     memset(&p, 0, sizeof(p));
@@ -1209,13 +1129,9 @@ static int hwgrad_run(const void* T, const float* i0, const float* i1, const flo
     p.PWp = (PW + 4 + 15) / 16 * 16;
     if (p.PWp > 128) return 1;
     // tile rows: every tile re-stages bh + 4 image rows for bh output rows, so taller tiles cut the halo traffic that bounds
-    // this kernel reads (5x at bh = 1, 3x at 2, 2.3x at 3) -- which turned out NOT to be its bound; rows = bh * PWp <= 256 (ones slab). A ragged last tile is fine: TMA
-    // zero-fills the T rows below the image. FMRI_HW_BH caps bh (A/B switch).
-    static int bh_cap = 0;
-    if (!bh_cap) {
-        const char* e = getenv("FMRI_HW_BH");
-        bh_cap = e ? std::max(1, atoi(e)) : 2;  // measured: bh = 2 is 0-3 % faster than 1; bh = 3 needs one CTA per SM and is 10 % slower
-    }
+    // this kernel reads (5x at bh = 1, 3x at 2, 2.3x at 3) -- which turned out NOT to be its bound; rows = bh * PWp <= 256
+    // (ones slab). A ragged last tile is fine: TMA zero-fills the T rows below the image.
+    const int bh_cap = 2;  // measured: bh = 2 is 0-3 % faster than 1; bh = 3 needs one CTA per SM and is 10 % slower
     p.bh = std::max(1, std::min(std::min(PH, bh_cap), 256 / p.PWp));
     p.tiles_y = cdiv(PH, p.bh);
     p.slab_rows = ((p.bh + 4) * p.PWp + 16 + 7) / 8 * 8;
@@ -1242,7 +1158,7 @@ static int hwgrad_run(const void* T, const float* i0, const float* i1, const flo
     }
     LAUNCH_OK();
     p.img8 = img8;
-    p.dwk = dwk; p.dbias = dbias; p.flip = flip; p.desc_variant = g_hw_variant;
+    p.dwk = dwk; p.dbias = dbias; p.flip = flip;
     const int smem = hw_smem_bytes(p);
     static int attr_smem = 0;
     if (smem > attr_smem) {
@@ -1694,27 +1610,13 @@ static int bn_bwd_reduce_t(const void* x, const void* dy, long long rows, int C,
     LAUNCH_OK();
     return 0;
 }
-static int bn_bwd_sums(const void* x, int x_dtype, const void* dy, int g_dtype, long long rows, int C, const float* mean,
-                       const float* invstd, const float* gamma, const float* beta, int relu, double* ws, cudaStream_t st) {
-    if (C < 256 && (256 % C)) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward C=%d", C);
-    if (x_dtype == FMRI_BF16 && g_dtype == FMRI_BF16)
-        return bn_bwd_reduce_t<__nv_bfloat16, __nv_bfloat16>(x, dy, rows, C, mean, invstd, gamma, beta, relu, ws, st);
-    if (x_dtype == FMRI_F32 && g_dtype == FMRI_BF16)
-        return bn_bwd_reduce_t<float, __nv_bfloat16>(x, dy, rows, C, mean, invstd, gamma, beta, relu, ws, st);
-    if (x_dtype == FMRI_F32 && g_dtype == FMRI_F32)
-        return bn_bwd_reduce_t<float, float>(x, dy, rows, C, mean, invstd, gamma, beta, relu, ws, st);
-    return fail(FMRI_ERR_UNSUPPORTED, "bn_backward dtype combination");
-}
 template <typename Tx, typename Tg>
 static int bn_bwd_t(const void* x, const void* dy, void* dx, long long rows, int C, const float* mean,
                     const float* invstd, const float* gamma, const float* beta, int relu, int train, float* dgamma,
-                    float* dbeta, int accumulate, double* ws, int sums_ready, cudaStream_t st, long long row0 = 0,
-                    long long nrows = -1) {
+                    float* dbeta, int accumulate, double* ws, cudaStream_t st, long long row0 = 0, long long nrows = -1) {
     // [row0, row0 + nrows): the rows dx is produced for (dx points at the first of them); the sums always run over all rows
-    if (!sums_ready) {
-        int rc = bn_bwd_reduce_t<Tx, Tg>(x, dy, rows, C, mean, invstd, gamma, beta, relu, ws, st);
-        if (rc) return rc;
-    }
+    int rc = bn_bwd_reduce_t<Tx, Tg>(x, dy, rows, C, mean, invstd, gamma, beta, relu, ws, st);
+    if (rc) return rc;
     float* mean_g = reinterpret_cast<float*>(ws + 2 * C);  // third C doubles of the workspace: 2C floats
     float* mean_gx = mean_g + C;
     bn_param_grad_kernel<<<cdiv(C, 128), 128, 0, st>>>(ws, ws + C, (double)rows, C, mean_g, mean_gx, dgamma, dbeta, accumulate);
@@ -1749,35 +1651,34 @@ static int bn_bwd_t(const void* x, const void* dy, void* dx, long long rows, int
 }
 extern "C" int fmri_bn_backward(const void* x, int x_dtype, const void* dy, void* dx, int g_dtype, long long rows, int C,
                                 const float* mean, const float* invstd, const float* gamma, const float* beta,
-                                int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws,
-                                int sums_ready, void* stream) {
+                                int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws, void* stream) {
     if (C < 256 && (256 % C)) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward C=%d", C);
     if (x_dtype == FMRI_BF16 && g_dtype == FMRI_BF16)
         return bn_bwd_t<__nv_bfloat16, __nv_bfloat16>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train,
-                                                      dgamma, dbeta, accumulate, ws, sums_ready, S(stream));
+                                                      dgamma, dbeta, accumulate, ws, S(stream));
     if (x_dtype == FMRI_F32 && g_dtype == FMRI_BF16)
         return bn_bwd_t<float, __nv_bfloat16>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train, dgamma, dbeta,
-                                              accumulate, ws, sums_ready, S(stream));
+                                              accumulate, ws, S(stream));
     if (x_dtype == FMRI_F32 && g_dtype == FMRI_F32)
         return bn_bwd_t<float, float>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train, dgamma, dbeta,
-                                      accumulate, ws, sums_ready, S(stream));
+                                      accumulate, ws, S(stream));
     return fail(FMRI_ERR_UNSUPPORTED, "bn_backward dtype combination");
 }
 extern "C" int fmri_bn_backward_slice(const void* x, int x_dtype, const void* dy, void* dx, int g_dtype, long long rows,
                                       long long row0, long long nrows, int C, const float* mean, const float* invstd,
                                       const float* gamma, const float* beta, int relu, int train, float* dgamma,
-                                      float* dbeta, int accumulate, double* ws, int sums_ready, void* stream) {
+                                      float* dbeta, int accumulate, double* ws, void* stream) {
     if (C < 256 && (256 % C)) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward C=%d", C);
     if (row0 < 0 || nrows < 0 || row0 + nrows > rows) return fail(FMRI_ERR_ARG, "bn_backward_slice: bad row range");
     if (x_dtype == FMRI_BF16 && g_dtype == FMRI_BF16)
         return bn_bwd_t<__nv_bfloat16, __nv_bfloat16>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train,
-                                                      dgamma, dbeta, accumulate, ws, sums_ready, S(stream), row0, nrows);
+                                                      dgamma, dbeta, accumulate, ws, S(stream), row0, nrows);
     if (x_dtype == FMRI_F32 && g_dtype == FMRI_BF16)
         return bn_bwd_t<float, __nv_bfloat16>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train, dgamma, dbeta,
-                                              accumulate, ws, sums_ready, S(stream), row0, nrows);
+                                              accumulate, ws, S(stream), row0, nrows);
     if (x_dtype == FMRI_F32 && g_dtype == FMRI_F32)
         return bn_bwd_t<float, float>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train, dgamma, dbeta,
-                                      accumulate, ws, sums_ready, S(stream), row0, nrows);
+                                      accumulate, ws, S(stream), row0, nrows);
     return fail(FMRI_ERR_UNSUPPORTED, "bn_backward dtype combination");
 }
 extern "C" int fmri_relu_backward(const void* y, const void* dy, void* dx, int dtype, long long n, void* stream) {

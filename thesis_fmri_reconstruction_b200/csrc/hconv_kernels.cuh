@@ -42,7 +42,8 @@ struct HcParams {
     int pl_ys[4], pl_xs[4];      // input step per halo row / column (1, or 2 for stride-parity planes)
     int pl_yoff[4], pl_xoff[4];  // input y of halo row sy is (oy0 + sy) * ys + yoff, likewise x
     int PW, PH;                  // halo tile width / height (pixels)
-    int issuers_max;             // active MMA-issuing warps (<= HC_ISSUERS; A/B switch FMRI_HC_ISSUERS)
+    int skip;                    // diagnostic (FMRI_HC_SKIP): bit 0 producers skip the halo copies, bit 1 epilogue skips its global
+                                 // stores, bit 2 issuers skip the MMAs -- which role bounds the kernel (results are garbage)
     int slab_rows;               // allocated rows per slab (>= halo rows; 2 mod 8 when there are several channel chunks)
     int num_steps;
     HcStep steps[HC_MAX_STEPS];
@@ -55,8 +56,6 @@ struct HcParams {
     const float* bias;           // [n_out] / [BN] or null
     int act;
     int n_out;
-    int skip;                    // diagnostic (FMRI_HC_SKIP): bit 0 producers skip the halo copies, bit 1 epilogue skips its global
-                                 // stores, bit 2 issuers skip the MMAs -- which role bounds the kernel (results are garbage)
 };
 
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, uint32_t src_bytes) {
@@ -117,8 +116,7 @@ __global__ void __launch_bounds__(HC_THREADS, 2) hconv_kernel(const __grid_const
     if (threadIdx.x < 64) s_bias[threadIdx.x] = (p.bias && p.epi == 1 && (int)threadIdx.x < BN) ? p.bias[threadIdx.x] : 0.f;
     const int total_tiles = p.N * p.tiles_y;
     const int acc_cols = p.MT * BN;  // TMEM columns of one accumulator buffer
-    const int issuers_cap = p.issuers_max < HC_ISSUERS ? p.issuers_max : HC_ISSUERS;
-    const int issuers = p.MT < issuers_cap ? p.MT : issuers_cap;
+    const int issuers = p.MT < HC_ISSUERS ? p.MT : HC_ISSUERS;
     uint32_t tmem_cols = 32;
     while ((int)tmem_cols < 2 * acc_cols) tmem_cols <<= 1;
 

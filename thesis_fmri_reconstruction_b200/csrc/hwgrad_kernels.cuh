@@ -30,7 +30,6 @@ struct HwParams {
     float* dwk;                  // [75][C] fp32, +=
     float* dbias;                // [C] fp32 += sum_p T[p][c], nullable
     int flip;                    // write tap 24-tap (C -> 3 conv: T is the conv input, img the output gradient)
-    int desc_variant;            // B descriptor stride assignment (see kernel)
     int stages;                  // pipeline depth (<= HW_MAX_STAGES): the tiles are small, so depth hides the L2 latency
     int d_chunk;                 // bytes between the two 64-channel chunks of an A stage (rows*128 rounded up to 1 KB)
     // Stride-2 convolutions run as four launches, one per input parity plane (ph, pw): img8 then holds the plane
@@ -116,7 +115,7 @@ __global__ void __launch_bounds__(HW_THREADS) hwgrad_kernel(const __grid_constan
         const uint32_t idesc1 = umma_idesc_bf16(64, 16, true, true);
         const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
         // B (image slab, MN-major, no swizzle): 16-byte N chunks one slab row apart; K advances in 8-pixel groups of 128 B.
-        const uint32_t b_lbo = p.desc_variant ? 16 : 128, b_sbo = p.desc_variant ? 128 : 16;
+        constexpr uint32_t b_lbo = 128, b_sbo = 16;
         const int ksteps = rows / 16;
         int it = 0;
         for (int t = blockIdx.x; t < total_tiles; t += gridDim.x, ++it) {

@@ -61,24 +61,13 @@ struct IgParams {
     const void* mask_y;     // persistent kernel, bf16 output: zero the output where this bf16 tensor (same layout) is <= 0
                             // (ReLU backward of a bias+ReLU layer fused into the data-gradient epilogue)
     const uint32_t* mask_bits;  // same mask as 1 bit per element of a 32-channel pixel (bits[(offset) >> 5]); preferred over mask_y
-    int legacy_producer;    // persistent kernel: 1 = single-lane TMA producer (A/B switch), 0 = warp-converged elected issue
     int yr;                 // persistent kernel, row-reuse gather (see IgSmem): mapA[plane] boxes are MT*bh+2 rows tall
-    int pair;               // persistent kernel: 128-byte-line stores through chunk pairs (A/B switch FMRI_IG_PAIR, default on)
+    int pair;               // persistent kernel: 128-byte-line stores through chunk pairs (dispatch_ig_persistent decides)
     int skip;               // diagnostic (FMRI_IG_SKIP, persistent kernel): bit 0 the producer issues no TMA loads, bit 1 the
                             // epilogue does nothing but hand the accumulators back, bit 2 no MMAs are issued, bit 3 the
                             // epilogue skips only its global stores -- which role bounds a launch (results are garbage)
     int merge_oh, merge_ow; // fine output extent
     long long merge_sy;     // fine row stride (elements)
-    // Fused BatchNorm-backward statistics (persistent kernel, bf16 output): when this launch is the data gradient that
-    // produces dy for a BN(+ReLU) layer, the epilogue also accumulates, per channel, sum(g) and sum(g * xhat) into
-    // stat_sum / stat_sq, with g = the stored dy masked by the forward ReLU and xhat from that layer's pre-BN tensor bnb_x
-    // (same layout as `out`). This removes the separate reduction pass of BN backward (2 of its 5 tensor passes).
-    const void* bnb_x;
-    const float* bnb_mean;
-    const float* bnb_invstd;
-    const float* bnb_gamma;
-    const float* bnb_beta;
-    int bnb_relu;
 };
 
 // MT = number of 128-row M sub-tiles one CTA accumulates against the SAME B (weight) tile: the kernels are bound by
@@ -88,10 +77,10 @@ struct IgParams {
 // filter column read the SAME stride-parity plane shifted by whole rows, so ONE tall box of MT*4+2 rows x 32 pixels per
 // (kw, py) feeds up to three taps: tap i of sub-tile m starts (4m + i) rows (= a multiple of the swizzle period) into the
 // box. 10 boxes of 10 rows instead of 25 x 8 rows: the activation bytes per tile halve, the weights are fetched as before.
-// EXTRA / PERS: what the persistent kernel adds behind the stage ring -- the [4][256] BatchNorm-backward coefficients of its
-// EXTRA instantiations, and a 2 KB per epilogue warp staging buffer through which bf16 output rows are re-ordered into
-// full 32-byte sectors before they are stored (dropped where it does not fit beside four stages, BN = 256 + EXTRA).
-template <int BN, int KCH, int STAGES, int MT = 1, bool YR = false, int EXTRA = 0, bool PERS = false>
+// PERS: what the persistent kernel adds behind the stage ring -- a 2 KB per epilogue warp staging buffer through which bf16
+// output rows are re-ordered into full 32-byte sectors before they are stored (dropped where it does not fit beside four
+// stages, BN = 256).
+template <int BN, int KCH, int STAGES, int MT = 1, bool YR = false, bool PERS = false>
 struct IgSmem {
     static constexpr int A_SUB = 128 * KCH * 2;
     static constexpr int A_BYTES = YR ? (MT * 4 + 2) * 32 * KCH * 2 : MT * A_SUB;
@@ -101,9 +90,7 @@ struct IgSmem {
     static constexpr int BAR_OFF = STAGES * STAGE_BYTES;
     static constexpr int STAT_OFF = BAR_OFF + (2 * STAGES + 4) * 8 + 16;
     static constexpr int STAT_SLOTS = 8;                        // persistent kernel: one private [2][BN] slot per epilogue warp
-    static constexpr int BNP_OFF = STAT_OFF + STAT_SLOTS * 2 * BN * 4;  // [4][256] BN-backward coefficients (mean, scale, beta, invstd)
-    static constexpr int BNP_BYTES = (EXTRA == 2 || !PERS) ? 4 * 256 * 4 : 0;
-    static constexpr int STG_OFF = (BNP_OFF + BNP_BYTES + 127) & ~127;
+    static constexpr int STG_OFF = (STAT_OFF + STAT_SLOTS * 2 * BN * 4 + 127) & ~127;
     static constexpr int STG_BYTES = (PERS && STG_OFF + 8 * 2048 + 1024 <= 227 * 1024) ? 8 * 2048 : 0;
     static constexpr int TOTAL = STG_OFF + STG_BYTES + 1024;  // +1024: manual base alignment
 };
@@ -416,12 +403,11 @@ __device__ __forceinline__ IgTile ig_decode_tile(const IgParams& p, int t, int m
 constexpr int IGP_EPI_WARPS = 8;
 constexpr int IGP_THREADS = 64 + 32 * IGP_EPI_WARPS;
 
-// EXTRA = 1: the fused ReLU-mask epilogue is compiled in; EXTRA = 2: also the fused BatchNorm-backward sums (which keep the
-// register-accumulated statistics path and its 64 accumulators); the plain
-// instantiation keeps them out of the register allocation of the common case (the epilogue sits at the 168-register cap).
-template <int BN, int KCH, int STAGES, int MT, int EXTRA = 0, bool YR = false>
+// MASK: the fused ReLU-mask epilogue is compiled in; the plain instantiation keeps it out of the register allocation of the
+// common case (the epilogue sits at the 168-register cap).
+template <int BN, int KCH, int STAGES, int MT, bool MASK = false, bool YR = false>
 __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __grid_constant__ IgParams p, int num_classes) {
-    using L = IgSmem<BN, KCH, STAGES, MT, YR, EXTRA, true>;
+    using L = IgSmem<BN, KCH, STAGES, MT, YR, true>;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + L::BAR_OFF);
@@ -454,17 +440,6 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
     }
     if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
     for (int i = threadIdx.x; i < L::STAT_SLOTS * 2 * BN; i += blockDim.x) s_stat[i] = 0.f;
-    float* s_bnp = reinterpret_cast<float*>(smem + L::BNP_OFF);
-    if (EXTRA == 2 && p.bnb_x) {
-        const int nch = p.merge ? 32 : p.n_total;  // channels of the BN layer (<= 256)
-        for (int i = threadIdx.x; i < nch; i += blockDim.x) {
-            const float is = p.bnb_invstd[i];
-            s_bnp[i] = p.bnb_mean[i];
-            s_bnp[256 + i] = p.bnb_gamma[i] * is;
-            s_bnp[512 + i] = p.bnb_beta[i];
-            s_bnp[768 + i] = is;
-        }
-    }
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -497,38 +472,7 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
                                           ((py + 2 * i) * 5 + kw) * p.n_total + brow0);
                 }
             }
-        } else
-        if (p.legacy_producer) {   // single-lane producer (A/B switch FMRI_IG_PRODUCER=0)
-            if (lane == 0) {
-                int it = 0;
-                for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
-                    const IgTile tl = ig_decode_tile<MT>(p, t, m_groups);
-                    if (!tl.any) continue;
-                    const TapClass& c = p.cls[tl.cls];
-                    int nlive = 0;
-#pragma unroll
-                    for (int m = 0; m < MT; ++m) nlive += tl.live[m] ? 1 : 0;
-                    const int nks = c.num_taps * p.num_chunks;
-                    for (int ks = 0; ks < nks; ++ks, ++it) {
-                        const int st = it % STAGES;
-                        const uint32_t ph = (it / STAGES) & 1;
-                        mbar_wait(&empty_bar[st], ph ^ 1);
-                        mbar_arrive_expect_tx(&full_bar[st], nlive * p.a_bytes + L::B_BYTES);
-                        const int tap = ks / p.num_chunks;
-                        const int ch = ks - tap * p.num_chunks;
-                        const TapDesc td = c.taps[tap];
-                        uint8_t* sa = smem + st * L::STAGE_BYTES;
-#pragma unroll
-                        for (int m = 0; m < MT; ++m)
-                            if (tl.live[m])
-                                tma_load_4d(sa + m * L::A_SUB, &p.mapA[td.map], &full_bar[st], ch * KCH, tl.x0[m] + td.dx,
-                                            tl.y0[m] + td.dy, tl.n0[m]);
-                        tma_load_2d(sa + L::A_BYTES, &p.mapB, &full_bar[st], ch * KCH, td.brow + tl.nt * BN);
-                    }
-                }
-            }
-        } else
-        {
+        } else {
             int it = 0;
             for (int t = blockIdx.x; t < total_tiles; t += gridDim.x) {
                 const IgTile tl = ig_decode_tile<MT>(p, t, m_groups);
@@ -649,7 +593,7 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
         const uint32_t stage_u32 = smem_u32(smem + L::STG_OFF) + (warp - 2) * 2048;   // this warp's store staging (2 KB)
         // BatchNorm statistics of the stored values: with the staging buffer a lane reads ONE COLUMN of the staged chunk
         // (32 two-byte loads, conflict-free) -- no 2 x 32 per-thread accumulators, no transposing shuffle reduction
-        constexpr bool SMEM_STATS = (L::STG_BYTES > 0) && EXTRA != 2;
+        constexpr bool SMEM_STATS = L::STG_BYTES > 0;
         // per-channel sums of the tiles processed so far wait in the warps' shared-memory slots and go to the fp64 global
         // accumulators every 16 tiles (or when the column block changes): two named barriers + BN atomics per flush
         int stat_nt = -1, stat_cnt = 0;
@@ -731,7 +675,7 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
                             }
                             addr = off + c0;
                             uint32_t mbits = 0xffffffffu;
-                            if (EXTRA >= 1 && p.mask_bits && valid) mbits = __ldg(p.mask_bits + (addr >> 5));
+                            if (MASK && p.mask_bits && valid) mbits = __ldg(p.mask_bits + (addr >> 5));
                             uint32_t v[32];
                             tmem_ld32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * ACC_COLS + m * BN + c0, v);
                             tmem_ld_wait();
@@ -753,11 +697,11 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
 #pragma unroll
                                 for (int j = 0; j < 32; ++j) f[j] = 1.f / (1.f + __expf(-f[j]));
                             }
-                            if (EXTRA >= 1 && p.mask_bits) {
+                            if (MASK && p.mask_bits) {
 #pragma unroll
                                 for (int j = 0; j < 32; ++j)
                                     if (!((mbits >> j) & 1u)) f[j] = 0.f;
-                            } else if (EXTRA >= 1 && p.mask_y && valid) {
+                            } else if (MASK && p.mask_y && valid) {
                                 const __nv_bfloat16* yp = reinterpret_cast<const __nv_bfloat16*>(p.mask_y) + addr;
 #pragma unroll
                                 for (int j4 = 0; j4 < 4; ++j4) {
@@ -862,7 +806,7 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
                     }
                     // fused ReLU mask as a bit word (one 4-byte load, issued before the TMEM load so its latency hides)
                     uint32_t mbits = 0xffffffffu;
-                    if (EXTRA >= 1 && p.mask_bits && valid) mbits = __ldg(p.mask_bits + ((off + c0) >> 5));
+                    if (MASK && p.mask_bits && valid) mbits = __ldg(p.mask_bits + ((off + c0) >> 5));
                     uint32_t v[32];
                     tmem_ld32(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * ACC_COLS + m * BN + c0, v);
                     tmem_ld_wait();
@@ -884,11 +828,11 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
 #pragma unroll
                         for (int j = 0; j < 32; ++j) f[j] = 1.f / (1.f + __expf(-f[j]));
                     }
-                    if (EXTRA >= 1 && p.mask_bits) {
+                    if (MASK && p.mask_bits) {
 #pragma unroll
                         for (int j = 0; j < 32; ++j)
                             if (!((mbits >> j) & 1u)) f[j] = 0.f;
-                    } else if (EXTRA >= 1 && p.mask_y && valid) {
+                    } else if (MASK && p.mask_y && valid) {
                         const __nv_bfloat16* yp = reinterpret_cast<const __nv_bfloat16*>(p.mask_y) + off + c0;
 #pragma unroll
                         for (int j4 = 0; j4 < 4; ++j4) {
@@ -973,36 +917,10 @@ __global__ void __launch_bounds__(IGP_THREADS) igemm_persistent_kernel(const __g
                     }
                     if (!SMEM_STATS && do_stats) {
                         float g2[32];
-                        if (EXTRA == 2 && p.bnb_x) {  // BN-backward sums: f <- g = dy * relu-mask, g2 <- g * xhat
-                            const int cb = (p.merge ? 0 : nt * BN) + stat_col;
-                            float xv[32];
-                            if (valid) {
-                                const __nv_bfloat16* xp = reinterpret_cast<const __nv_bfloat16*>(p.bnb_x) + off + c0;
 #pragma unroll
-                                for (int j4 = 0; j4 < 4; ++j4) {
-                                    const uint4 raw = __ldg(reinterpret_cast<const uint4*>(xp + 8 * j4));
-                                    const uint32_t rr[4] = {raw.x, raw.y, raw.z, raw.w};
-#pragma unroll
-                                    for (int j = 0; j < 4; ++j) {
-                                        xv[8 * j4 + 2 * j] = __uint_as_float(rr[j] << 16);
-                                        xv[8 * j4 + 2 * j + 1] = __uint_as_float(rr[j] & 0xffff0000u);
-                                    }
-                                }
-                            }
-#pragma unroll
-                            for (int j = 0; j < 32; ++j) {
-                                const float xc = (valid ? xv[j] : 0.f) - s_bnp[cb + j];
-                                float g = valid ? f[j] : 0.f;
-                                if (p.bnb_relu && !(xc * s_bnp[256 + cb + j] + s_bnp[512 + cb + j] > 0.f)) g = 0.f;
-                                f[j] = g;
-                                g2[j] = g * (xc * s_bnp[768 + cb + j]);
-                            }
-                        } else {
-#pragma unroll
-                            for (int j = 0; j < 32; ++j) {
-                                f[j] = valid ? f[j] : 0.f;
-                                g2[j] = f[j] * f[j];
-                            }
+                        for (int j = 0; j < 32; ++j) {
+                            f[j] = valid ? f[j] : 0.f;
+                            g2[j] = f[j] * f[j];
                         }
 #pragma unroll
                         for (int j = 0; j < 32; ++j) {
@@ -1051,15 +969,14 @@ struct WgParams {
     CUtensorMap mapS[4];  // shifted operand planes, box (NCH, bw, bh, bn)
     TapDesc taps[25];
     int num_taps;
+    int rows;  // bw*bh*bn, multiple of 16
+    float* out;
+    long long split_stride;  // elements between the output slices of consecutive splits (0: all splits add into one)
     int bw, bh, bn;
     int tiles_x, tiles_y, tiles_n;  // pixel tiles (the reduction)
     int m_total, n_total;
     int m_tiles, n_tiles;
     int splits;
-    int rows;  // bw*bh*bn, multiple of 16
-    int merge_taps;  // one N = TG*BN MMA per K step when the kernel supports it (A/B switch)
-    float* out;
-    long long split_stride;  // elements between the output slices of consecutive splits (0: all splits add into one)
 };
 
 // TG = filter taps handled by one CTA against the SAME dense-operand tile: with a 32-channel shifted side the dense tile
@@ -1175,25 +1092,22 @@ __global__ void __launch_bounds__(192) wgrad_kernel(const __grid_constant__ WgPa
                 if constexpr (TG > 1 && BN == NCH && TG * BN <= 256) {
                     // One channel chunk per tap: the TG shifted tiles sit at a fixed stride in the stage, which is exactly
                     // an MN-major operand whose N-direction atom stride (LBO) is the tile stride. ONE N = TG*BN MMA per
-                    // K step instead of TG N = BN ones (FMRI_WG_MERGE=0 keeps the per-tap issue for A/B): the 32-channel
-                    // layers were issue-bound at 40 N = 32 MMAs per stage.
-                    if (p.merge_taps) {
-                        const uint32_t idesc_m = umma_idesc_bf16(128, tg_live * BN, true, true);
-                        const uint64_t bdesc = umma_smem_desc(sd + L::D_BYTES, L::S_BYTES, 8 * s_row, s_layout);
-                        for (int k = 0; k < ksteps; ++k)
-                            umma_bf16_elect(tmem_u, adesc + ((k * 16 * 128) >> 4), bdesc + ((k * 16 * s_row) >> 4), idesc_m,
-                                            (i | k) != 0);
-                        umma_commit_elect(&empty_bar[st]);
-                        continue;
-                    }
-                }
-#pragma unroll
-                for (int tg = 0; tg < TG; ++tg) {
-                    if (tg >= tg_live) break;
-                    const uint64_t bdesc = umma_smem_desc(sd + L::D_BYTES + tg * L::S_BYTES, s_chunk_bytes, 8 * s_row, s_layout);
+                    // K step instead of TG N = BN ones: the 32-channel layers were issue-bound at 40 N = 32 MMAs per stage.
+                    const uint32_t idesc_m = umma_idesc_bf16(128, tg_live * BN, true, true);
+                    const uint64_t bdesc = umma_smem_desc(sd + L::D_BYTES, L::S_BYTES, 8 * s_row, s_layout);
                     for (int k = 0; k < ksteps; ++k)
-                        umma_bf16_elect(tmem_u + tg * BN, adesc + ((k * 16 * 128) >> 4), bdesc + ((k * 16 * s_row) >> 4),
-                                        idesc, (i | k) != 0);
+                        umma_bf16_elect(tmem_u, adesc + ((k * 16 * 128) >> 4), bdesc + ((k * 16 * s_row) >> 4), idesc_m,
+                                        (i | k) != 0);
+                } else {
+#pragma unroll
+                    for (int tg = 0; tg < TG; ++tg) {
+                        if (tg >= tg_live) break;
+                        const uint64_t bdesc =
+                            umma_smem_desc(sd + L::D_BYTES + tg * L::S_BYTES, s_chunk_bytes, 8 * s_row, s_layout);
+                        for (int k = 0; k < ksteps; ++k)
+                            umma_bf16_elect(tmem_u + tg * BN, adesc + ((k * 16 * 128) >> 4),
+                                            bdesc + ((k * 16 * s_row) >> 4), idesc, (i | k) != 0);
+                    }
                 }
                 umma_commit_elect(&empty_bar[st]);
             }

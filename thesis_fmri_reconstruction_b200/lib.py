@@ -32,9 +32,8 @@ class EdgeDesc(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("N", "H", "W", "C", "stride", "dtype")]
 
 
-class BnFuse(C.Structure):
-    _fields_ = [("x", C.c_void_p), ("mean", C.c_void_p), ("invstd", C.c_void_p), ("gamma", C.c_void_p),
-                ("beta", C.c_void_p), ("relu", C.c_int), ("sums", C.c_void_p), ("mask_bits", C.c_void_p)]
+class ReluMask(C.Structure):
+    _fields_ = [("y", C.c_void_p), ("bits", C.c_void_p)]
 
 
 class LinearDesc(C.Structure):
@@ -203,21 +202,17 @@ def conv_fprop(d, x, w, pack_f, bias, act, y, stat_sum=None, stat_sq=None):
                                   ptr(stat_sq), stream()))
 
 
-def conv_dgrad(d, dy, w, pack_d, dx, fuse=None):
-    """fuse = (x, mean, invstd, gamma, beta, relu, sums): also produce the BN-backward sums of the layer dx feeds."""
+def conv_dgrad(d, dy, w, pack_d, dx, relu_mask=None):
+    """relu_mask = (y, bits or None): dx is the upstream gradient of a bias+ReLU layer with output y; the call also
+    applies its ReLU backward, dx *= (y > 0) (bits: relu_bitmask of y, 32-channel tensors)."""
     _require_cuda(dy, w, pack_d, dx)
     _note_flops(_conv_flops(d))
-    f = None
-    if fuse is not None and fuse[1] is None:   # (y, None x5 [, bits]): ReLU mask of a bias+ReLU layer, dx *= (y > 0)
-        bits = fuse[7] if len(fuse) > 7 else None
-        _require_cuda(fuse[0], bits)
-        f = BnFuse(fuse[0].data_ptr(), None, None, None, None, 1, None, bits.data_ptr() if bits is not None else None)
-    elif fuse is not None:
-        x, mean, invstd, gamma, beta, relu, sums = fuse
-        _require_cuda(x, mean, invstd, gamma, beta, sums)
-        f = BnFuse(x.data_ptr(), mean.data_ptr(), invstd.data_ptr(), gamma.data_ptr(), beta.data_ptr(), int(relu),
-                   sums.data_ptr(), None)
-    _check(load().fmri_conv_dgrad(C.byref(d), ptr(dy), ptr(w), ptr(pack_d), ptr(dx), C.byref(f) if f else None, stream()))
+    m = None
+    if relu_mask is not None:
+        y, bits = relu_mask
+        _require_cuda(y, bits)
+        m = ReluMask(ptr(y), ptr(bits))
+    _check(load().fmri_conv_dgrad(C.byref(d), ptr(dy), ptr(w), ptr(pack_d), ptr(dx), C.byref(m) if m else None, stream()))
 
 
 def conv_wgrad_workspace(d):
@@ -327,20 +322,19 @@ def bn_apply(x, y, rows, Cc, mean, invstd, gamma, beta, relu):
                                 ptr(beta), int(relu), stream()))
 
 
-def bn_backward(x, dy, dx, rows, Cc, mean, invstd, gamma, beta, relu, train, dgamma, dbeta, accumulate, ws,
-                sums_ready=False):
+def bn_backward(x, dy, dx, rows, Cc, mean, invstd, gamma, beta, relu, train, dgamma, dbeta, accumulate, ws):
     _require_cuda(x, dy, dx, mean, invstd, gamma, beta, dgamma, dbeta, ws)
     _check(load().fmri_bn_backward(ptr(x), dt(x), ptr(dy), ptr(dx), dt(dy), _ll(rows), Cc, ptr(mean), ptr(invstd),
                                    ptr(gamma), ptr(beta), int(relu), int(train), ptr(dgamma), ptr(dbeta),
-                                   int(accumulate), ptr(ws), int(sums_ready), stream()))
+                                   int(accumulate), ptr(ws), stream()))
 
 
-def bn_backward_slice(x, dy, dx, rows, row0, nrows, Cc, mean, invstd, gamma, beta, relu, train, ws, sums_ready=False):
+def bn_backward_slice(x, dy, dx, rows, row0, nrows, Cc, mean, invstd, gamma, beta, relu, train, ws):
     """BatchNorm backward whose sums run over all `rows` but whose dx is produced for rows [row0, row0 + nrows) only."""
     _require_cuda(x, dy, dx, mean, invstd, gamma, beta, ws)
     _check(load().fmri_bn_backward_slice(ptr(x), dt(x), ptr(dy), ptr(dx), dt(dy), _ll(rows), _ll(row0), _ll(nrows), Cc,
                                          ptr(mean), ptr(invstd), ptr(gamma), ptr(beta), int(relu), int(train), None, None,
-                                         0, ptr(ws), int(sums_ready), stream()))
+                                         0, ptr(ws), stream()))
 
 
 def relu_backward(y, dy, dx):

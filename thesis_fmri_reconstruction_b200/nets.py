@@ -86,17 +86,7 @@ class BatchNorm:
         L.bn_apply(raw, y, rows, C, mean, invstd, P[pre + "weight"], P[pre + "bias"], relu)
         return y, Ctx(raw=raw, mean=mean, invstd=invstd, rows=rows, relu=relu, train=train)
 
-    def fuse_spec(self, P, c):
-        """Arguments that let the data-gradient kernel producing this layer's dy also compute its backward sums
-        (fmri_bn_fuse); only for train-mode BN over at most 256 channels stored in bf16."""
-        if not c.train or self.C > 256 or c.raw.dtype != BF16:
-            return None
-        if self._ws is None:
-            self._ws = E(3 * self.C, dtype=F64)
-        pre = self.prefix
-        return (c.raw, c.mean, c.invstd, P[pre + "weight"], P[pre + "bias"], c.relu, self._ws)
-
-    def backward(self, P, c, dy, G, acc, need_dw, sums_ready=False):
+    def backward(self, P, c, dy, G, acc, need_dw):
         """dy has the gradient dtype; returns d(raw) in the same dtype."""
         C, pre = self.C, self.prefix
         if self._ws is None:
@@ -104,7 +94,7 @@ class BatchNorm:
         draw = torch.empty(c.raw.shape, dtype=dy.dtype, device=dy.device)
         L.bn_backward(c.raw, dy, draw, c.rows, C, c.mean, c.invstd, P[pre + "weight"], P[pre + "bias"], c.relu,
                       c.train, G[pre + "weight"] if need_dw else None, G[pre + "bias"] if need_dw else None, acc,
-                      self._ws, sums_ready)
+                      self._ws)
         return draw
 
 
@@ -144,13 +134,12 @@ class ConvBlock:
                                 stats if train else None, nbt)
         return y, Ctx(d=d, x=x, bn=cb, pack_f=self.pack_f, pack_d=self.pack_d, OH=OH, OW=OW)
 
-    def backward(self, P, c, dy, G, acc, need_dw, need_dx, sums_ready=False, fuse=None):
-        """sums_ready: the kernel that produced dy already left this BN's backward sums (see fuse_spec).
-        fuse: fuse_spec of the layer BELOW, handed to this layer's data-gradient kernel."""
-        draw = self.bn.backward(P, c.bn, dy, G, acc, need_dw, sums_ready)
-        return self.backward_raw(P, c, draw, G, acc, need_dw, need_dx, fuse)
+    def backward(self, P, c, dy, G, acc, need_dw, need_dx, relu_mask=None):
+        """relu_mask: (y, bits) of the bias+ReLU layer BELOW, whose ReLU backward this layer's data-gradient kernel applies."""
+        draw = self.bn.backward(P, c.bn, dy, G, acc, need_dw)
+        return self.backward_raw(P, c, draw, G, acc, need_dw, need_dx, relu_mask)
 
-    def backward_dx_slice(self, P, c, dy, n0, n1, fuse=None, sums_ready=False):
+    def backward_dx_slice(self, P, c, dy, n0, n1, relu_mask=None):
         """Data gradient only, for images [n0, n1) of the batch. Train-mode BatchNorm couples all samples through its two
         backward sums, so those run over the whole batch; the BN apply pass and the conv data gradient run on the slice only
         (the discriminator's feature-tap sweep needs the image gradient of ONE of its three sources). Returns dx of the slice."""
@@ -161,19 +150,19 @@ class ConvBlock:
             self.bn._ws = E(3 * C, dtype=F64)
         draw = E(n1 - n0, c.OH, c.OW, C, dtype=dy.dtype)
         L.bn_backward_slice(cb.raw, dy, draw, N * per, n0 * per, (n1 - n0) * per, C, cb.mean, cb.invstd, P[pre + "weight"],
-                            P[pre + "bias"], cb.relu, cb.train, self.bn._ws, sums_ready)
+                            P[pre + "bias"], cb.relu, cb.train, self.bn._ws)
         dsub = self.desc(n1 - n0, c.d.H, c.d.W)
         dx = E(n1 - n0, c.d.H, c.d.W, self.Cin, dtype=self.adt)
-        L.conv_dgrad(dsub, draw, P[self.prefix + "conv.weight"], c.pack_d, dx, fuse)
+        L.conv_dgrad(dsub, draw, P[self.prefix + "conv.weight"], c.pack_d, dx, relu_mask)
         return dx
 
-    def backward_raw(self, P, c, draw, G, acc, need_dw, need_dx, fuse=None):
+    def backward_raw(self, P, c, draw, G, acc, need_dw, need_dx, relu_mask=None):
         """Backward from a gradient on the raw (pre-BN) conv output -- the discriminator's feature tap (vae_gan.py:169-173)."""
         w = P[self.prefix + "conv.weight"]
         dx = None
         if need_dx:
             dx = torch.empty(c.x.shape, dtype=self.adt, device=draw.device)
-            L.conv_dgrad(c.d, draw, w, c.pack_d, dx, fuse)
+            L.conv_dgrad(c.d, draw, w, c.pack_d, dx, relu_mask)
         if need_dw:
             if self._ws is None:
                 self._ws = E(max(1, L.conv_wgrad_workspace(c.d)), dtype=torch.uint8)
@@ -246,25 +235,7 @@ class BlockNet:
         return dxo
 
 
-# Fusing the BN-backward reduction into the data-gradient epilogue (fmri_bn_fuse) removes 2 of BN-backward's 5 tensor passes
-# (-8.5 ms/step at B = 4096) but the heavier epilogue stops hiding behind the next tile's main loop in the persistent kernel
-# (+15.6 ms/step on the data-gradient launches), so it is OFF by default until the epilogue is spread over more warps.
 import os as _os
-
-# FMRI_FUSE_BN: "0" never (default), "1" always, "auto": only in data-gradient launches with a deep contraction (>= 128 channels
-# x 25 taps per tile). Measured at batch 4096 on one B200 (round 2, same box): off 110.9 ms/step (igemm 47.4, BN backward 18.6),
-# auto 113.5 (56.2 / 13.3), always 114.7 (57.8 / 11.9). Even where the epilogue hides behind the next tile's MMAs the fused
-# launch still has to read the pre-BN tensor (the same bytes the separate reduction pass reads at 4.8 TB/s) and that traffic
-# competes with the TMA operand stream of an L2-bandwidth-bound kernel: the pass it removes is cheaper than the slowdown it causes.
-FUSE_BN_MODE = _os.environ.get("FMRI_FUSE_BN", "0")
-FUSE_BN_BWD = FUSE_BN_MODE != "0"
-
-
-def _want_fuse(block):
-    """Should `block`'s data-gradient kernel also produce the BatchNorm-backward sums of the layer below it?"""
-    if FUSE_BN_MODE == "1":
-        return True
-    return FUSE_BN_MODE == "auto" and block.Cout >= 128   # the data gradient contracts over the block's output channels
 
 # Tensor-core weight gradients on a side stream: OFF by default (FMRI_WGRAD_STREAM=1 enables). Measured on one B200: -0.7 % step
 # time at batch 4096 (the GPU is power-capped, so overlapping tensor-pipe and HBM-bound kernels buys little), but 2x slower at
@@ -292,25 +263,12 @@ def side_into(stream):
         stream.wait_stream(_SIDE)
 
 
-def _backward_chain(blocks, ctxs, P, dy, G, acc, need_dw, lower=None, first_ready=False, relu_mask=None):
-    """Backward through a stack of ConvBlocks (last block first). Each block's data-gradient kernel also produces the
-    BatchNorm-backward sums of the block below it (fmri_bn_fuse), so that block's BN backward skips its reduction pass.
-    lower = (BatchNorm, ctx) of the BN below blocks[0], if any. Returns (dx of blocks[0], sums_ready for `lower`)."""
-    ready = first_ready
+def _backward_chain(blocks, ctxs, P, dy, G, acc, need_dw, relu_mask=None):
+    """Backward through a stack of ConvBlocks (last block first); returns dx of blocks[0]. relu_mask = (y, bits): the layer
+    below blocks[0] is bias+ReLU without BatchNorm, and its ReLU backward rides in blocks[0]'s data-gradient epilogue."""
     for i in range(len(blocks) - 1, -1, -1):
-        if not _want_fuse(blocks[i]):
-            fuse = None
-        elif i > 0:
-            fuse = blocks[i - 1].bn.fuse_spec(P, ctxs[i - 1].bn)
-        else:
-            fuse = lower[0].fuse_spec(P, lower[1]) if lower is not None else None
-        if i == 0 and relu_mask is not None:
-            # the layer below blocks[0] is bias+ReLU without BatchNorm: its ReLU backward rides in this data-gradient epilogue
-            y_below, bits = relu_mask if isinstance(relu_mask, tuple) else (relu_mask, None)
-            fuse = (y_below, None, None, None, None, 1, None, bits)
-        dy = blocks[i].backward(P, ctxs[i], dy, G, acc, need_dw, True, ready, fuse)
-        ready = fuse is not None and fuse[1] is not None
-    return dy, ready
+        dy = blocks[i].backward(P, ctxs[i], dy, G, acc, need_dw, True, relu_mask if i == 0 else None)
+    return dy
 
 
 # ====================================================================================================== linear pieces
@@ -529,8 +487,8 @@ class EncoderNet:
         else:
             dy = E(B, h, w, self.Clast, dtype=self.adt)
             L.nchw_to_nhwc(dflat, dy, B, self.Clast, h, w)
-        dy, ready = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw, (self.bn0, c.c0))
-        draw0 = self.bn0.backward(P, c.c0, dy, G, acc, need_dw, ready)
+        dy = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw)
+        draw0 = self.bn0.backward(P, c.c0, dy, G, acc, need_dw)
         if need_dw:
             L.edge_in_wgrad(c.d0, [c.x], B, draw0, G["conv.0.conv.weight"], acc, self._ews)
 
@@ -600,7 +558,7 @@ class DecoderNet:
             L.edge_out_wgrad(c.d3, c.a3, dpre, G["conv.3.0.weight"], acc, self._ews)
         dy = torch.empty(c.a3.shape, dtype=self.adt, device=dpre.device)
         L.edge_out_dgrad(c.d3, dpre, P["conv.3.0.weight"], dy, self._ews)
-        dy, _ = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw)
+        dy = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw)
         f = self.fi
         dflat = E(B, self.size * f * f, dtype=self.adt)
         L.nhwc_to_nchw(dy, dflat, B, self.size, f, f)
@@ -709,27 +667,22 @@ class DiscriminatorNet:
         else:
             dy = E(N, h, w, self.Cl, dtype=self.adt)
             L.nchw_to_nhwc(dflat, dy, N, self.Cl, h, w)
-        dy, _ = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw, relu_mask=(c.y0, c.mask0))
+        dy = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw, (c.y0, c.mask0))
         return self._conv0_backward(P, c, dy, G, acc, need_dw, img_slices)
 
     def backward_rec(self, P, c, draw3, G=None, acc=False, need_dw=False, img_slices=None, live=None):
         """Backward of the feature-tap path from a gradient on the raw conv output of block 3 [N,h,w,C] (adt).
         live = (s0, s1): only sources [s0, s1) of draw3 are non-zero (the feature-matching loss compares x and x_tilde; the
         x_p third gets no gradient at the tap, train_vgan_stage1.py:369 / vae_gan.py:313).
-        Data-gradient-only fast path (need_dw False, no fused BN sums): block 3's data gradient runs on the live sources only
+        Data-gradient-only fast path (need_dw False): block 3's data gradient runs on the live sources only
         (the rest of its output is exactly zero), and block 1's BN apply + data gradient + conv[0] run on the requested image
         slice only -- BatchNorm's coupling of the whole 3B batch is kept by running every BN's backward SUMS over all of it."""
         top = self.level - 1
+        mask0 = (c.y0, c.mask0)
         if top != 2:   # feature tap below block 3: plain chain from the tap's block down
-            fuse = None
-            if top > 0 and _want_fuse(self.blocks[top]):
-                fuse = self.blocks[top - 1].bn.fuse_spec(P, c.blocks[top - 1].bn)
-            elif top == 0:
-                fuse = (c.y0, None, None, None, None, 1, None, c.mask0)
-            dy = self.blocks[top].backward_raw(P, c.blocks[top], draw3, G, acc, need_dw, True, fuse)
+            dy = self.blocks[top].backward_raw(P, c.blocks[top], draw3, G, acc, need_dw, True, mask0 if top == 0 else None)
             if top > 0:
-                dy, _ = _backward_chain(self.blocks[:top], c.blocks[:top], P, dy, G, acc, need_dw, None, fuse is not None,
-                                        relu_mask=(c.y0, c.mask0))
+                dy = _backward_chain(self.blocks[:top], c.blocks[:top], P, dy, G, acc, need_dw, mask0)
             return self._conv0_backward(P, c, dy, G, acc, need_dw, img_slices)
         if not need_dw and img_slices is not None and len(c.imgs) > 1:
             Bs = c.Bs
@@ -740,26 +693,20 @@ class DiscriminatorNet:
                 dy[:l0 * Bs].zero_()
             if l1 < len(c.imgs):
                 dy[l1 * Bs:].zero_()
-            # fused BN-backward sums of block 2 over the live rows only: the other rows of dy are exactly zero
-            f2 = self.blocks[1].bn.fuse_spec(P, c.blocks[1].bn) if _want_fuse(b3) else None
             L.conv_dgrad(b3.desc((l1 - l0) * Bs, c3.d.H, c3.d.W), draw3[l0 * Bs:l1 * Bs], P[b3.prefix + "conv.weight"],
-                         c3.pack_d, dy[l0 * Bs:l1 * Bs], f2)
-            f1 = self.blocks[0].bn.fuse_spec(P, c.blocks[0].bn) if _want_fuse(self.blocks[1]) else None
-            dy = self.blocks[1].backward(P, c.blocks[1], dy, None, False, False, True, f2 is not None, f1)
+                         c3.pack_d, dy[l0 * Bs:l1 * Bs])
+            dy = self.blocks[1].backward(P, c.blocks[1], dy, None, False, False, True)
             s0, s1 = img_slices
             OH, OW = c.hw0
             bits = c.mask0[s0 * Bs * OH * OW:s1 * Bs * OH * OW] if c.mask0 is not None else None
-            dy0 = self.blocks[0].backward_dx_slice(P, c.blocks[0], dy, s0 * Bs, s1 * Bs,
-                                                   (c.y0[s0 * Bs:s1 * Bs], None, None, None, None, 1, None, bits), f1 is not None)
+            dy0 = self.blocks[0].backward_dx_slice(P, c.blocks[0], dy, s0 * Bs, s1 * Bs, (c.y0[s0 * Bs:s1 * Bs], bits))
             n = (s1 - s0) * Bs
             dimg = E(n, 3, c.H, c.W)
             L.edge_in_dgrad(L.edge_desc(n, c.H, c.W, self.C0, self.stride0, self.adt), dy0, P["conv.0.0.weight"], dimg,
                             self._ews)
             return dimg
-        fuse = self.blocks[1].bn.fuse_spec(P, c.blocks[1].bn) if _want_fuse(self.blocks[2]) else None
-        dy = self.blocks[2].backward_raw(P, c.blocks[2], draw3, G, acc, need_dw, True, fuse)
-        dy, _ = _backward_chain(self.blocks[:2], c.blocks[:2], P, dy, G, acc, need_dw, None, fuse is not None,
-                                relu_mask=(c.y0, c.mask0))
+        dy = self.blocks[2].backward_raw(P, c.blocks[2], draw3, G, acc, need_dw, True)
+        dy = _backward_chain(self.blocks[:2], c.blocks[:2], P, dy, G, acc, need_dw, mask0)
         return self._conv0_backward(P, c, dy, G, acc, need_dw, img_slices)
 
 
