@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FMRI_ABI_VERSION 4
+#define FMRI_ABI_VERSION 5
 
 typedef enum { FMRI_OK = 0, FMRI_ERR_ARG = -1, FMRI_ERR_UNSUPPORTED = -2, FMRI_ERR_CUDA = -3, FMRI_ERR_WORKSPACE = -4 } fmri_status;
 typedef enum { FMRI_F32 = 0, FMRI_BF16 = 1 } fmri_dtype;
@@ -267,6 +267,28 @@ int fmri_pearson(const float* a, const float* b, long long n, float* out, double
 int fmri_ssim(const float* a, const float* b, int N, int C, int H, int W, float* out, double* ws, void* stream);
 int fmri_image_pipeline(const unsigned char* src, int N, int H, int W, int Csrc, const int* flip, const int* shift_yx,
                         const float* mean3, const float* std3, float* dst, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
+ * All-pairs similarity and n-way identification: the exhaustive, exact-expectation form of the reference's sampled
+ * objective_assessment (train/train_utils.py:752).
+ * fmri_pairwise_similarity: out[i, j] (fp32, [N, M] row-major) = the metric of pred[i] (of [N, C, H, W]) against
+ *   target[j] (of [M, C, H, W]), both fp32 NCHW:
+ *     FMRI_METRIC_PCC  PearsonCorrelation()(pred[i:i+1], target[j:j+1])      (train_utils.py:267-293)
+ *     FMRI_METRIC_SSIM StructuralSimilarity()(pred[i:i+1], target[j:j+1])    (train_utils.py:295-425; the window and
+ *                      constants of fmri_ssim; H or W below 11 is FMRI_ERR_UNSUPPORTED)
+ *   ws: fmri_pairwise_workspace() bytes, 16-byte aligned (FMRI_ERR_WORKSPACE when smaller). CUDA-core fp32 with fp64
+ *   accumulation, no atomics: two calls on the same inputs give the same bits.
+ * fmri_identification: from a square similarity matrix sim [N, N] (row i: reconstruction i, column i: its own target),
+ *   wins[i] = #{j != i : sim[i, i] > sim[i, j]} (strict; NaN never wins) and, for each n = ns[q] (a HOST array,
+ *   2 <= n <= N), acc[q] = (1/N) sum_i C(wins[i], n-1) / C(N-1, n-1): the probability that the true target beats n-1
+ *   distractors drawn uniformly without replacement, averaged over the rows, in fp64.
+ * Every argument is checked before the first launch (FMRI_ERR_ARG for N < 2, n outside [2, N], non-positive sizes).
+ * --------------------------------------------------------------------------------------------------------- */
+typedef enum { FMRI_METRIC_PCC = 0, FMRI_METRIC_SSIM = 1 } fmri_metric;
+size_t fmri_pairwise_workspace(int N, int M, int C, int H, int W, int metric); /* bytes; 0 for invalid arguments */
+int fmri_pairwise_similarity(const float* pred, int N, const float* target, int M, int C, int H, int W, int metric,
+                             float* out, void* ws, size_t ws_bytes, void* stream);
+int fmri_identification(const float* sim, int N, const int* ns, int n_count, int* wins, double* acc, void* stream);
 
 #ifdef __cplusplus
 }

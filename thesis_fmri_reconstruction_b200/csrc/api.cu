@@ -14,6 +14,7 @@
 #include "cto3_kernels.cuh"
 #include "mmd_kernels.cuh"
 #include "eval_kernels.cuh"
+#include "similarity_kernels.cuh"
 
 using namespace fmri;
 
@@ -2069,23 +2070,26 @@ extern "C" int fmri_pearson(const float* a, const float* b, long long n, float* 
     LAUNCH_OK();
     return 0;
 }
-extern "C" int fmri_ssim(const float* a, const float* b, int N, int C, int H, int W, float* out, double* ws, void* stream) {
-    if (!a || !b || !out || !ws || N <= 0 || C <= 0 || H <= 0 || W <= 0) return fail(FMRI_ERR_ARG, "ssim arguments");
-    // below 11 pixels the reference pads by 5 around a SMALLER window and its SSIM map outgrows the image (train_utils.py:378-390)
-    if (H < 11 || W < 11) return fail(FMRI_ERR_UNSUPPORTED, "ssim: images smaller than the 11 x 11 window (%d x %d)", H, W);
-    // gaussian(window_size, 1.5) of train_utils.py:310-323, evaluated in double and rounded to float like torch.Tensor([...])
-    const int win = std::min(11, std::min(H, W));
+// gaussian(window_size, 1.5) of train_utils.py:310-323, evaluated in double and rounded to float like torch.Tensor([...]),
+// normalised by its fp32 sum; taps beyond `win` are zero. fmri_ssim and fmri_pairwise_similarity share these floats.
+static SsimWindow ssim_window(int win) {
     SsimWindow wd;
-    double g[11], sum = 0.0;
+    double g[11];
     for (int x = 0; x < win; ++x) {
         const double d = x - win / 2;
         g[x] = (double)(float)exp(-(d * d) / (2.0 * 1.5 * 1.5));
-        sum += (double)(float)g[x];
     }
     float fs = 0.f;
     for (int x = 0; x < win; ++x) fs += (float)g[x];
     for (int x = 0; x < 11; ++x) wd.g[x] = x < win ? (float)g[x] / fs : 0.f;
-    (void)sum;
+    return wd;
+}
+extern "C" int fmri_ssim(const float* a, const float* b, int N, int C, int H, int W, float* out, double* ws, void* stream) {
+    if (!a || !b || !out || !ws || N <= 0 || C <= 0 || H <= 0 || W <= 0) return fail(FMRI_ERR_ARG, "ssim arguments");
+    // below 11 pixels the reference pads by 5 around a SMALLER window and its SSIM map outgrows the image (train_utils.py:378-390)
+    if (H < 11 || W < 11) return fail(FMRI_ERR_UNSUPPORTED, "ssim: images smaller than the 11 x 11 window (%d x %d)", H, W);
+    const int win = std::min(11, std::min(H, W));
+    const SsimWindow wd = ssim_window(win);
     CUDA_OK(cudaMemsetAsync(ws, 0, sizeof(double), S(stream)));
     const long long total = (long long)N * C * H * W;
     ssim_kernel<<<grid1d(total, 256, 148 * 8), 256, 0, S(stream)>>>(a, b, N * C, H, W, win, wd, ws);
@@ -2102,5 +2106,87 @@ extern "C" int fmri_image_pipeline(const unsigned char* src, int N, int H, int W
     image_pipeline_kernel<<<grid1d((long long)N * 3 * H * W, 256, 148 * 8), 256, 0, S(stream)>>>(
         src, N, H, W, Csrc, flip, shift_yx, m[0], m[1], m[2], sd[0], sd[1], sd[2], dst);
     LAUNCH_OK();
+    return 0;
+}
+
+// ================================================================================================ all-pairs similarity
+static inline long long ssim_pitch_w(int W) { return ((long long)W + 7) / 8 * 8; }
+extern "C" size_t fmri_pairwise_workspace(int N, int M, int C, int H, int W, int metric) {
+    if (N <= 0 || M <= 0 || C <= 0 || H <= 0 || W <= 0) return 0;
+    if (metric == FMRI_METRIC_PCC) return sizeof(double2) * ((size_t)N + (size_t)M);
+    if (metric == FMRI_METRIC_SSIM) return sizeof(float) * 2 * ((size_t)N + (size_t)M) * C * H * ssim_pitch_w(W);
+    return 0;
+}
+extern "C" int fmri_pairwise_similarity(const float* pred, int N, const float* target, int M, int C, int H, int W,
+                                        int metric, float* out, void* ws, size_t ws_bytes, void* stream) {
+    if (!pred || !target || !out || N <= 0 || M <= 0 || C <= 0 || H <= 0 || W <= 0)
+        return fail(FMRI_ERR_ARG, "pairwise_similarity arguments");
+    if (metric != FMRI_METRIC_PCC && metric != FMRI_METRIC_SSIM) return fail(FMRI_ERR_ARG, "unknown metric %d", metric);
+    if (metric == FMRI_METRIC_SSIM && (H < 11 || W < 11))
+        return fail(FMRI_ERR_UNSUPPORTED, "ssim: images smaller than the 11 x 11 window (%d x %d)", H, W);
+    const size_t need = fmri_pairwise_workspace(N, M, C, H, W, metric);
+    if (!ws || ws_bytes < need) return fail(FMRI_ERR_WORKSPACE, "pairwise_similarity workspace %zu < %zu", ws_bytes, need);
+    if (reinterpret_cast<uintptr_t>(ws) % 16) return fail(FMRI_ERR_ARG, "pairwise_similarity workspace not 16-byte aligned");
+    const long long K = (long long)C * H * W;
+    if (metric == FMRI_METRIC_PCC) {
+        if (cdiv(M, PG_BN) > 65535) return fail(FMRI_ERR_UNSUPPORTED, "pairwise pcc: M = %d targets", M);
+        double2* sa = reinterpret_cast<double2*>(ws);
+        double2* sb = sa + N;
+        pcc_stats_kernel<<<N, PCC_STAT_THREADS, 0, S(stream)>>>(pred, K, sa);
+        LAUNCH_OK();
+        pcc_stats_kernel<<<M, PCC_STAT_THREADS, 0, S(stream)>>>(target, K, sb);
+        LAUNCH_OK();
+        pcc_gemm_kernel<<<dim3(cdiv(N, PG_BM), cdiv(M, PG_BN)), PG_THREADS, 0, S(stream)>>>(pred, N, target, M, K, sa, sb,
+                                                                                              out);
+        LAUNCH_OK();
+        return 0;
+    }
+    if (cdiv(M, SS_TJ) > 65535) return fail(FMRI_ERR_UNSUPPORTED, "pairwise ssim: M = %d targets", M);
+    SsimPairArgs p;
+    p.a = pred;
+    p.b = target;
+    p.N = N, p.M = M, p.C = C, p.H = H, p.W = W, p.WP = (int)ssim_pitch_w(W);
+    const long long plane = (long long)H * p.WP;
+    float* maps = reinterpret_cast<float*>(ws);
+    p.mu_a = maps;
+    p.sig_a = maps + (long long)N * C * plane;
+    p.mu_b = maps + 2LL * N * C * plane;
+    p.sig_b = p.mu_b + (long long)M * C * plane;
+    // equal column groups of at most SS_MAXW * 8 columns, each a multiple of 8 wide
+    const int groups = cdiv(W, SS_MAXW * SS_R);
+    p.cols = cdiv(cdiv(W, groups), SS_R) * SS_R;
+    p.pitch = ss_pitch(p.cols + 10);
+    p.inv_count = 1.0 / (double)K;
+    p.wd = ssim_window(11);
+    p.out = out;
+    const size_t smem = sizeof(float) * 2 * SS_BAND * SS_IMGS * p.pitch;   // two band buffers
+    CUDA_OK(cudaFuncSetAttribute(ssim_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ssim_maps_kernel<<<grid1d((long long)N * C * plane, 256), 256, 0, S(stream)>>>(pred, (long long)N * C, H, W, p.WP, p.wd,
+                                                                                     const_cast<float*>(p.mu_a),
+                                                                                     const_cast<float*>(p.sig_a));
+    LAUNCH_OK();
+    ssim_maps_kernel<<<grid1d((long long)M * C * plane, 256), 256, 0, S(stream)>>>(target, (long long)M * C, H, W, p.WP,
+                                                                                     p.wd, const_cast<float*>(p.mu_b),
+                                                                                     const_cast<float*>(p.sig_b));
+    LAUNCH_OK();
+    ssim_pair_kernel<<<dim3(cdiv(N, SS_TI), cdiv(M, SS_TJ)), p.cols / SS_R * 32, smem, S(stream)>>>(p);
+    LAUNCH_OK();
+    return 0;
+}
+extern "C" int fmri_identification(const float* sim, int N, const int* ns, int n_count, int* wins, double* acc,
+                                   void* stream) {
+    if (!sim || !wins || N < 2) return fail(FMRI_ERR_ARG, "identification needs an [N, N] matrix with N >= 2 (N = %d)", N);
+    if (n_count <= 0 || !ns || !acc) return fail(FMRI_ERR_ARG, "identification: needs n_count >= 1, ns and acc");
+    for (int q = 0; q < n_count; ++q)
+        if (ns[q] < 2 || ns[q] > N) return fail(FMRI_ERR_ARG, "identification: n = %d outside [2, %d]", ns[q], N);
+    ident_wins_kernel<<<cdiv(N, 8), 256, 0, S(stream)>>>(sim, N, wins);
+    LAUNCH_OK();
+    for (int q0 = 0; q0 < n_count; q0 += IDENT_MAX_NS) {
+        IdentNs p;
+        p.count = std::min(IDENT_MAX_NS, n_count - q0);
+        for (int q = 0; q < p.count; ++q) p.n[q] = ns[q0 + q];
+        ident_acc_kernel<<<1, 256, 0, S(stream)>>>(wins, N, p, acc + q0);
+        LAUNCH_OK();
+    }
     return 0;
 }

@@ -12,6 +12,15 @@ Reference behaviour reproduced (all paths relative to /root/reference):
     written twice.
   * metrics: PearsonCorrelation, StructuralSimilarity (train/train_utils.py:267-425), nn.MSELoss -- as the train scripts'
     per-epoch evaluation computes them (train/train_vgan_stage1.py:489-560).
+  * identification (the question objective_assessment, train_utils.py:752, answers by sampling distractors on the host):
+    is reconstruction i more similar to its own stimulus than to the others? similarity_matrix() gives every PCC or SSIM
+    value of reconstructions against stimuli, identification() the wins per reconstruction and the exact expected n-way
+    accuracy over all distractor draws. Over a test set:
+
+        r = Reconstructor(checkpoint, hp.CFG64, z=128, kind="cognitive")
+        recon = torch.cat([r(fmri_batch, sample=False) for fmri_batch in test_fmri])       # [N, 3, 64, 64]
+        S = similarity_matrix(recon, stimuli, metric="ssim")                               # [N, N], row i vs stimulus j
+        wins, acc = identification(S, ns=(2, 5, 10))                                       # acc[0]: pairwise accuracy
 """
 from __future__ import annotations
 
@@ -241,3 +250,44 @@ def ssim(pred, target):
     out, ws = E(1), torch.empty(1, dtype=F64, device="cuda")
     L.ssim(pred.to("cuda", F32).contiguous(), target.to("cuda", F32).contiguous(), out, ws)
     return out[0]
+
+
+# ---- all-pairs similarity and n-way identification
+_METRICS = {"pcc": L.METRIC_PCC, "ssim": L.METRIC_SSIM}
+
+
+def similarity_matrix(pred, target, metric="ssim"):
+    """fp32 [N, M] device tensor of metric(pred[i:i+1], target[j:j+1]) (PearsonCorrelation or StructuralSimilarity of
+    train/train_utils.py:267-425) for pred [N, C, H, W] and target [M, C, H, W]."""
+    if metric not in _METRICS:
+        raise L.FmriError(f"metric must be 'ssim' or 'pcc', not {metric!r}")
+    if pred.dim() != 4 or target.dim() != 4 or tuple(pred.shape[1:]) != tuple(target.shape[1:]):
+        raise L.FmriError(f"pred {tuple(pred.shape)} and target {tuple(target.shape)} must be [N, C, H, W] and [M, C, H, W]")
+    N, Cc, H, W = pred.shape
+    M = target.shape[0]
+    if min(N, M, Cc, H, W) <= 0:
+        raise L.FmriError("similarity_matrix needs non-empty image sets")
+    if metric == "ssim" and (H < 11 or W < 11):
+        raise L.FmriError(f"ssim: images smaller than the 11 x 11 window ({H} x {W})")
+    p, t = pred.to("cuda", F32).contiguous(), target.to("cuda", F32).contiguous()
+    ws = torch.empty(L.pairwise_workspace(N, M, Cc, H, W, _METRICS[metric]), dtype=torch.uint8, device="cuda")
+    out = E(N, M)
+    L.pairwise_similarity(p, t, _METRICS[metric], out, ws)
+    return out
+
+
+def identification(sim, ns=(2, 5, 10)):
+    """(wins int32 [N], acc float64 [len(ns)]) on the device, no host sync, from a square similarity matrix sim [N, N]
+    whose row i is reconstruction i and column i its own target: wins[i] = #{j != i : sim[i, i] > sim[i, j]} (strict, a
+    NaN never wins) and acc[q] = mean_i C(wins[i], n-1) / C(N-1, n-1) for n = ns[q] in [2, N], the probability that the
+    true target beats n-1 distractors drawn without replacement (n = 2: pairwise identification, n = N: top-1)."""
+    if sim.dim() != 2 or sim.shape[0] != sim.shape[1]:
+        raise L.FmriError(f"identification needs a square [N, N] matrix, got {tuple(sim.shape)}")
+    N = sim.shape[0]
+    ns = [int(n) for n in ns]
+    if N < 2 or not ns or any(n < 2 or n > N for n in ns):
+        raise L.FmriError(f"identification needs N >= 2 and every n in [2, N = {N}] (ns = {ns})")
+    s = sim.to("cuda", F32).contiguous()
+    wins, acc = E(N, dtype=torch.int32), E(len(ns), dtype=F64)
+    L.identification(s, ns, wins, acc)
+    return wins, acc

@@ -18,6 +18,7 @@ HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "fmri_b200.h")
 
 F32, BF16 = 0, 1
 ACT_NONE, ACT_RELU, ACT_TANH, ACT_SIGMOID = 0, 1, 2, 3
+METRIC_PCC, METRIC_SSIM = 0, 1
 
 
 class FmriError(RuntimeError):
@@ -62,7 +63,8 @@ class _Proxy:
     def __getattr__(self, name):
         f = getattr(self._c, name)
         if PROF is None or name in ("fmri_last_error", "fmri_conv_out_hw", "fmri_conv_wgrad_workspace",
-                                    "fmri_edge_workspace", "fmri_launch_count", "fmri_version", "fmri_conv_pack_elems"):
+                                    "fmri_edge_workspace", "fmri_launch_count", "fmri_version", "fmri_conv_pack_elems",
+                                    "fmri_pairwise_workspace"):
             return f
 
         def timed(*a):
@@ -127,6 +129,7 @@ def load():
         c.fmri_conv_wgrad_workspace.restype = C.c_size_t
         c.fmri_conv_pack_elems.restype = C.c_size_t
         c.fmri_edge_workspace.restype = C.c_size_t
+        c.fmri_pairwise_workspace.restype = C.c_size_t
         c.fmri_conv_out_hw.restype = None
         c.fmri_launch_count.restype = C.c_longlong
         _lib = _Proxy(c)
@@ -517,3 +520,25 @@ def image_pipeline(src_u8, flip, shift_yx, mean3, std3, dst):
     m = (C.c_float * 3)(*[float(v) for v in mean3])
     s = (C.c_float * 3)(*[float(v) for v in std3])
     _check(load().fmri_image_pipeline(ptr(src_u8), N, H, W, Cs, ptr(flip), ptr(shift_yx), m, s, ptr(dst), stream()))
+
+
+# ------------------------------------------------------------------------------------------------ all-pairs similarity
+def pairwise_workspace(N, M, Cc, H, W, metric):
+    """Bytes of workspace fmri_pairwise_similarity needs (0 for invalid arguments)."""
+    return int(load().fmri_pairwise_workspace(int(N), int(M), int(Cc), int(H), int(W), int(metric)))
+
+
+def pairwise_similarity(pred, target, metric, out, ws):
+    """out[i, j] = metric(pred[i], target[j]) for fp32 NCHW pred [N, C, H, W], target [M, C, H, W]; out fp32 [N, M];
+    ws: a device buffer of at least pairwise_workspace(...) bytes."""
+    _require_cuda(pred, target, out, ws)
+    N, Cc, H, W = pred.shape
+    _check(load().fmri_pairwise_similarity(ptr(pred), N, ptr(target), target.shape[0], Cc, H, W, int(metric), ptr(out),
+                                           ptr(ws), _wsb(ws) if ws is not None else C.c_size_t(0), stream()))
+
+
+def identification(sim, ns, wins, acc):
+    """wins int32 [N] and acc float64 [len(ns)] from a square fp32 similarity matrix sim [N, N]; ns: host ints."""
+    _require_cuda(sim, wins, acc)
+    arr = (C.c_int * len(ns))(*[int(n) for n in ns])
+    _check(load().fmri_identification(ptr(sim), sim.shape[0], arr, len(ns), ptr(wins), ptr(acc), stream()))
