@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FMRI_ABI_VERSION 5
+#define FMRI_ABI_VERSION 6
 
 typedef enum { FMRI_OK = 0, FMRI_ERR_ARG = -1, FMRI_ERR_UNSUPPORTED = -2, FMRI_ERR_CUDA = -3, FMRI_ERR_WORKSPACE = -4 } fmri_status;
 typedef enum { FMRI_F32 = 0, FMRI_BF16 = 1 } fmri_dtype;
@@ -151,6 +151,20 @@ int fmri_bn_backward_slice(const void* x, int x_dtype, const void* dy, void* dx,
                            long long nrows, int C, const float* mean, const float* invstd, const float* gamma,
                            const float* beta, int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws,
                            void* stream);
+/* Two upstreams a, b through one BatchNorm layer (two backward sweeps over the same saved forward state): the sums read x once
+ * for both (3 passes instead of 4), the apply reads x once and writes both gradients (5 passes instead of 6). Each upstream's
+ * dx equals that of fmri_bn_backward bit for bit (same kernels' arithmetic and row partition; only the order of the fp64
+ * atomics behind the means may differ). dgamma / dbeta (nullable) take upstream a's parameter gradient. ws: 6*C doubles. */
+int fmri_bn_backward_pair(const void* x, int x_dtype, const void* dy_a, const void* dy_b, void* dx_a, void* dx_b, int g_dtype,
+                          long long rows, int C, const float* mean, const float* invstd, const float* gamma,
+                          const float* beta, int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws,
+                          void* stream);
+/* The same with upstream b's dx produced for rows [row0, row0 + nrows) only (dx_b points at the first of them); dx_a covers
+ * all rows and the sums of both run over all rows (the discriminator's class path and feature-tap sweeps through block 1). */
+int fmri_bn_backward_pair_slice(const void* x, int x_dtype, const void* dy_a, const void* dy_b, void* dx_a, void* dx_b,
+                                int g_dtype, long long rows, long long row0, long long nrows, int C, const float* mean,
+                                const float* invstd, const float* gamma, const float* beta, int relu, int train,
+                                float* dgamma, float* dbeta, int accumulate, double* ws, void* stream);
 /* bits[pixel] bit j = (y[pixel][j] > 0): ReLU mask of a channels-last bf16 tensor with exactly 32 channels, 4 B per pixel
  * (consumed by fmri_conv_dgrad through fmri_relu_mask.bits) */
 int fmri_relu_bitmask(const void* y, int dtype, long long pixels, int C, unsigned* bits, void* stream);

@@ -1581,20 +1581,38 @@ extern "C" int fmri_bn_apply(const void* x, int x_dtype, void* y, int y_dtype, l
     LAUNCH_OK();
     return 0;
 }
+// the channel-pair kernels tile C when a row's channel pairs fill whole 256-thread blocks or divide one evenly
+static bool bn_cp_ok(int C) { return C % 2 == 0 && ((C / 2) >= 256 ? (C / 2) % 256 == 0 : 256 % (C / 2) == 0); }
+// resident CTAs per SM of a BatchNorm-backward kernel (queried once per instantiation): its grid is exactly one wave
+template <typename K>
+static int bn_occupancy(K kernel, int& cache) {
+    if (!cache) {
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cache, kernel, 256, 0) != cudaSuccess) return 0;
+        cache = std::max(1, cache);
+    }
+    return cache;
+}
+static long long bn_cp_rows_per_block(long long rows, int C, int occ) {
+    const int ry = std::max(1, 256 / (C / 2));
+    return std::max<long long>((long long)ry * 16, (rows + 148 * occ - 1) / (148 * occ));
+}
+template <typename Tx, typename Tg>
+static int bn_cp_reduce_per(long long rows, int C, long long* per) {
+    static int occ1 = 0;
+    if (!bn_occupancy(bn_bwd_cp_kernel<1, Tx, Tg>, occ1)) return fail(FMRI_ERR_CUDA, "occupancy query of bn_bwd_cp_kernel");
+    *per = bn_cp_rows_per_block(rows, C, occ1);
+    return 0;
+}
 template <typename Tx, typename Tg>
 static int bn_bwd_reduce_t(const void* x, const void* dy, long long rows, int C, const float* mean, const float* invstd,
                            const float* gamma, const float* beta, int relu, double* ws, cudaStream_t st) {
     const int rpb = rows_per_block_for(rows);
     dim3 grid(cdiv(rows, rpb), std::min(8, cdiv(C, 256)));
     CUDA_OK(cudaMemsetAsync(ws, 0, sizeof(double) * 2 * C, st));
-    if (C % 2 == 0 && ((C / 2) >= 256 ? (C / 2) % 256 == 0 : 256 % (C / 2) == 0)) {
-        const int ry = std::max(1, 256 / (C / 2));
-        static int occ1 = 0;  // resident CTAs per SM of this instantiation: the grid is exactly one wave
-        if (!occ1) {
-            CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ1, bn_bwd_cp_kernel<1, Tx, Tg>, 256, 0));
-            occ1 = std::max(1, occ1);
-        }
-        const long long per = std::max<long long>((long long)ry * 16, (rows + 148 * occ1 - 1) / (148 * occ1));
+    if (bn_cp_ok(C)) {
+        long long per;
+        int rc = bn_cp_reduce_per<Tx, Tg>(rows, C, &per);
+        if (rc) return rc;
         dim3 gcp(cdiv(rows, per), std::max(1, std::min(8, (C / 2) / 256)));
         bn_bwd_cp_kernel<1, Tx, Tg><<<gcp, 256, 0, st>>>(reinterpret_cast<const Tx*>(x), reinterpret_cast<const Tg*>(dy), nullptr,
                                                        rows, C, mean, invstd, gamma, beta, relu, 1, nullptr, nullptr, ws,
@@ -1609,6 +1627,30 @@ static int bn_bwd_reduce_t(const void* x, const void* dy, long long rows, int C,
                                                                     invstd, gamma, beta, relu, ws, ws + C, rpb);
     }
     LAUNCH_OK();
+    return 0;
+}
+// dx = gamma*invstd * (g - mean_g - xhat*mean_gx) over `rows` rows (x, dy, dx point at the first of them)
+template <typename Tx, typename Tg>
+static int bn_bwd_apply_t(const void* x, const void* dy, void* dx, long long rows, int C, const float* mean,
+                          const float* invstd, const float* gamma, const float* beta, int relu, int train,
+                          const float* mean_g, const float* mean_gx, cudaStream_t st) {
+    if (rows == 0) return 0;
+    if (bn_cp_ok(C)) {
+        static int occ2 = 0;
+        if (!bn_occupancy(bn_bwd_cp_kernel<2, Tx, Tg>, occ2)) return fail(FMRI_ERR_CUDA, "occupancy query of bn_bwd_cp_kernel");
+        const long long per = bn_cp_rows_per_block(rows, C, occ2);
+        dim3 gcp(cdiv(rows, per), std::max(1, std::min(8, (C / 2) / 256)));
+        bn_bwd_cp_kernel<2, Tx, Tg><<<gcp, 256, 0, st>>>(reinterpret_cast<const Tx*>(x), reinterpret_cast<const Tg*>(dy),
+                                                       reinterpret_cast<Tg*>(dx), rows, C, mean, invstd, gamma, beta, relu,
+                                                       train, mean_g, mean_gx, nullptr, nullptr, (int)per);
+        LAUNCH_OK();
+    } else {
+        if (C % 8) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward needs C %% 8 == 0");
+        bn_bwd_apply_kernel<Tx, Tg><<<grid1d((rows * C + 7) / 8, 256, 148 * 8), 256, 0, st>>>(
+            reinterpret_cast<const Tx*>(x), reinterpret_cast<const Tg*>(dy), reinterpret_cast<Tg*>(dx), rows * C, C,
+            (double)rows, mean, invstd, gamma, beta, relu, train, mean_g, mean_gx);
+        LAUNCH_OK();
+    }
     return 0;
 }
 template <typename Tx, typename Tg>
@@ -1626,28 +1668,64 @@ static int bn_bwd_t(const void* x, const void* dy, void* dx, long long rows, int
         x = reinterpret_cast<const Tx*>(x) + row0 * C;
         dy = reinterpret_cast<const Tg*>(dy) + row0 * C;
         rows = nrows;
-        if (rows == 0) return 0;
     }
-    if (dx && C % 2 == 0 && ((C / 2) >= 256 ? (C / 2) % 256 == 0 : 256 % (C / 2) == 0)) {
-        const int ry = std::max(1, 256 / (C / 2));
-        static int occ2 = 0;
-        if (!occ2) {
-            CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, bn_bwd_cp_kernel<2, Tx, Tg>, 256, 0));
-            occ2 = std::max(1, occ2);
-        }
-        const long long per = std::max<long long>((long long)ry * 16, (rows + 148 * occ2 - 1) / (148 * occ2));
-        dim3 gcp(cdiv(rows, per), std::max(1, std::min(8, (C / 2) / 256)));
-        bn_bwd_cp_kernel<2, Tx, Tg><<<gcp, 256, 0, st>>>(reinterpret_cast<const Tx*>(x), reinterpret_cast<const Tg*>(dy),
-                                                       reinterpret_cast<Tg*>(dx), rows, C, mean, invstd, gamma, beta, relu,
-                                                       train, mean_g, mean_gx, nullptr, nullptr, (int)per);
-        LAUNCH_OK();
-    } else if (dx) {
-        if (C % 8) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward needs C %% 8 == 0");
-        bn_bwd_apply_kernel<Tx, Tg><<<grid1d((rows * C + 7) / 8, 256, 148 * 8), 256, 0, st>>>(
-            reinterpret_cast<const Tx*>(x), reinterpret_cast<const Tg*>(dy), reinterpret_cast<Tg*>(dx), rows * C, C,
-            (double)rows, mean, invstd, gamma, beta, relu, train, mean_g, mean_gx);
-        LAUNCH_OK();
+    if (!dx) return 0;
+    return bn_bwd_apply_t<Tx, Tg>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train, mean_g, mean_gx, st);
+}
+// Two upstreams a, b through one BatchNorm; dgamma/dbeta (nullable) take upstream a's parameter gradient. dx_a covers all
+// rows, dx_b rows [row0, row0 + nrows). ws: 6*C doubles = [sums a | sums b | fp32 means a | fp32 means b].
+template <typename Tx, typename Tg>
+static int bn_bwd_pair_t(const void* x, const void* dya, const void* dyb, void* dxa, void* dxb, long long rows,
+                         long long row0, long long nrows, int C, const float* mean, const float* invstd, const float* gamma,
+                         const float* beta, int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws,
+                         cudaStream_t st) {
+    if (!bn_cp_ok(C)) {   // shapes the channel-pair kernels do not tile: the two single-upstream passes
+        int rc = bn_bwd_t<Tx, Tg>(x, dya, dxa, rows, C, mean, invstd, gamma, beta, relu, train, dgamma, dbeta, accumulate,
+                                  ws, st);
+        if (rc) return rc;
+        return bn_bwd_t<Tx, Tg>(x, dyb, dxb, rows, C, mean, invstd, gamma, beta, relu, train, nullptr, nullptr, 0, ws + 3 * C,
+                                st, row0, nrows);
     }
+    const Tx* xp = reinterpret_cast<const Tx*>(x);
+    const Tg *ap = reinterpret_cast<const Tg*>(dya), *bp = reinterpret_cast<const Tg*>(dyb);
+    Tg *dap = reinterpret_cast<Tg*>(dxa), *dbp = reinterpret_cast<Tg*>(dxb);
+    // the sums: the grid and rows_per_block of the single-upstream reduce, so that each upstream's partials match it
+    long long per;
+    int rc = bn_cp_reduce_per<Tx, Tg>(rows, C, &per);
+    if (rc) return rc;
+    static int occ2 = 0;   // the apply's grid: one wave of the paired kernel
+    if (!bn_occupancy(bn_bwd_cp2_kernel<2, Tx, Tg>, occ2)) return fail(FMRI_ERR_CUDA, "occupancy query of bn_bwd_cp2_kernel");
+    const int gy = std::max(1, std::min(8, (C / 2) / 256));
+    CUDA_OK(cudaMemsetAsync(ws, 0, sizeof(double) * 4 * C, st));
+    bn_bwd_cp2_kernel<1, Tx, Tg><<<dim3(cdiv(rows, per), gy), 256, 0, st>>>(
+        xp, ap, bp, nullptr, nullptr, rows, C, mean, invstd, gamma, beta, relu, 1, nullptr, nullptr, nullptr, nullptr, ws,
+        ws + C, ws + 2 * C, ws + 3 * C, (int)per);
+    LAUNCH_OK();
+    float* mga = reinterpret_cast<float*>(ws + 4 * C);
+    float* mgxa = mga + C;
+    float* mgb = mgxa + C;
+    float* mgxb = mgb + C;
+    bn_param_grad_kernel<<<cdiv(C, 128), 128, 0, st>>>(ws, ws + C, (double)rows, C, mga, mgxa, dgamma, dbeta, accumulate);
+    LAUNCH_OK();
+    bn_param_grad_kernel<<<cdiv(C, 128), 128, 0, st>>>(ws + 2 * C, ws + 3 * C, (double)rows, C, mgb, mgxb, nullptr, nullptr, 0);
+    LAUNCH_OK();
+    // the apply: upstream a alone outside the slice, both upstreams on it
+    const long long row1 = row0 + nrows;
+    if (row0 > 0) {
+        rc = bn_bwd_apply_t<Tx, Tg>(xp, ap, dap, row0, C, mean, invstd, gamma, beta, relu, train, mga, mgxa, st);
+        if (rc) return rc;
+    }
+    if (row1 < rows) {
+        rc = bn_bwd_apply_t<Tx, Tg>(xp + row1 * C, ap + row1 * C, dap + row1 * C, rows - row1, C, mean, invstd, gamma, beta,
+                                    relu, train, mga, mgxa, st);
+        if (rc) return rc;
+    }
+    if (nrows == 0) return 0;
+    const long long per2 = bn_cp_rows_per_block(nrows, C, occ2);
+    bn_bwd_cp2_kernel<2, Tx, Tg><<<dim3(cdiv(nrows, per2), gy), 256, 0, st>>>(
+        xp + row0 * C, ap + row0 * C, bp + row0 * C, dap + row0 * C, dbp, nrows, C, mean, invstd, gamma, beta, relu, train,
+        mga, mgxa, mgb, mgxb, nullptr, nullptr, nullptr, nullptr, (int)per2);
+    LAUNCH_OK();
     return 0;
 }
 extern "C" int fmri_bn_backward(const void* x, int x_dtype, const void* dy, void* dx, int g_dtype, long long rows, int C,
@@ -1681,6 +1759,44 @@ extern "C" int fmri_bn_backward_slice(const void* x, int x_dtype, const void* dy
         return bn_bwd_t<float, float>(x, dy, dx, rows, C, mean, invstd, gamma, beta, relu, train, dgamma, dbeta,
                                       accumulate, ws, S(stream), row0, nrows);
     return fail(FMRI_ERR_UNSUPPORTED, "bn_backward dtype combination");
+}
+static int bn_pair_entry(const void* x, int x_dtype, const void* dya, const void* dyb, void* dxa, void* dxb, int g_dtype,
+                         long long rows, long long row0, long long nrows, int C, const float* mean, const float* invstd,
+                         const float* gamma, const float* beta, int relu, int train, float* dgamma, float* dbeta,
+                         int accumulate, double* ws, void* stream) {
+    // every argument is checked before the first launch
+    if (C <= 0 || (C < 256 && (256 % C))) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward_pair C=%d", C);
+    if (!bn_cp_ok(C) && C % 8) return fail(FMRI_ERR_UNSUPPORTED, "bn_backward_pair needs C %% 8 == 0");
+    if (rows < 0 || row0 < 0 || nrows < 0 || row0 + nrows > rows) return fail(FMRI_ERR_ARG, "bn_backward_pair: bad row range");
+    if (!x || !dya || !dyb || !dxa || (!dxb && nrows > 0) || !mean || !invstd || !gamma || !beta || !ws)
+        return fail(FMRI_ERR_ARG, "bn_backward_pair: null tensor argument");
+    if (!dgamma != !dbeta) return fail(FMRI_ERR_ARG, "bn_backward_pair: dgamma and dbeta go together");
+    if (dya == dyb || dxa == dxb) return fail(FMRI_ERR_ARG, "bn_backward_pair: the two upstreams need their own buffers");
+    if (x_dtype == FMRI_BF16 && g_dtype == FMRI_BF16)
+        return bn_bwd_pair_t<__nv_bfloat16, __nv_bfloat16>(x, dya, dyb, dxa, dxb, rows, row0, nrows, C, mean, invstd, gamma,
+                                                           beta, relu, train, dgamma, dbeta, accumulate, ws, S(stream));
+    if (x_dtype == FMRI_F32 && g_dtype == FMRI_BF16)
+        return bn_bwd_pair_t<float, __nv_bfloat16>(x, dya, dyb, dxa, dxb, rows, row0, nrows, C, mean, invstd, gamma, beta,
+                                                   relu, train, dgamma, dbeta, accumulate, ws, S(stream));
+    if (x_dtype == FMRI_F32 && g_dtype == FMRI_F32)
+        return bn_bwd_pair_t<float, float>(x, dya, dyb, dxa, dxb, rows, row0, nrows, C, mean, invstd, gamma, beta, relu,
+                                           train, dgamma, dbeta, accumulate, ws, S(stream));
+    return fail(FMRI_ERR_UNSUPPORTED, "bn_backward_pair dtype combination");
+}
+extern "C" int fmri_bn_backward_pair(const void* x, int x_dtype, const void* dy_a, const void* dy_b, void* dx_a, void* dx_b,
+                                     int g_dtype, long long rows, int C, const float* mean, const float* invstd,
+                                     const float* gamma, const float* beta, int relu, int train, float* dgamma,
+                                     float* dbeta, int accumulate, double* ws, void* stream) {
+    return bn_pair_entry(x, x_dtype, dy_a, dy_b, dx_a, dx_b, g_dtype, rows, 0, rows, C, mean, invstd, gamma, beta, relu,
+                         train, dgamma, dbeta, accumulate, ws, stream);
+}
+extern "C" int fmri_bn_backward_pair_slice(const void* x, int x_dtype, const void* dy_a, const void* dy_b, void* dx_a,
+                                           void* dx_b, int g_dtype, long long rows, long long row0, long long nrows, int C,
+                                           const float* mean, const float* invstd, const float* gamma, const float* beta,
+                                           int relu, int train, float* dgamma, float* dbeta, int accumulate, double* ws,
+                                           void* stream) {
+    return bn_pair_entry(x, x_dtype, dy_a, dy_b, dx_a, dx_b, g_dtype, rows, row0, nrows, C, mean, invstd, gamma, beta, relu,
+                         train, dgamma, dbeta, accumulate, ws, stream);
 }
 extern "C" int fmri_relu_backward(const void* y, const void* dy, void* dx, int dtype, long long n, void* stream) {
     if (dtype == FMRI_BF16)

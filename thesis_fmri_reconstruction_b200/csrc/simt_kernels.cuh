@@ -994,6 +994,103 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_cp_kernel(const Tx* __restrict_
     }
 }
 
+// Two upstreams a, b through ONE train-mode BatchNorm (two backward sweeps over the same saved forward state): the backward is
+// linear in its upstream once the forward is fixed, so the two share the reads of x.
+//   MODE 1: sums of both upstreams; reads x, dy_a, dy_b (3 passes instead of 4)
+//   MODE 2: dx_a and dx_b; reads x, dy_a, dy_b, writes dx_a, dx_b (5 passes instead of 6)
+// Per upstream every expression (mask, fmaf order, the row walk of a thread) is that of bn_bwd_cp_kernel: launched with the
+// same grid and rows_per_block, each upstream gets the fp32 partial sums, and dx, of a single-upstream call (a thread still
+// accumulates its rows in row order; batching the loads does not change that order).
+template <int MODE, typename Tx, typename Tg>
+__global__ void __launch_bounds__(256, 4) bn_bwd_cp2_kernel(
+    const Tx* __restrict__ x, const Tg* __restrict__ dya, const Tg* __restrict__ dyb, Tg* __restrict__ dxa,
+    Tg* __restrict__ dxb, long long rows, int C, const float* __restrict__ mean, const float* __restrict__ invstd,
+    const float* __restrict__ gamma, const float* __restrict__ beta, int relu, int train, const float* __restrict__ mga,
+    const float* __restrict__ mgxa, const float* __restrict__ mgb, const float* __restrict__ mgxb,
+    double* __restrict__ sga, double* __restrict__ sgxa, double* __restrict__ sgb, double* __restrict__ sgxb,
+    int rows_per_block) {
+    constexpr int D = 8;                      // rows per load batch
+    const int cp = C >> 1;
+    const int tx_n = cp >= 256 ? 256 : cp;
+    const int ry = 256 / tx_n;
+    const int tx = threadIdx.x % tx_n, ty = threadIdx.x / tx_n;
+    const long long r0 = (long long)blockIdx.x * rows_per_block;
+    const long long r1 = min(rows, r0 + rows_per_block);
+    __shared__ float sred[8][256];
+    for (int pb = blockIdx.y * tx_n; pb < cp; pb += gridDim.y * tx_n) {
+        const int c = (pb + tx) * 2;
+        const bool live = (pb + tx) < cp;
+        float mu0 = 0, mu1 = 0, is0 = 0, is1 = 0, sc0 = 0, sc1 = 0, be0 = 0, be1 = 0;
+        float ka10 = 0, ka11 = 0, ka20 = 0, ka21 = 0, kb10 = 0, kb11 = 0, kb20 = 0, kb21 = 0;
+        if (live) {
+            mu0 = mean[c]; mu1 = mean[c + 1]; is0 = invstd[c]; is1 = invstd[c + 1];
+            sc0 = gamma[c] * is0; sc1 = gamma[c + 1] * is1; be0 = beta[c]; be1 = beta[c + 1];
+            if (MODE == 2 && train) {
+                ka10 = -sc0 * mga[c]; ka11 = -sc1 * mga[c + 1];
+                ka20 = -sc0 * is0 * mgxa[c]; ka21 = -sc1 * is1 * mgxa[c + 1];
+                kb10 = -sc0 * mgb[c]; kb11 = -sc1 * mgb[c + 1];
+                kb20 = -sc0 * is0 * mgxb[c]; kb21 = -sc1 * is1 * mgxb[c + 1];
+            }
+        }
+        float sa0 = 0.f, sa1 = 0.f, qa0 = 0.f, qa1 = 0.f, sb0 = 0.f, sb1 = 0.f, qb0 = 0.f, qb1 = 0.f;
+        // one row of this thread's two channels, both upstreams
+        auto row = [&](long long r, typename Pair<Tx>::Raw xw, typename Pair<Tg>::Raw aw, typename Pair<Tg>::Raw bw) {
+            const float2 xv = Pair<Tx>::cvt(xw), av = Pair<Tg>::cvt(aw), bv = Pair<Tg>::cvt(bw);
+            const float xc0 = xv.x - mu0, xc1 = xv.y - mu1;
+            const bool z0 = relu && !(xc0 * sc0 + be0 > 0.f), z1 = relu && !(xc1 * sc1 + be1 > 0.f);
+            float ga0 = av.x, ga1 = av.y, gb0 = bv.x, gb1 = bv.y;
+            if (z0) { ga0 = 0.f; gb0 = 0.f; }
+            if (z1) { ga1 = 0.f; gb1 = 0.f; }
+            if (MODE == 1) {
+                sa0 += ga0; sa1 += ga1; qa0 = fmaf(ga0, xc0, qa0); qa1 = fmaf(ga1, xc1, qa1);
+                sb0 += gb0; sb1 += gb1; qb0 = fmaf(gb0, xc0, qb0); qb1 = fmaf(gb1, xc1, qb1);
+            } else {
+                Pair<Tg>::st(dxa + r * C + c, fmaf(ga0, sc0, fmaf(xc0, ka20, ka10)), fmaf(ga1, sc1, fmaf(xc1, ka21, ka11)));
+                Pair<Tg>::st(dxb + r * C + c, fmaf(gb0, sc0, fmaf(xc0, kb20, kb10)), fmaf(gb1, sc1, fmaf(xc1, kb21, kb11)));
+            }
+        };
+        if (live) {
+            // batches of D rows: all 3 x D loads of a batch are issued before its math. With three streams a second buffer
+            // for the next batch would not fit 64 registers; 32 resident warps per SM keep the loads of other batches in
+            // flight while one does its math, and 3 x 8 loads per thread outstanding exceed the single kernel's 2 x 8.
+            long long r = r0 + ty;
+#pragma unroll 1
+            for (; r + (D - 1LL) * ry < r1; r += (long long)D * ry) {
+                typename Pair<Tx>::Raw xr[D];
+                typename Pair<Tg>::Raw ar[D], br[D];
+#pragma unroll
+                for (int u = 0; u < D; ++u) {
+                    const long long o = (r + (long long)u * ry) * C + c;
+                    xr[u] = Pair<Tx>::raw(x + o); ar[u] = Pair<Tg>::raw(dya + o); br[u] = Pair<Tg>::raw(dyb + o);
+                }
+#pragma unroll
+                for (int u = 0; u < D; ++u) row(r + (long long)u * ry, xr[u], ar[u], br[u]);
+            }
+            for (; r < r1; r += ry)
+                row(r, Pair<Tx>::raw(x + r * C + c), Pair<Tg>::raw(dya + r * C + c), Pair<Tg>::raw(dyb + r * C + c));
+        }
+        if (MODE == 1) {
+            qa0 *= is0; qa1 *= is1; qb0 *= is0; qb1 *= is1;
+            sred[0][threadIdx.x] = sa0; sred[1][threadIdx.x] = sa1; sred[2][threadIdx.x] = qa0; sred[3][threadIdx.x] = qa1;
+            sred[4][threadIdx.x] = sb0; sred[5][threadIdx.x] = sb1; sred[6][threadIdx.x] = qb0; sred[7][threadIdx.x] = qb1;
+            __syncthreads();
+            if (ty == 0 && live) {
+                for (int l = 1; l < ry; ++l) {
+                    sa0 += sred[0][l * tx_n + tx]; sa1 += sred[1][l * tx_n + tx];
+                    qa0 += sred[2][l * tx_n + tx]; qa1 += sred[3][l * tx_n + tx];
+                    sb0 += sred[4][l * tx_n + tx]; sb1 += sred[5][l * tx_n + tx];
+                    qb0 += sred[6][l * tx_n + tx]; qb1 += sred[7][l * tx_n + tx];
+                }
+                atomicAdd(sga + c, (double)sa0); atomicAdd(sga + c + 1, (double)sa1);
+                atomicAdd(sgxa + c, (double)qa0); atomicAdd(sgxa + c + 1, (double)qa1);
+                atomicAdd(sgb + c, (double)sb0); atomicAdd(sgb + c + 1, (double)sb1);
+                atomicAdd(sgxb + c, (double)qb0); atomicAdd(sgxb + c + 1, (double)qb1);
+            }
+            __syncthreads();
+        }
+    }
+}
+
 // per channel, once: the fp32 means the apply pass needs (one fp64 division per CHANNEL instead of per thread) and the
 // parameter gradients dgamma = sum(g*xhat), dbeta = sum(g) (nullable)
 __global__ void bn_param_grad_kernel(const double* __restrict__ sum_g, const double* __restrict__ sum_gx, double count,

@@ -240,7 +240,10 @@ class VaeGanStage1(_TrainerBase):
         return NN.Ctx(B=B, x=x, eps=eps, ce=ce, cd1=cd1, cd2=cd2, cc=cc, raw3=raw3, p=p, mu=mu, lv=lv, out=out)
 
     def backward(self, st):
-        """The three used gradients (SURVEY.md 0-7) from the saved forward state, as four sweeps."""
+        """The three used gradients (SURVEY.md 0-7) from the saved forward state. Four sweeps, run as two paired ones: the
+        discriminator's class path (1) and feature tap (2), and the decoder's sweeps (3) and (4) on decoder call 1, each walk
+        back through one saved forward state, and train-mode BatchNorm is linear in its upstream once that state is fixed, so
+        each pair shares every BatchNorm backward (x read once for both upstreams) and stacks its data gradients."""
         if self.mode in ("dcgan", "vae"):
             return self._backward_pixel_nle(st)
         hp, B = self.hp, st.B
@@ -253,19 +256,18 @@ class VaeGanStage1(_TrainerBase):
         ones = self._ones(3 * B)
         L.bce_bwd(p[:B], ones, gp[:B], B, True, 1.0)
         L.bce_bwd(p[B:], ones, gp[B:], 2 * B, False, 1.0)
-        dimg_bce = self.dis.backward_gan(bc.P, cc, gp, bc.G, False, True, (1, 3))
-        self._allreduce_async([bc.flat_g])
         # (2) discriminator, feature-tap path: d sum(mse) / d x_tilde (data gradient only; BN couples the whole 3B batch)
         draw3 = torch.empty_like(raw3)
         draw3[2 * B:].zero_()
         L.rowsqdiff_bwd(raw3[:B], raw3[B:2 * B], ones, draw3[:B], draw3[B:2 * B], B, Fd, 0.5)
-        dimg_mse = self.dis.backward_rec(bc.P, cc, draw3, None, False, False, (1, 2), live=(0, 2))
-        # (3) decoder: g_dec = d [lambda * mse - (1 - lambda) * loss_dis] / d decoder over both decoder calls
-        self.dec.backward(bd.P, cd1, lam, dimg_mse, -(1.0 - lam), dimg_bce[:B], bd.G, False, True, False)
+        dimg_bce, dimg_mse = self.dis.backward_pair(bc.P, cc, gp, draw3, bc.G, False, live=(0, 2),
+                                                    after_dw=lambda: self._allreduce_async([bc.flat_g]))
+        # (3) decoder: g_dec = d [lambda * mse - (1 - lambda) * loss_dis] / d decoder over both decoder calls, paired on call 1
+        # with (4): the mse term flows x_tilde -> decoder (data gradient) -> z. Call 1 accumulates first, as in four sweeps.
+        dz = self.dec.backward_pair(bd.P, cd1, lam, dimg_mse, -(1.0 - lam), dimg_bce[:B], 1.0, dimg_mse, bd.G, False)
         self.dec.backward(bd.P, cd2, -(1.0 - lam), dimg_bce[B:], 0.0, None, bd.G, True, True, False)
         self._ev_dec = self._allreduce_async([bd.flat_g])   # loss sums, discriminator and decoder buckets are reduced here
-        # (4) encoder: g_enc = d [sum kl + sum mse] / d encoder; the mse term flows x_tilde -> decoder (data gradient) -> z
-        dz = self.dec.backward(bd.P, cd1, 1.0, dimg_mse, 0.0, None, None, False, False, True)
+        # (4, continued) encoder: g_enc = d [sum kl + sum mse] / d encoder
         dycat = self._encoder_backward(st, dz)
         st.sweeps = dict(dimg_bce=dimg_bce, dimg_mse=dimg_mse, dz=dz, dycat=dycat)
 

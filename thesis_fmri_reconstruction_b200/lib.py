@@ -340,6 +340,31 @@ def bn_backward_slice(x, dy, dx, rows, row0, nrows, Cc, mean, invstd, gamma, bet
                                          0, ptr(ws), stream()))
 
 
+def _same_grad_dtype(*ts):
+    if len({t.dtype for t in ts if t is not None}) > 1:
+        raise FmriError("the two upstreams and their gradients share one dtype")
+
+
+def bn_backward_pair(x, dya, dyb, dxa, dxb, rows, Cc, mean, invstd, gamma, beta, relu, train, dgamma, dbeta, accumulate, ws):
+    """Two upstreams through one BatchNorm (x read once for both); dgamma / dbeta take upstream a's. ws: 6*C doubles."""
+    _same_grad_dtype(dya, dyb, dxa, dxb)
+    _require_cuda(x, dya, dyb, dxa, dxb, mean, invstd, gamma, beta, dgamma, dbeta, ws)
+    _check(load().fmri_bn_backward_pair(ptr(x), dt(x), ptr(dya), ptr(dyb), ptr(dxa), ptr(dxb), dt(dya), _ll(rows), Cc,
+                                        ptr(mean), ptr(invstd), ptr(gamma), ptr(beta), int(relu), int(train), ptr(dgamma),
+                                        ptr(dbeta), int(accumulate), ptr(ws), stream()))
+
+
+def bn_backward_pair_slice(x, dya, dyb, dxa, dxb, rows, row0, nrows, Cc, mean, invstd, gamma, beta, relu, train, dgamma,
+                           dbeta, accumulate, ws):
+    """bn_backward_pair with upstream b's dx produced for rows [row0, row0 + nrows) only (dxb holds just those rows)."""
+    _same_grad_dtype(dya, dyb, dxa, dxb)
+    _require_cuda(x, dya, dyb, dxa, dxb, mean, invstd, gamma, beta, dgamma, dbeta, ws)
+    _check(load().fmri_bn_backward_pair_slice(ptr(x), dt(x), ptr(dya), ptr(dyb), ptr(dxa), ptr(dxb), dt(dya), _ll(rows),
+                                              _ll(row0), _ll(nrows), Cc, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta),
+                                              int(relu), int(train), ptr(dgamma), ptr(dbeta), int(accumulate), ptr(ws),
+                                              stream()))
+
+
 def relu_backward(y, dy, dx):
     _require_cuda(y, dy, dx)
     _check(load().fmri_relu_backward(ptr(y), ptr(dy), ptr(dx), dt(y), _ll(y.numel()), stream()))

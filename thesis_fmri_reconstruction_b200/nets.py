@@ -60,7 +60,7 @@ class BatchNorm:
 
     def __init__(self, prefix, C):
         self.prefix, self.C = prefix, C
-        self._ws = None
+        self._ws = self._ws2 = None
 
     def names(self):
         return [self.prefix + "weight", self.prefix + "bias"]
@@ -96,6 +96,24 @@ class BatchNorm:
                       c.train, G[pre + "weight"] if need_dw else None, G[pre + "bias"] if need_dw else None, acc,
                       self._ws)
         return draw
+
+    def backward_pair(self, P, c, dya, dyb, G, acc, need_dw, rows_b=None):
+        """Two upstreams through this layer with the forward tensor read once for both (the layer is linear in its upstream).
+        Parameter gradients come from upstream a. rows_b = (row0, nrows): upstream b's gradient for those rows only.
+        Returns one buffer holding d(raw) of a, then of b, stacked along the leading (batch) dimension."""
+        C, pre = self.C, self.prefix
+        if self._ws2 is None:
+            self._ws2 = E(6 * C, dtype=F64)
+        lead, per = c.raw.shape[0], c.rows // c.raw.shape[0]
+        row0, nb = rows_b if rows_b is not None else (0, c.rows)
+        out = torch.empty((lead + nb // per,) + tuple(c.raw.shape[1:]), dtype=dya.dtype, device=dya.device)
+        args = (C, c.mean, c.invstd, P[pre + "weight"], P[pre + "bias"], c.relu, c.train,
+                G[pre + "weight"] if need_dw else None, G[pre + "bias"] if need_dw else None, acc, self._ws2)
+        if rows_b is None:
+            L.bn_backward_pair(c.raw, dya, dyb, out[:lead], out[lead:], c.rows, *args)
+        else:
+            L.bn_backward_pair_slice(c.raw, dya, dyb, out[:lead], out[lead:], c.rows, row0, nb, *args)
+        return out
 
 
 # ====================================================================================================== conv blocks
@@ -138,6 +156,17 @@ class ConvBlock:
         """relu_mask: (y, bits) of the bias+ReLU layer BELOW, whose ReLU backward this layer's data-gradient kernel applies."""
         draw = self.bn.backward(P, c.bn, dy, G, acc, need_dw)
         return self.backward_raw(P, c, draw, G, acc, need_dw, need_dx, relu_mask)
+
+    def backward_pair(self, P, c, dya, dyb, G, acc, need_dw):
+        """Two upstreams through this block's saved forward state: one BatchNorm backward for both, one data-gradient launch
+        over the two stacked along the batch, the weight gradient from upstream a. Returns dx of a, then of b, stacked
+        [2N, H, W, Cin]."""
+        N = c.d.N
+        draw = self.bn.backward_pair(P, c.bn, dya, dyb, G, acc, need_dw)
+        dx = E(2 * N, c.d.H, c.d.W, self.Cin, dtype=self.adt)
+        L.conv_dgrad(self.desc(2 * N, c.d.H, c.d.W), draw, P[self.prefix + "conv.weight"], c.pack_d, dx)
+        self.backward_raw(P, c, draw[:N], G, acc, need_dw, False)
+        return dx
 
     def backward_dx_slice(self, P, c, dy, n0, n1, relu_mask=None):
         """Data gradient only, for images [n0, n1) of the batch. Train-mode BatchNorm couples all samples through its two
@@ -372,6 +401,19 @@ class LinearBlock:
             self.lin.dgrad(P, draw, self.N, c.M, dx, self.K, packs=c.packs)
         return dx
 
+    def backward_pair(self, P, c, dya, dyb, G, acc, dx_dtype=None):
+        """Upstream a -> the parameter gradients, upstream b -> the input gradient, with one BatchNorm backward for both."""
+        M = c.M
+        draw = self.bn.backward_pair(P, c.bn, dya, dyb, G, acc, True)
+        if draw.dtype != self.adt:
+            t = E(2 * M, self.N, dtype=self.adt)
+            L.cast2d(draw, self.N, t, self.N, 2 * M, self.N)
+            draw = t
+        self.lin.wgrad(c.x, c.ldx, draw[:M], self.N, M, G, acc)
+        dx = E(M, self.K, dtype=dx_dtype or self.adt)
+        self.lin.dgrad(P, draw[M:], self.N, M, dx, self.K, packs=c.packs)
+        return dx
+
 
 class LatentHeads:
     """l_mu / l_var (vae_gan.py:84-85, 206-207): two Linear(1024, z) + bias writing the halves of one [B, 2z] fp32 matrix."""
@@ -564,6 +606,29 @@ class DecoderNet:
         L.nhwc_to_nchw(dy, dflat, B, self.size, f, f)
         return self.fc.backward(P, c.fc, dflat, G, acc, need_dw, need_dz, dx_dtype=F32)
 
+    def backward_pair(self, P, c, a, gx, b, gy, a2, gx2, G, acc=False):
+        """Two sweeps through one saved forward state: upstream (a*gx + b*gy) -> parameter gradients into G, upstream a2*gx2
+        -> dz. The same as backward(P, c, a, gx, b, gy, G, acc, True, False) followed by backward(P, c, a2, gx2, 0, None, None,
+        need_dw=False, need_dz=True), with every BatchNorm backward shared by the two and every data gradient run once over
+        the two upstreams stacked along the batch (the 3-channel output conv's data gradient stays two launches: its kernel
+        does not give the same bits for a doubled batch at every size). Returns dz [B, z] fp32."""
+        B = c.B
+        h, w = c.hw
+        dpre = E(2 * B, 3, h, w)
+        L.axpby_tanh_bwd(a, gx, b, gy, c.img, dpre[:B])
+        L.axpby_tanh_bwd(a2, gx2, 0.0, None, c.img, dpre[B:])
+        L.chansum_nchw(dpre[:B], B, 3, h * w, G["conv.3.0.bias"], acc)
+        L.edge_out_wgrad(c.d3, c.a3, dpre[:B], G["conv.3.0.weight"], acc, self._ews)
+        dy = E(2 * B, h, w, self.Cl, dtype=self.adt)
+        L.edge_out_dgrad(c.d3, dpre[:B], P["conv.3.0.weight"], dy[:B], self._ews)
+        L.edge_out_dgrad(c.d3, dpre[B:], P["conv.3.0.weight"], dy[B:], self._ews)
+        for i in range(len(self.blocks) - 1, -1, -1):
+            dy = self.blocks[i].backward_pair(P, c.blocks[i], dy[:B], dy[B:], G, acc, True)
+        f = self.fi
+        dflat = E(2 * B, self.size * f * f, dtype=self.adt)
+        L.nhwc_to_nchw(dy, dflat, 2 * B, self.size, f, f)
+        return self.fc.backward_pair(P, c.fc, dflat[:B], dflat[B:], G, acc, dx_dtype=F32)
+
 
 # ====================================================================================================== Discriminator
 class DiscriminatorNet:
@@ -669,6 +734,63 @@ class DiscriminatorNet:
             L.nchw_to_nhwc(dflat, dy, N, self.Cl, h, w)
         dy = _backward_chain(self.blocks, c.blocks, P, dy, G, acc, need_dw, (c.y0, c.mask0))
         return self._conv0_backward(P, c, dy, G, acc, need_dw, img_slices)
+
+    def backward_pair(self, P, c, gp, draw3, G, acc=False, live=(0, 2), after_dw=None):
+        """The class path (backward_gan with img_slices=(1, 3)) and the feature tap of recon_level 3 (backward_rec with
+        need_dw=False, img_slices=(1, 2)) in one sweep over the saved forward state of three sources: below the tap both
+        upstreams share every BatchNorm backward, and block 2's data gradient runs once over the two. after_dw(): called once the last weight gradient is issued. Returns (image gradient of the class path for
+        sources 1 and 2 [2Bs, 3, H, W], image gradient of the feature tap for source 1 [Bs, 3, H, W])."""
+        if self.level != 3 or len(c.imgs) != 3:
+            raise L.FmriError("the paired discriminator sweep needs recon_level 3 and three image sources")
+        Bs, N = c.Bs, c.N
+        (b1, b2, b3), (c1, c2, c3) = self.blocks, c.blocks
+        dh = E(N, self.F, dtype=self.adt)
+        if not acc:
+            G["fc.3.weight"].zero_()
+            G["fc.3.bias"].zero_()
+        L.head_sigmoid_bwd(c.hfc, P["fc.3.weight"], c.p, gp, dh, G["fc.3.weight"], G["fc.3.bias"], N, self.F)
+        dflat = self.fc.backward(P, c.fc, dh, G, acc, True, True)
+        h, w = c.hw
+        if self.fc.nhwc_in:
+            dy = dflat.view(N, h, w, self.Cl)
+        else:
+            dy = E(N, h, w, self.Cl, dtype=self.adt)
+            L.nchw_to_nhwc(dflat, dy, N, self.Cl, h, w)
+        # block 3: the class path through its BatchNorm; the feature tap enters at its raw conv output, live sources only
+        dy2 = E(2 * N, c3.d.H, c3.d.W, b3.Cin, dtype=self.adt)
+        dy2b = dy2[N:]
+        draw =b3.bn.backward(P, c3.bn, dy, G, acc, True)
+        w3 = P[b3.prefix + "conv.weight"]
+        L.conv_dgrad(c3.d, draw, w3, c3.pack_d, dy2[:N])
+        b3.backward_raw(P, c3, draw, G, acc, True, False)
+        l0, l1 = live
+        if l0 > 0:
+            dy2b[:l0 * Bs].zero_()
+        if l1 < 3:
+            dy2b[l1 * Bs:].zero_()
+        L.conv_dgrad(b3.desc((l1 - l0) * Bs, c3.d.H, c3.d.W), draw3[l0 * Bs:l1 * Bs], w3, c3.pack_d, dy2b[l0 * Bs:l1 * Bs])
+        # block 2: both upstreams
+        dy1 = b2.backward_pair(P, c2, dy2[:N], dy2b, G, acc, True)
+        # block 1: the class path over all N images, the feature tap on source 1 only (the BatchNorm sums of both run over N)
+        per = c1.OH * c1.OW
+        draw = b1.bn.backward_pair(P, c1.bn, dy1[:N], dy1[N:], G, acc, True, rows_b=(Bs * per, Bs * per))
+        OH, OW = c.hw0
+        dy0 = E(N + Bs, OH, OW, self.C0, dtype=self.adt)
+        w1 = P[b1.prefix + "conv.weight"]
+        L.conv_dgrad(c1.d, draw[:N], w1, c1.pack_d, dy0[:N], (c.y0, c.mask0))
+        bits = c.mask0[Bs * OH * OW:2 * Bs * OH * OW] if c.mask0 is not None else None
+        L.conv_dgrad(b1.desc(Bs, c1.d.H, c1.d.W), draw[N:], w1, c1.pack_d, dy0[N:], (c.y0[Bs:2 * Bs], bits))
+        b1.backward_raw(P, c1, draw[:N], G, acc, True, False)
+        # conv[0]: weight gradient of the class path, image gradients of its sources 1, 2 and of the feature tap's source 1
+        # (two launches: the edge kernel does not give the same bits for the merged 3Bs rows at every batch size)
+        L.edge_in_wgrad(c.d0, c.imgs, Bs, dy0[:N], G["conv.0.0.weight"], acc, self._ews, G["conv.0.0.bias"])
+        if after_dw is not None:
+            after_dw()
+        dimg = E(N, 3, c.H, c.W)
+        w0 = P["conv.0.0.weight"]
+        for n, src, dst in ((2 * Bs, dy0[Bs:N], dimg[:2 * Bs]), (Bs, dy0[N:], dimg[2 * Bs:])):
+            L.edge_in_dgrad(L.edge_desc(n, c.H, c.W, self.C0, self.stride0, self.adt), src, w0, dst, self._ews)
+        return dimg[:2 * Bs], dimg[2 * Bs:]
 
     def backward_rec(self, P, c, draw3, G=None, acc=False, need_dw=False, img_slices=None, live=None):
         """Backward of the feature-tap path from a gradient on the raw conv output of block 3 [N,h,w,C] (adt).
