@@ -26,10 +26,6 @@ from .dp import FlatBucket
 from .nets import BF16, F32, E, Z
 
 
-def Bucket(prefix, named_params, n_states):
-    return FlatBucket(prefix, named_params, n_states, "cuda")
-
-
 def _split(full, prefix):
     return OrderedDict((k[len(prefix):], v) for k, v in full.items() if k.startswith(prefix))
 
@@ -49,7 +45,25 @@ class _TrainerBase:
             self.t_dev = torch.zeros(1, dtype=torch.int32, device="cuda")
         self.t_dev.fill_(int(v))
 
-    def _setup_dist(self, dist_group):
+    def _setup(self, params, buffers, nets, n_states, lr, dist_group):
+        """Device state of a trainer of `nets` (prefix -> network, in bucket order): one flat bucket per network with its
+        reference-named parameters and n_states[prefix] optimizer-state buffers, learning rates `lr`, device copies of the
+        BatchNorm buffers, 16 loss-sum / gate slots `sc`, the exchange state and the operand packs."""
+        self.nets = nets
+        self.buckets = OrderedDict()
+        for pre, net in nets.items():
+            named = _split(params, pre)
+            diff = set(net.param_names()) ^ set(named)
+            if diff:
+                raise L.FmriError(f"parameter names of {pre} differ from the reference layout: {sorted(diff)}")
+            self.buckets[pre] = FlatBucket(pre, OrderedDict((k, named[k].to("cuda", F32)) for k in named), n_states[pre],
+                                           "cuda")
+        self.S = OrderedDict((k, v.to("cuda").clone()) for k, v in buffers.items())
+        self.Ssub = {pre: _split(self.S, pre) for pre in self.buckets}
+        self.nbt = {}
+        self.sc = Z(16)
+        self.lr = lr
+        self._ones_buf = None
         self.dist = dist_group
         self.world = 1
         if dist_group is not None:
@@ -58,6 +72,43 @@ class _TrainerBase:
             self.td = td
             self.world = td.get_world_size(group=dist_group)
             self.comm_stream = torch.cuda.Stream()
+        self.refresh()
+
+    def refresh(self):
+        """Re-derive the bf16 operand packs from the fp32 master weights."""
+        for pre, net in self.nets.items():
+            net.refresh(self.buckets[pre].P, inplace=True)
+
+    def _ones(self, n):
+        """At least n fp32 ones on the device: the upstream gradient of a loss sum."""
+        if self._ones_buf is None or self._ones_buf.numel() < n:
+            self._ones_buf = torch.ones(n, device="cuda")
+        return self._ones_buf
+
+    def _count_bn_updates(self, pre, counts):
+        """Add one forward's BatchNorm running-statistics updates (name -> count, names under `pre`) to the pending
+        num_batches_tracked increments. Reads self.nbt on every call: GraphedStep swaps it around a capture."""
+        for k, v in counts.items():
+            self.nbt[pre + k] = self.nbt.get(pre + k, 0) + v
+
+    def _latent_d_phase(self, net, b, z_real, z_fake, scale, sums):
+        """Discriminator phase of a latent WaeDiscriminator `net` (bucket `b`): L_fake = -scale sum log(d(z_fake) + 1e-3)
+        into sums[0], L_real = -scale sum log(1 - d(z_real) + 1e-3) into sums[1], and their gradient in b.G.
+        Returns d(z_real), d(z_fake) and the [2B] loss / score-gradient scratch, which the G-phase reuses."""
+        B = z_real.shape[0]
+        ones = self._ones(B)
+        p_real, cr = net.forward(b.P, z_real)
+        p_fake, cf = net.forward(b.P, z_fake)
+        l, gp = E(2 * B), E(2 * B)
+        L.bce_fwd(p_fake, l[:B], B, True, scale)
+        L.bce_fwd(p_real, l[B:], B, False, scale)
+        L.vecsum(l[:B], B, 1.0, sums[0:1])
+        L.vecsum(l[B:], B, 1.0, sums[1:2])
+        L.bce_bwd(p_fake, ones, gp[:B], B, True, scale)
+        L.bce_bwd(p_real, ones, gp[B:], B, False, scale)
+        net.backward(b.P, cf, gp[:B], b.G, False, True, False)
+        net.backward(b.P, cr, gp[B:], b.G, True, True, False)
+        return p_real, p_fake, l, gp
 
     def _allreduce_async(self, tensors):
         """SUM all-reduce on the side stream, ordered after everything issued so far on the compute stream."""
@@ -125,11 +176,7 @@ class _TrainerBase:
         self.hp.update(sd["hp"])
         if self.t_dev is not None:
             self.t = int(sd["t"])
-        if hasattr(self, "nets"):
-            for pre, net in self.nets.items():
-                net.refresh(self.buckets[pre].P, inplace=True)
-        if hasattr(self, "refresh"):
-            self.refresh()
+        self.refresh()
 
     def named_parameters(self):
         out = OrderedDict()
@@ -160,6 +207,7 @@ class VaeGanStage1(_TrainerBase):
     gate=False applies the mix's own flags without the gate: 'vae' trains the decoder only, every other mix trains both."""
 
     MODES = ("vae-gan", "beta-vae", "dcgan", "vae")
+    LATENT_DISCRIMINATOR = False
 
     def __init__(self, params, buffers, cfg, z=128, adt=BF16, hp=None, dist_group=None, gate=True, mode="vae-gan", beta=1.0):
         from .hp import HP_VGAN
@@ -174,26 +222,13 @@ class VaeGanStage1(_TrainerBase):
         self.enc = NN.EncoderNet(cfg, z, adt)
         self.dec = NN.DecoderNet(cfg, z, adt)
         self.dis = NN.DiscriminatorNet(cfg, adt)
-        dev = torch.device("cuda")
-        self.buckets = OrderedDict()
-        for pre, net in (("encoder.", self.enc), ("decoder.", self.dec), ("discriminator.", self.dis)):
-            named = _split(params, pre)
-            missing = set(net.param_names()) ^ set(named)
-            if missing:
-                raise L.FmriError(f"parameter names of {pre} differ from the reference layout: {sorted(missing)}")
-            self.buckets[pre] = Bucket(pre, OrderedDict((k, named[k].to(dev, F32)) for k in named), 1)
-        self.S = OrderedDict((k, v.to(dev).clone()) for k, v in buffers.items())
-        self.Ssub = {pre: _split(self.S, pre) for pre in self.buckets}
-        self.nbt = {}
-        self.sc = Z(16)      # [0..5] = sum bce_o, bce_p, bce_s, kl, mse, nle ; [8],[9] = gates (train_dis, train_dec)
-        self.lr = {pre: float(self.hp["lr"]) for pre in self.buckets}
-        self._setup_dist(dist_group)
-        self.refresh()
-
-    def refresh(self):
-        """Re-derive the bf16 operand packs from the fp32 master weights (after every optimizer step)."""
-        for pre, net in (("encoder.", self.enc), ("decoder.", self.dec), ("discriminator.", self.dis)):
-            net.refresh(self.buckets[pre].P, inplace=True)
+        nets = OrderedDict((("encoder.", self.enc), ("decoder.", self.dec), ("discriminator.", self.dis)))
+        if self.LATENT_DISCRIMINATOR:
+            self.ldis = NN.WaeDiscriminatorNet(z, adt)
+            nets["latent_discriminator."] = self.ldis
+        self._ev_dec = None   # exchange of the loss sums, discriminator and decoder, issued by backward()
+        # sc: [0..5] = sum bce_o, bce_p, bce_s, kl, mse, nle ; [8],[9] = gates (train_dis, train_dec)
+        self._setup(params, buffers, nets, dict.fromkeys(nets, 1), dict.fromkeys(nets, float(self.hp["lr"])), dist_group)
 
     def forward_backward(self, x, eps, z_p):
         """x [B,3,H,W] fp32 NCHW, eps / z_p [B,z] fp32, all on the device. Leaves gradients in the buckets' flat_g and the
@@ -218,8 +253,7 @@ class VaeGanStage1(_TrainerBase):
         x_p, cd2 = self.dec.forward(bd.P, Sd, z_p, True, 1, nbd)
         raw3, p, cc = self.dis.forward(bc.P, Sc, [x, x_tilde, x_p], True, 2, True, nbc)  # REC + GAN passes -> 2 BN updates
         for pre, d in (("encoder.", nbe), ("decoder.", nbd), ("discriminator.", nbc)):
-            for k, v in d.items():
-                self.nbt[pre + k] = self.nbt.get(pre + k, 0) + v
+            self._count_bn_updates(pre, d)
         # ------------------------------------------------------------------ losses (vae_gan.py:302-320, stage1 :369-372)
         Fd = raw3[0].numel()
         mse, nle = E(B), E(B)
@@ -334,11 +368,6 @@ class VaeGanStage1(_TrainerBase):
     def _before_encoder_backward(self, mu, dycat):
         pass
 
-    def _ones(self, n):
-        if getattr(self, "_ones_buf", None) is None or self._ones_buf.numel() < n:
-            self._ones_buf = torch.ones(n, device="cuda")
-        return self._ones_buf
-
     def update(self, B_global):
         """Equilibrium gate (device side) + the three RMSprop updates (train_vgan_stage1.py:396-432), then repack."""
         hp = self.hp
@@ -346,7 +375,7 @@ class VaeGanStage1(_TrainerBase):
         # the gate, their two updates and their repacks run while the last exchange (the encoder's conv part, issued after the
         # final backward kernel: 0.2 ms exposed at 8 GPUs in profiles/r2_nccl_overlap_N8_B512_per_rank.txt) is still in flight;
         # only the encoder update waits for it. The three buckets are independent, so the order changes nothing numerically.
-        ev = getattr(self, "_ev_dec", None)
+        ev = self._ev_dec
         staged = self.world > 1 and ev is not None
         if staged:
             NN.join_side()
@@ -361,7 +390,6 @@ class VaeGanStage1(_TrainerBase):
         else:
             gates[0:1].fill_(1.0 if dis_in else 0.0)
             gates[1:2].fill_(1.0)
-        nets = {"encoder.": self.enc, "decoder.": self.dec, "discriminator.": self.dis}
         for pre, g in (("decoder.", gates[1:2]), ("discriminator.", gates[0:1]), ("encoder.", None)):
             if pre == "encoder." and self.mode == "dcgan":
                 continue   # :374-380 trains no encoder: its parameters, square_avg and operand packs stay as they are
@@ -370,7 +398,7 @@ class VaeGanStage1(_TrainerBase):
             b = self.buckets[pre]
             L.multi_tensor_rmsprop([b.flat_p], [b.flat_g], [b.states[0]], self.lr[pre], hp["alpha"], hp["eps"], 0.0,
                                    None, g)
-            nets[pre].refresh(b.P, inplace=True)
+            self.nets[pre].refresh(b.P, inplace=True)
 
     def step(self, x, eps, z_p):
         """One full training iteration on device-resident inputs. Returns the device tensor of loss sums."""
@@ -382,21 +410,49 @@ class VaeGanStage1(_TrainerBase):
         """Host view of the last step's (globally reduced) loss sums, as the reference logs them (stage1 :391-394)."""
         s = self.sc.tolist()
         lam = float(self.hp["lambda_mse"])
-        mode = getattr(self, "mode", "vae-gan")
-        if mode in ("dcgan", "vae"):   # train_vgan_stage1.py:374-387 (the 'dcgan' loss_encoder is logged, not trained)
+        if self.mode in ("dcgan", "vae"):   # train_vgan_stage1.py:374-387 (the 'dcgan' loss_encoder is logged, not trained)
             loss_dis = s[0] + s[2]
             loss_enc = s[3] + s[5]
-            loss_dec = lam * s[5] - ((1 - lam) * loss_dis if mode == "dcgan" else 0.0)
+            loss_dec = lam * s[5] - ((1 - lam) * loss_dis if self.mode == "dcgan" else 0.0)
         else:
             loss_dis = s[0] + s[1] + s[2]
-            loss_enc = getattr(self, "_klw", 1.0) * s[3] + s[4]
+            loss_enc = self._klw * s[3] + s[4]
             loss_dec = lam * s[4] - (1 - lam) * loss_dis
         return dict(loss_encoder=loss_enc, loss_discriminator=loss_dis, loss_decoder=loss_dec,
                     nle=s[5], bce_o=s[0], bce_p=s[1], bce_s=s[2], kl=s[3], mse=s[4], train_dis=s[8] != 0,
                     train_dec=s[9] != 0)
 
 
-class WaeGanStage1(_TrainerBase):
+class _WaeTrainer(_TrainerBase):
+    """The Adam-trained WAE trainers: buckets "encoder." (the encoder that gives the latent z), "decoder." and the latent
+    "discriminator."; sc[0..3] = L_fake, L_real, L_rec, L_pen."""
+
+    def _adam(self, pre):
+        b, hp = self.buckets[pre], self.hp
+        L.multi_tensor_adam_dev([b.flat_p], [b.flat_g], [b.states[0]], [b.states[1]], self.lr[pre], hp["beta1"], hp["beta2"],
+                                hp["eps"], self.t_dev)
+        self.nets[pre].refresh(b.P, inplace=True)
+
+    def _encoder_tail(self, ce, dmu):
+        """End of the G-phase: the encoder sweep from dmu = d loss / d z (fp32 [B, z]; l_var receives no gradient), its
+        exchange together with the loss sums, and the encoder's Adam step."""
+        B, z = dmu.shape[0], self.z
+        be = self.buckets["encoder."]
+        dycat = Z(B, 2 * z, dtype=self.adt)
+        L.cast2d(dmu, z, dycat[:, :z], 2 * z, B, z)
+        be.flat_g.zero_()  # l_var receives no gradient (logvar unused): its slots stay zero and Adam leaves it unchanged
+        self.nets["encoder."].backward(be.P, ce, dycat, be.G, False, True, False)
+        self._allreduce_async([be.flat_g, self.sc[:8]])
+        self._wait_comm()
+        self._adam("encoder.")
+
+    def losses(self):
+        s = self.sc.tolist()
+        return dict(loss_discriminator_fake=s[0], loss_discriminator_real=s[1], loss_reconstruction=s[2],
+                    loss_penalty=s[3])
+
+
+class WaeGanStage1(_WaeTrainer):
     """Stage-I WAE/GAN trainer (/root/reference/train/train_wae_stage1.py:259-311): visual Encoder, Decoder, latent
     WaeDiscriminator, three Adam(betas=(0.5, 0.999)) optimizers (the discriminator at lr / 2).
 
@@ -405,6 +461,10 @@ class WaeGanStage1(_TrainerBase):
     second time on unchanged weights (:296) -- same z_real, so it is computed once and the BN running statistics are
     updated twice; x_recon = decoder(z_real), d(z_real) with the UPDATED discriminator, L_rec = sum 0.5 (x_recon - x)^2,
     L_pen = -10 sum log(d + 1e-3); Adam on the encoder (grad of L_rec + L_pen; l_var gets none) and the decoder (L_rec).
+
+    penalty='mmd' (EXTENSION, parity unpinned: the reference has no MMD, SURVEY.md 0-3): no latent discriminator and no
+    D-phase; L_pen = lambda_mmd * B * MMD_IMQ(z_real, z_fake) over this rank's batch (per-rank, like BatchNorm), one encoder
+    forward. Everything else as train_wae_stage1.py:292-311.
     """
 
     def __init__(self, params, buffers, cfg, z=128, adt=BF16, hp=None, dist_group=None, penalty="gan", lambda_mmd=10.0,
@@ -418,138 +478,63 @@ class WaeGanStage1(_TrainerBase):
         self.hp = dict(HP_WAE if hp is None else hp)
         self.enc = NN.EncoderNet(cfg, z, adt)
         self.dec = NN.DecoderNet(cfg, z, adt)
-        dev = torch.device("cuda")
-        self.buckets = OrderedDict()
-        self.nets = OrderedDict((("encoder.", self.enc), ("decoder.", self.dec)))
+        nets = OrderedDict((("encoder.", self.enc), ("decoder.", self.dec)))
         if penalty == "gan":
             self.dis = NN.WaeDiscriminatorNet(z, adt)
-            self.nets["discriminator."] = self.dis
-        for pre, net in self.nets.items():
-            named = _split(params, pre)
-            diff = set(net.param_names()) ^ set(named)
-            if diff:
-                raise L.FmriError(f"parameter names of {pre} differ from the reference layout: {sorted(diff)}")
-            self.buckets[pre] = Bucket(pre, OrderedDict((k, named[k].to(dev, F32)) for k in named), 2)
-        self.S = OrderedDict((k, v.to(dev).clone()) for k, v in buffers.items())
-        self.Ssub = {pre: _split(self.S, pre) for pre in self.buckets}
-        self.nbt = {}
-        self.sc = Z(16)  # [0..3] = L_fake, L_real, L_rec, L_pen (sums)
-        self.lr = {"encoder.": float(self.hp["lr"]), "decoder.": float(self.hp["lr"]),
-                   "discriminator.": 0.5 * float(self.hp["lr"])}
+            nets["discriminator."] = self.dis
+        lr = {"encoder.": float(self.hp["lr"]), "decoder.": float(self.hp["lr"]), "discriminator.": 0.5 * float(self.hp["lr"])}
+        self._setup(params, buffers, nets, dict.fromkeys(nets, 2), lr, dist_group)
         self.t = 0
-        self._ones_buf = None
-        self._mmd_ws = torch.empty(3, dtype=torch.float64, device=dev)
-        self._setup_dist(dist_group)
-        for pre, net in self.nets.items():
-            net.refresh(self.buckets[pre].P, inplace=True)
-
-    def _ones(self, n):
-        if self._ones_buf is None or self._ones_buf.numel() < n:
-            self._ones_buf = torch.ones(n, device="cuda")
-        return self._ones_buf
-
-    def _adam(self, pre):
-        b, hp = self.buckets[pre], self.hp
-        L.multi_tensor_adam_dev([b.flat_p], [b.flat_g], [b.states[0]], [b.states[1]], self.lr[pre], hp["beta1"], hp["beta2"],
-                                hp["eps"], self.t_dev)
-        self.nets[pre].refresh(b.P, inplace=True)
+        self._mmd_ws = torch.empty(3, dtype=torch.float64, device="cuda")
 
     def step(self, x, z_fake):
         """x [B,3,H,W] fp32 NCHW, z_fake [B,z] fp32 (= 0.5 * N(0,1), train_wae_stage1.py:276), device resident."""
-        if self.penalty == "mmd":
-            return self._step_mmd(x, z_fake)
-        B, z = x.shape[0], self.z
-        be, bd, bc = self.buckets["encoder."], self.buckets["decoder."], self.buckets["discriminator."]
-        L.step_increment(self.t_dev)
-        sc, ones = self.sc, self._ones(B)
-        nbe, nbd = {}, {}
-        # ---------------- discriminator phase (:271-288)
-        ycat, ce = self.enc.forward(be.P, self.Ssub["encoder."], x, True, 2, nbe)
-        z_real = ycat[:, :z]
-        p_real, cr = self.dis.forward(bc.P, z_real)
-        p_fake, cf = self.dis.forward(bc.P, z_fake)
-        l = E(2 * B)
-        L.bce_fwd(p_fake, l[:B], B, True, 10.0)
-        L.bce_fwd(p_real, l[B:], B, False, 10.0)
-        L.vecsum(l[:B], B, 1.0, sc[0:1])
-        L.vecsum(l[B:], B, 1.0, sc[1:2])
-        gp = E(2 * B)
-        L.bce_bwd(p_fake, ones, gp[:B], B, True, 10.0)
-        L.bce_bwd(p_real, ones, gp[B:], B, False, 10.0)
-        self.dis.backward(bc.P, cf, gp[:B], bc.G, False, True, False)
-        self.dis.backward(bc.P, cr, gp[B:], bc.G, True, True, False)
-        self._allreduce_async([bc.flat_g])
-        self._wait_comm()
-        self._adam("discriminator.")
-        # ---------------- generator phase (:292-311)
-        x_recon, cd = self.dec.forward(bd.P, self.Ssub["decoder."], z_real, True, 1, nbd)
-        p_real2, cr2 = self.dis.forward(bc.P, z_real)
-        rec = E(B)
-        L.rowsqdiff_fwd(x_recon, x, rec, B, x[0].numel(), 0.5)
-        L.vecsum(rec, B, 1.0, sc[2:3])
-        L.bce_fwd(p_real2, l[:B], B, True, 10.0)
-        L.vecsum(l[:B], B, 1.0, sc[3:4])
-        dxr = torch.empty_like(x_recon)
-        L.rowsqdiff_bwd(x_recon, x, ones, dxr, None, B, x[0].numel(), 0.5)
-        L.bce_bwd(p_real2, ones, gp[:B], B, True, 10.0)
-        dz_pen = self.dis.backward(bc.P, cr2, gp[:B], None, False, False, True)
-        dz_rec = self.dec.backward(bd.P, cd, 1.0, dxr, 0.0, None, bd.G, False, True, True)
-        self._allreduce_async([bd.flat_g])
-        dmu = E(B, z)
-        L.axpby_tanh_bwd(1.0, dz_rec, 1.0, dz_pen, None, dmu)
-        dycat = Z(B, 2 * z, dtype=self.adt)
-        L.cast2d(dmu, z, dycat[:, :z], 2 * z, B, z)
-        be.flat_g.zero_()  # l_var receives no gradient (logvar unused): its slots stay zero and Adam leaves it unchanged
-        self.enc.backward(be.P, ce, dycat, be.G, False, True, False)
-        self._allreduce_async([be.flat_g, sc[:8]])
-        self._wait_comm()
-        self._adam("encoder.")
-        self._adam("decoder.")
-        for pre, d in (("encoder.", nbe), ("decoder.", nbd)):
-            for k, v in d.items():
-                self.nbt[pre + k] = self.nbt.get(pre + k, 0) + v
-        return dict(z_real=z_real, x_recon=x_recon, d_real=p_real, d_fake=p_fake, d_real_g=p_real2)
-
-    def _step_mmd(self, x, z_fake):
-        """WAE-MMD variant (EXTENSION, parity unpinned: the reference has no MMD, SURVEY.md 0-3): no latent discriminator;
-        L_pen = lambda_mmd * B * MMD_IMQ(z_real, z_fake) over this rank's batch (per-rank, like BatchNorm), one encoder
-        forward. Everything else as train_wae_stage1.py:292-311."""
-        B, z = x.shape[0], self.z
+        B, z, gan = x.shape[0], self.z, self.penalty == "gan"
         be, bd = self.buckets["encoder."], self.buckets["decoder."]
         L.step_increment(self.t_dev)
         sc, ones = self.sc, self._ones(B)
         nbe, nbd = {}, {}
-        ycat, ce = self.enc.forward(be.P, self.Ssub["encoder."], x, True, 1, nbe)
+        ycat, ce = self.enc.forward(be.P, self.Ssub["encoder."], x, True, 2 if gan else 1, nbe)
         z_real = ycat[:, :z]
+        if gan:   # ---------------- discriminator phase (:271-288)
+            bc = self.buckets["discriminator."]
+            p_real, p_fake, l, gp = self._latent_d_phase(self.dis, bc, z_real, z_fake, 10.0, sc)
+            self._allreduce_async([bc.flat_g])
+            self._wait_comm()
+            self._adam("discriminator.")
+        # ---------------- generator phase (:292-311)
         x_recon, cd = self.dec.forward(bd.P, self.Ssub["decoder."], z_real, True, 1, nbd)
+        out = dict(z_real=z_real, x_recon=x_recon)
+        if gan:
+            p_real2, cr2 = self.dis.forward(bc.P, z_real)
+            out.update(d_real=p_real, d_fake=p_fake, d_real_g=p_real2)
         rec = E(B)
         L.rowsqdiff_fwd(x_recon, x, rec, B, x[0].numel(), 0.5)
         L.vecsum(rec, B, 1.0, sc[2:3])
-        lam = self.lambda_mmd * B
-        L.mmd_imq_fwd(z_real, z_fake, B, z, self.sigma2, lam, sc[3:4], self._mmd_ws)
+        if gan:
+            L.bce_fwd(p_real2, l[:B], B, True, 10.0)
+            L.vecsum(l[:B], B, 1.0, sc[3:4])
+        else:
+            lam = self.lambda_mmd * B
+            L.mmd_imq_fwd(z_real, z_fake, B, z, self.sigma2, lam, sc[3:4], self._mmd_ws)
         dxr = torch.empty_like(x_recon)
         L.rowsqdiff_bwd(x_recon, x, ones, dxr, None, B, x[0].numel(), 0.5)
+        if gan:
+            L.bce_bwd(p_real2, ones, gp[:B], B, True, 10.0)
+            dz_pen = self.dis.backward(bc.P, cr2, gp[:B], None, False, False, True)
         dz_rec = self.dec.backward(bd.P, cd, 1.0, dxr, 0.0, None, bd.G, False, True, True)
         self._allreduce_async([bd.flat_g])
-        dmu = dz_rec if dz_rec.dtype == F32 and dz_rec.is_contiguous() else dz_rec.to(F32).contiguous()
-        L.mmd_imq_bwd(z_real, z_fake, B, z, self.sigma2, lam, dmu, accumulate=True)
-        dycat = Z(B, 2 * z, dtype=self.adt)
-        L.cast2d(dmu, z, dycat[:, :z], 2 * z, B, z)
-        be.flat_g.zero_()
-        self.enc.backward(be.P, ce, dycat, be.G, False, True, False)
-        self._allreduce_async([be.flat_g, sc[:8]])
-        self._wait_comm()
-        self._adam("encoder.")
+        if gan:
+            dmu = E(B, z)
+            L.axpby_tanh_bwd(1.0, dz_rec, 1.0, dz_pen, None, dmu)
+        else:
+            dmu = dz_rec if dz_rec.dtype == F32 and dz_rec.is_contiguous() else dz_rec.to(F32).contiguous()
+            L.mmd_imq_bwd(z_real, z_fake, B, z, self.sigma2, lam, dmu, accumulate=True)
+        self._encoder_tail(ce, dmu)
         self._adam("decoder.")
-        for pre, d in (("encoder.", nbe), ("decoder.", nbd)):
-            for k, v in d.items():
-                self.nbt[pre + k] = self.nbt.get(pre + k, 0) + v
-        return dict(z_real=z_real, x_recon=x_recon)
-
-    def losses(self):
-        s = self.sc.tolist()
-        return dict(loss_discriminator_fake=s[0], loss_discriminator_real=s[1], loss_reconstruction=s[2],
-                    loss_penalty=s[3])
+        self._count_bn_updates("encoder.", nbe)
+        self._count_bn_updates("decoder.", nbd)
+        return out
 
 
 class VaeGanCognitiveStage(_TrainerBase):
@@ -565,6 +550,7 @@ class VaeGanCognitiveStage(_TrainerBase):
     Parameter keys: encoder.* (CognitiveEncoder), decoder.*, discriminator.*, teacher_net.encoder.* (stage 2 only)."""
 
     LATENT_DISCRIMINATOR = False
+    mode, _klw = "vae-gan", 1.0   # losses() is VaeGanStage1's, with the 'vae-gan' formulas
 
     def __init__(self, params, buffers, cfg, stage, z=128, adt=BF16, hp=None, dist_group=None, voxels=None):
         from .hp import HP_VGAN, NUM_VOXELS
@@ -576,36 +562,16 @@ class VaeGanCognitiveStage(_TrainerBase):
         self.cog = NN.CognitiveEncoderNet(voxels or NUM_VOXELS, z, adt)
         self.dec = NN.DecoderNet(cfg, z, adt)
         self.dis = NN.DiscriminatorNet(cfg, adt)
-        self.nets = OrderedDict((("encoder.", self.cog), ("decoder.", self.dec), ("discriminator.", self.dis)))
+        nets = OrderedDict((("encoder.", self.cog), ("decoder.", self.dec), ("discriminator.", self.dis)))
         if stage == 2 or self.LATENT_DISCRIMINATOR:
             self.tenc = NN.EncoderNet(cfg, z, adt)
-            self.nets["teacher_net.encoder."] = self.tenc
+            nets["teacher_net.encoder."] = self.tenc
         if self.LATENT_DISCRIMINATOR:
             self.ldis = NN.WaeDiscriminatorNet(z, adt)
-            self.nets["latent_discriminator."] = self.ldis
-        dev = torch.device("cuda")
-        self.buckets = OrderedDict()
-        for pre, net in self.nets.items():
-            named = _split(params, pre)
-            diff = set(net.param_names()) ^ set(named)
-            if diff:
-                raise L.FmriError(f"parameter names of {pre} differ from the reference layout: {sorted(diff)}")
-            self.buckets[pre] = Bucket(pre, OrderedDict((k, named[k].to(dev, F32)) for k in named),
-                                       2 if pre == "latent_discriminator." else 1)
-        self.S = OrderedDict((k, v.to(dev).clone()) for k, v in buffers.items())
-        self.Ssub = {pre: _split(self.S, pre) for pre in self.buckets}
-        self.nbt = {}
-        self.sc = Z(16)      # [0..5] as VaeGanStage1; [6], [7] = latent L_fake, L_real; [8], [9] = gates
-        self.lr = {pre: float(self.hp["lr"]) for pre in self.buckets}
-        self._ones_buf = None
-        self._setup_dist(dist_group)
-        for pre, net in self.nets.items():
-            net.refresh(self.buckets[pre].P, inplace=True)
-
-    def _ones(self, n):
-        if self._ones_buf is None or self._ones_buf.numel() < n:
-            self._ones_buf = torch.ones(n, device="cuda")
-        return self._ones_buf
+            nets["latent_discriminator."] = self.ldis
+        # sc: [0..5] as VaeGanStage1; [8], [9] = gates
+        self._setup(params, buffers, nets, {pre: 2 if pre == "latent_discriminator." else 1 for pre in nets},
+                    dict.fromkeys(nets, float(self.hp["lr"])), dist_group)
 
     def forward_backward(self, fmri, image, eps, eps_t, z_p):
         """fmri [B,V], image [B,3,H,W], eps / eps_t / z_p [B,z]: fp32, device resident (eps_t is used in stage 2 only)."""
@@ -630,8 +596,7 @@ class VaeGanCognitiveStage(_TrainerBase):
         raw3, p, cc = self.dis.forward(bc.P, self.Ssub["discriminator."], [gt_x, x_tilde, x_p], True, 2, True,
                                        nb["discriminator."])
         for pre, d in nb.items():
-            for k, v in d.items():
-                self.nbt[pre + k] = self.nbt.get(pre + k, 0) + v
+            self._count_bn_updates(pre, d)
         Fd = raw3[0].numel()
         mse, nle, bce = E(B), E(B), E(3 * B)
         L.rowsqdiff_fwd(raw3[:B], raw3[B:2 * B], mse, B, Fd, 0.5)
@@ -711,24 +676,12 @@ class DualCognitiveStage3(VaeGanCognitiveStage):
 
     def forward_backward(self, fmri, image, eps, z_p):
         out = super().forward_backward(fmri, image, eps, None, z_p)
-        B, z, sc = fmri.shape[0], self.z, self.sc
         bt, bl = self.buckets["teacher_net.encoder."], self.buckets["latent_discriminator."]
         nbt = {}
         yt, _ = self.tenc.forward(bt.P, self.Ssub["teacher_net.encoder."], image, True, 1, nbt)
-        for k, v in nbt.items():
-            self.nbt["teacher_net.encoder." + k] = self.nbt.get("teacher_net.encoder." + k, 0) + v
-        z_fake, z_real = out["mu"], yt[:, :z]
-        p_real, cr = self.ldis.forward(bl.P, z_real)
-        p_fake, cf = self.ldis.forward(bl.P, z_fake)
-        l, gp, ones = E(2 * B), E(2 * B), self._ones(3 * B)
-        L.bce_fwd(p_fake, l[:B], B, True, 10.0)
-        L.bce_fwd(p_real, l[B:], B, False, 10.0)
-        L.vecsum(l[:B], B, 1.0, self.lsc[0:1])
-        L.vecsum(l[B:], B, 1.0, self.lsc[1:2])
-        L.bce_bwd(p_fake, ones, gp[:B], B, True, 10.0)
-        L.bce_bwd(p_real, ones, gp[B:], B, False, 10.0)
-        self.ldis.backward(bl.P, cf, gp[:B], bl.G, False, True, False)
-        self.ldis.backward(bl.P, cr, gp[B:], bl.G, True, True, False)
+        self._count_bn_updates("teacher_net.encoder.", nbt)
+        z_fake, z_real = out["mu"], yt[:, :self.z]
+        p_real, p_fake, _, _ = self._latent_d_phase(self.ldis, bl, z_real, z_fake, 10.0, self.lsc)
         self._allreduce_async([bl.flat_g, self.lsc])
         out.update(z_real=z_real, d_real=p_real, d_fake=p_fake)
         return out
@@ -747,13 +700,13 @@ class DualCognitiveStage3(VaeGanCognitiveStage):
         return out
 
     def losses(self):
-        d = VaeGanStage1.losses(self)
+        d = super().losses()
         lf, lr = self.lsc.tolist()
         d.update(loss_discriminator_fake=lf, loss_discriminator_real=lr)
         return d
 
 
-class WaeCognitiveStage(_TrainerBase):
+class WaeCognitiveStage(_WaeTrainer):
     """Stage-II / Stage-III cognitive WAE/GAN trainer (/root/reference/train/train_wae_stage2.py:274-328,
     train_wae_stage3.py:295-347) over WaeGanCognitive (models/vae_gan.py:532-578) and the Stage-I teacher's visual encoder.
 
@@ -780,30 +733,12 @@ class WaeCognitiveStage(_TrainerBase):
         self.dec = NN.DecoderNet(cfg, z, adt)
         self.dis = NN.WaeDiscriminatorNet(z, adt)
         self.tenc = NN.EncoderNet(cfg, z, adt)
-        self.nets = OrderedDict((("encoder.", self.cog), ("decoder.", self.dec), ("discriminator.", self.dis),
-                                 ("teacher_net.encoder.", self.tenc)))
-        dev = torch.device("cuda")
-        self.buckets = OrderedDict()
-        for pre, net in self.nets.items():
-            named = _split(params, pre)
-            diff = set(net.param_names()) ^ set(named)
-            if diff:
-                raise L.FmriError(f"parameter names of {pre} differ from the reference layout: {sorted(diff)}")
-            self.buckets[pre] = Bucket(pre, OrderedDict((k, named[k].to(dev, F32)) for k in named), 2)
-        self.S = OrderedDict((k, v.to(dev).clone()) for k, v in buffers.items())
-        self.Ssub = {pre: _split(self.S, pre) for pre in self.buckets}
-        self.nbt = {}
-        self.sc = Z(16)  # [0..3] = L_fake, L_real (sums), L_rec, L_pen (global means)
-        self.lr = {"encoder.": float(self.hp["lr"]), "decoder.": float(self.hp["lr"]),
-                   "discriminator.": float(self.hp["lr_dis"])}
+        nets = OrderedDict((("encoder.", self.cog), ("decoder.", self.dec), ("discriminator.", self.dis),
+                            ("teacher_net.encoder.", self.tenc)))
+        # sc: [0..3] = L_fake, L_real (sums), L_rec, L_pen (global means)
+        lr = {"encoder.": float(self.hp["lr"]), "decoder.": float(self.hp["lr"]), "discriminator.": float(self.hp["lr_dis"])}
+        self._setup(params, buffers, nets, dict.fromkeys(nets, 2), lr, dist_group)
         self.t = 0
-        self._ones_buf = None
-        self._setup_dist(dist_group)
-        for pre, net in self.nets.items():
-            net.refresh(self.buckets[pre].P, inplace=True)
-
-    _ones = WaeGanStage1._ones
-    _adam = WaeGanStage1._adam
 
     def step(self, fmri, image):
         """fmri [B,V], image [B,3,H,W]: fp32, device resident."""
@@ -824,17 +759,7 @@ class WaeCognitiveStage(_TrainerBase):
         ycat, ce = self.cog.forward(be.P, self.Ssub["encoder."], fmri, True, 2, nb["encoder."])
         z_fake = ycat[:, :z]
         # ---------------- discriminator phase
-        p_real, cr = self.dis.forward(bc.P, z_real)
-        p_fake, cf = self.dis.forward(bc.P, z_fake)
-        l, gp = E(2 * B), E(2 * B)
-        L.bce_fwd(p_fake, l[:B], B, True, 10.0)
-        L.bce_fwd(p_real, l[B:], B, False, 10.0)
-        L.vecsum(l[:B], B, 1.0, sc[0:1])
-        L.vecsum(l[B:], B, 1.0, sc[1:2])
-        L.bce_bwd(p_fake, ones, gp[:B], B, True, 10.0)
-        L.bce_bwd(p_real, ones, gp[B:], B, False, 10.0)
-        self.dis.backward(bc.P, cf, gp[:B], bc.G, False, True, False)
-        self.dis.backward(bc.P, cr, gp[B:], bc.G, True, True, False)
+        p_real, p_fake, l, gp = self._latent_d_phase(self.dis, bc, z_real, z_fake, 10.0, sc)
         self._allreduce_async([bc.flat_g])
         self._wait_comm()
         self._adam("discriminator.")
@@ -855,27 +780,15 @@ class WaeCognitiveStage(_TrainerBase):
             dz_rec = self.dec.backward(bd.P, cd, 1.0, dxr, 0.0, None, None, False, False, True)
             dmu = E(B, z)
             L.axpby_tanh_bwd(1.0, dz_rec, 1.0, dz_pen, None, dmu)
-            dycat = Z(B, 2 * z, dtype=self.adt)
-            L.cast2d(dmu, z, dycat[:, :z], 2 * z, B, z)
-            be.flat_g.zero_()  # l_var receives no gradient (logvar unused): zero slots, Adam leaves it unchanged
-            self.cog.backward(be.P, ce, dycat, be.G, False, True, False)
-            self._allreduce_async([be.flat_g, sc[:8]])
-            self._wait_comm()
-            self._adam("encoder.")
+            self._encoder_tail(ce, dmu)
         else:
             self.dec.backward(bd.P, cd, 1.0, dxr, 0.0, None, bd.G, False, True, False)
             self._allreduce_async([bd.flat_g, sc[:8]])
             self._wait_comm()
             self._adam("decoder.")
         for pre, d in nb.items():
-            for k, v in d.items():
-                self.nbt[pre + k] = self.nbt.get(pre + k, 0) + v
+            self._count_bn_updates(pre, d)
         return dict(z_fake=z_fake, z_real=z_real, x_recon=x_recon, d_real=p_real, d_fake=p_fake, d_real_g=p2)
-
-    def losses(self):
-        s = self.sc.tolist()
-        return dict(loss_discriminator_fake=s[0], loss_discriminator_real=s[1], loss_reconstruction=s[2],
-                    loss_penalty=s[3])
 
 
 class GraphedStep:
@@ -947,44 +860,21 @@ class DualWaeVaeGanStage1(VaeGanStage1):
     Extra parameter keys: latent_discriminator.main.*; step(x, eps, z_p, z_fake)."""
 
     _enc_bn_updates = 3
+    LATENT_DISCRIMINATOR = True
 
     def __init__(self, params, buffers, cfg, z=128, adt=BF16, hp=None, dist_group=None, gate=True, lam=1.0):
         super().__init__(params, buffers, cfg, z, adt, hp, dist_group, gate)
         self.lam = float(lam)
-        self.ldis = NN.WaeDiscriminatorNet(z, adt)
-        pre = "latent_discriminator."
-        named = _split(params, pre)
-        diff = set(self.ldis.param_names()) ^ set(named)
-        if diff:
-            raise L.FmriError(f"parameter names of {pre} differ from the reference layout: {sorted(diff)}")
-        self.buckets[pre] = Bucket(pre, OrderedDict((k, named[k].to("cuda", F32)) for k in named), 1)
-        self.lr[pre] = float(self.hp["lr"])
-        self.ldis.refresh(self.buckets[pre].P, inplace=True)
         self.lsc = Z(4)   # L_fake, L_real, L_pen (batch sums)
         self._z_fake = None
-
-    def refresh(self):
-        super().refresh()
-        if hasattr(self, "ldis"):
-            self.ldis.refresh(self.buckets["latent_discriminator."].P, inplace=True)
 
     def _before_encoder_backward(self, mu, dycat):
         hp, z, lam = self.hp, self.z, self.lam
         B = mu.shape[0]
         bl, bd = self.buckets["latent_discriminator."], self.buckets["decoder."]
-        z_fake, ones = self._z_fake, self._ones(3 * B)
+        ones = self._ones(B)
         # ---- latent discriminator phase (:380-397)
-        p_real, cr = self.ldis.forward(bl.P, mu)
-        p_fake, cf = self.ldis.forward(bl.P, z_fake)
-        l, gp = E(2 * B), E(2 * B)
-        L.bce_fwd(p_fake, l[:B], B, True, lam)
-        L.bce_fwd(p_real, l[B:], B, False, lam)
-        L.vecsum(l[:B], B, 1.0, self.lsc[0:1])
-        L.vecsum(l[B:], B, 1.0, self.lsc[1:2])
-        L.bce_bwd(p_fake, ones, gp[:B], B, True, lam)
-        L.bce_bwd(p_real, ones, gp[B:], B, False, lam)
-        self.ldis.backward(bl.P, cf, gp[:B], bl.G, False, True, False)
-        self.ldis.backward(bl.P, cr, gp[B:], bl.G, True, True, False)
+        p_real, p_fake, l, gp = self._latent_d_phase(self.ldis, bl, mu, self._z_fake, lam, self.lsc)
         if self.world > 1:   # the penalty needs the globally updated latent discriminator
             self._allreduce_async([bl.flat_g])
             torch.cuda.current_stream().wait_stream(self.comm_stream)
@@ -994,8 +884,7 @@ class DualWaeVaeGanStage1(VaeGanStage1):
         # ---- penalty (:401-417): the unused reconstruction forward (BatchNorm running statistics), then d with the new weights
         nbd = {}
         self.dec.forward(bd.P, self.Ssub["decoder."], mu, True, 1, nbd)
-        for k, v in nbd.items():
-            self.nbt["decoder." + k] = self.nbt.get("decoder." + k, 0) + v
+        self._count_bn_updates("decoder.", nbd)
         p2, c2 = self.ldis.forward(bl.P, mu)
         L.bce_fwd(p2, l[:B], B, True, lam)
         L.vecsum(l[:B], B, 1.0, self.lsc[2:3])
