@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FMRI_ABI_VERSION 6
+#define FMRI_ABI_VERSION 7
 
 typedef enum { FMRI_OK = 0, FMRI_ERR_ARG = -1, FMRI_ERR_UNSUPPORTED = -2, FMRI_ERR_CUDA = -3, FMRI_ERR_WORKSPACE = -4 } fmri_status;
 typedef enum { FMRI_F32 = 0, FMRI_BF16 = 1 } fmri_dtype;
@@ -281,6 +281,28 @@ int fmri_pearson(const float* a, const float* b, long long n, float* out, double
 int fmri_ssim(const float* a, const float* b, int N, int C, int H, int W, float* out, double* ws, void* stream);
 int fmri_image_pipeline(const unsigned char* src, int N, int H, int W, int Csrc, const int* flip, const int* shift_yx,
                         const float* mean3, const float* std3, float* dst, void* stream);
+/* fmri_image_rescale: the BOLD5000 stimulus transform Rescale -> RandomShift -> SampleToTensor -> Normalization
+ *   (data_preprocessing/data_loader.py Rescale, :187-217 RandomShift, :93-111 Normalization; train/train_vgan_stage2.py:160-168)
+ *   on native-resolution sources: N uint8 HWC images of any size and 1 or 3 channels, each described by one fmri_image_src
+ *   (byte offset into `src`, which holds src_bytes bytes), -> normalised fp32 NCHW dst [N, 3, H, W]. Rescale is
+ *   skimage.transform.resize(img, (H, W)) with its defaults (skimage >= 0.19: order 1, mode 'reflect', anti-aliasing when
+ *   some axis downsamples, output in [0, 1]); per axis with f = in / out: a Gaussian pre-filter sigma = max(0, (f - 1) / 2),
+ *   radius int(4 sigma + 0.5), mirror boundary, then linear interpolation at u = (o + 0.5) f - 0.5. Flip, shift, GreyToColor
+ *   and normalisation are those of fmri_image_pipeline, applied to the resized image; with Hs = H and Ws = W the result is
+ *   bit-identical to fmri_image_pipeline. fp32 weights and sums, no atomics: two calls give the same bits.
+ *   `images` is a HOST array; every entry is checked before anything is launched (sizes >= 1 and <= 32768, C in {1, 3},
+ *   the image inside src_bytes; FMRI_ERR_UNSUPPORTED when an image's source band does not fit the shared memory of one
+ *   CTA), then the table is copied into ws (fmri_image_rescale_workspace(N) bytes, 8-byte aligned) on `stream`. ws must
+ *   stay untouched until the kernel has run; nothing is read back from the device. Not capturable in a CUDA graph (the
+ *   table is copied from host memory at call time). */
+typedef struct {
+    long long offset; /* byte offset of the image's first pixel in src */
+    int H, W, C;      /* source height, width, channels (1 or 3); the image is dense HWC */
+} fmri_image_src;
+size_t fmri_image_rescale_workspace(int N); /* bytes; 0 for N < 1 */
+int fmri_image_rescale(const unsigned char* src, size_t src_bytes, const fmri_image_src* images, int N, int H, int W,
+                       const int* flip, const int* shift_yx, const float* mean3, const float* std3, float* dst, void* ws,
+                       size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * All-pairs similarity and n-way identification: the exhaustive, exact-expectation form of the reference's sampled

@@ -15,6 +15,7 @@
 #include "mmd_kernels.cuh"
 #include "eval_kernels.cuh"
 #include "similarity_kernels.cuh"
+#include "rescale_kernels.cuh"
 
 using namespace fmri;
 
@@ -2221,6 +2222,57 @@ extern "C" int fmri_image_pipeline(const unsigned char* src, int N, int H, int W
     const float sd[3] = {std3 ? std3[0] : 1.f, std3 ? std3[1] : 1.f, std3 ? std3[2] : 1.f};
     image_pipeline_kernel<<<grid1d((long long)N * 3 * H * W, 256, 148 * 8), 256, 0, S(stream)>>>(
         src, N, H, W, Csrc, flip, shift_yx, m[0], m[1], m[2], sd[0], sd[1], sd[2], dst);
+    LAUNCH_OK();
+    return 0;
+}
+extern "C" size_t fmri_image_rescale_workspace(int N) { return N < 1 ? 0 : sizeof(fmri_image_src) * (size_t)N; }
+extern "C" int fmri_image_rescale(const unsigned char* src, size_t src_bytes, const fmri_image_src* images, int N, int H,
+                                  int W, const int* flip, const int* shift_yx, const float* mean3, const float* std3,
+                                  float* dst, void* ws, size_t ws_bytes, void* stream) {
+    const int kMaxSide = 32768;   // keeps the kernel's integer tap positions, (2o + 1) * in, below 2^31
+    if (!src || !images || !dst || N < 1 || H < 1 || W < 1 || H > kMaxSide || W > kMaxSide)
+        return fail(FMRI_ERR_ARG, "image_rescale arguments (N = %d, H = %d, W = %d)", N, H, W);
+    const size_t need = fmri_image_rescale_workspace(N);
+    if (!ws || ws_bytes < need) return fail(FMRI_ERR_WORKSPACE, "image_rescale workspace %zu < %zu", ws_bytes, need);
+    if (reinterpret_cast<uintptr_t>(ws) % 8) return fail(FMRI_ERR_ARG, "image_rescale workspace not 8-byte aligned");
+    for (int i = 0; i < N; ++i) {
+        const fmri_image_src& d = images[i];
+        if (d.H < 1 || d.W < 1 || d.H > kMaxSide || d.W > kMaxSide || (d.C != 1 && d.C != 3))
+            return fail(FMRI_ERR_ARG, "image_rescale: image %d is %d x %d x %d (sides 1..%d, 1 or 3 channels)", i, d.H, d.W,
+                        d.C, kMaxSide);
+        const unsigned long long bytes = (unsigned long long)d.H * d.W * d.C;
+        if (d.offset < 0 || (unsigned long long)d.offset > src_bytes || bytes > src_bytes - (unsigned long long)d.offset)
+            return fail(FMRI_ERR_ARG, "image_rescale: image %d (offset %lld, %llu bytes) outside the %zu-byte source", i,
+                        d.offset, bytes, src_bytes);
+    }
+    int dev = 0, optin = 0;
+    CUDA_OK(cudaGetDevice(&dev));
+    CUDA_OK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    // rows per CTA: the most (up to 4) whose largest source band still fits one CTA's shared memory
+    int ty = 4;
+    long long smem = 0;
+    for (; ty >= 1; ty /= 2) {
+        smem = 0;
+        for (int i = 0; i < N; ++i)
+            smem = std::max(smem, rs_smem_bytes(images[i].H, images[i].W, images[i].C, H, W, ty));
+        if (smem <= optin) break;
+    }
+    if (ty < 1) {
+        for (int i = 0; i < N; ++i)
+            if (rs_smem_bytes(images[i].H, images[i].W, images[i].C, H, W, 1) > optin)
+                return fail(FMRI_ERR_UNSUPPORTED, "image_rescale: the source band of image %d (%d x %d x %d -> %d x %d) needs "
+                            "%lld B of shared memory, more than the %d B of one CTA", i, images[i].H, images[i].W,
+                            images[i].C, H, W, rs_smem_bytes(images[i].H, images[i].W, images[i].C, H, W, 1), optin);
+    }
+    const int tiles = cdiv(H, ty);
+    if ((long long)N * tiles > 0x7fffffffLL) return fail(FMRI_ERR_UNSUPPORTED, "image_rescale: %d images x %d row tiles", N, tiles);
+    const float m[3] = {mean3 ? mean3[0] : 0.f, mean3 ? mean3[1] : 0.f, mean3 ? mean3[2] : 0.f};
+    const float sd[3] = {std3 ? std3[0] : 1.f, std3 ? std3[1] : 1.f, std3 ? std3[2] : 1.f};
+    CUDA_OK(cudaFuncSetAttribute(image_rescale_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_OK(cudaMemcpyAsync(ws, images, need, cudaMemcpyHostToDevice, S(stream)));
+    image_rescale_kernel<<<N * tiles, RS_THREADS, smem, S(stream)>>>(src, reinterpret_cast<const fmri_image_src*>(ws), H, W,
+                                                                       ty, tiles, flip, shift_yx, m[0], m[1], m[2], sd[0],
+                                                                       sd[1], sd[2], dst);
     LAUNCH_OK();
     return 0;
 }

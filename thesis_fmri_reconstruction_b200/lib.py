@@ -41,6 +41,11 @@ class LinearDesc(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("M", "N", "K", "dtype")]
 
 
+class ImageSrc(C.Structure):
+    """fmri_image_src: one uint8 HWC source image at a byte offset of a shared buffer."""
+    _fields_ = [("offset", C.c_longlong), ("H", C.c_int), ("W", C.c_int), ("C", C.c_int)]
+
+
 def header_functions():
     """Names of every function the public header declares (used by the CPU-side export test)."""
     src = open(HEADER_PATH).read()
@@ -64,7 +69,7 @@ class _Proxy:
         f = getattr(self._c, name)
         if PROF is None or name in ("fmri_last_error", "fmri_conv_out_hw", "fmri_conv_wgrad_workspace",
                                     "fmri_edge_workspace", "fmri_launch_count", "fmri_version", "fmri_conv_pack_elems",
-                                    "fmri_pairwise_workspace"):
+                                    "fmri_pairwise_workspace", "fmri_image_rescale_workspace"):
             return f
 
         def timed(*a):
@@ -130,6 +135,7 @@ def load():
         c.fmri_conv_pack_elems.restype = C.c_size_t
         c.fmri_edge_workspace.restype = C.c_size_t
         c.fmri_pairwise_workspace.restype = C.c_size_t
+        c.fmri_image_rescale_workspace.restype = C.c_size_t
         c.fmri_conv_out_hw.restype = None
         c.fmri_launch_count.restype = C.c_longlong
         _lib = _Proxy(c)
@@ -545,6 +551,31 @@ def image_pipeline(src_u8, flip, shift_yx, mean3, std3, dst):
     m = (C.c_float * 3)(*[float(v) for v in mean3])
     s = (C.c_float * 3)(*[float(v) for v in std3])
     _check(load().fmri_image_pipeline(ptr(src_u8), N, H, W, Cs, ptr(flip), ptr(shift_yx), m, s, ptr(dst), stream()))
+
+
+def image_src_table(entries):
+    """Host descriptor table (ctypes array of ImageSrc) from (byte offset, H, W, C) tuples."""
+    return (ImageSrc * len(entries))(*[ImageSrc(int(o), int(h), int(w), int(c)) for o, h, w, c in entries])
+
+
+def image_rescale_workspace(N):
+    """Bytes of device workspace fmri_image_rescale needs for N images (0 for N < 1)."""
+    return int(load().fmri_image_rescale_workspace(int(N)))
+
+
+def image_rescale(src_u8, table, flip, shift_yx, mean3, std3, dst, ws):
+    """src_u8: flat uint8 device buffer holding every source image; table: image_src_table(...) on the host (one entry per
+    output image); dst: fp32 [N, 3, H, W]; ws: a device buffer of at least image_rescale_workspace(N) bytes."""
+    _require_cuda(src_u8, flip, shift_yx, dst, ws)
+    if src_u8.dtype != torch.uint8 or dst.dtype != torch.float32 or dst.dim() != 4 or dst.shape[1] != 3:
+        raise FmriError("image_rescale expects a uint8 source buffer and a float32 [N, 3, H, W] output")
+    N, _, H, W = dst.shape
+    if len(table) != N:
+        raise FmriError(f"image_rescale: {len(table)} descriptors for {N} output images")
+    m = (C.c_float * 3)(*[float(v) for v in mean3])
+    s = (C.c_float * 3)(*[float(v) for v in std3])
+    _check(load().fmri_image_rescale(ptr(src_u8), C.c_size_t(src_u8.numel()), table, N, H, W, ptr(flip), ptr(shift_yx), m,
+                                     s, ptr(dst), ptr(ws), _wsb(ws) if ws is not None else C.c_size_t(0), stream()))
 
 
 # ------------------------------------------------------------------------------------------------ all-pairs similarity
