@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define FMRI_ABI_VERSION 7
+#define FMRI_ABI_VERSION 8
 
 typedef enum { FMRI_OK = 0, FMRI_ERR_ARG = -1, FMRI_ERR_UNSUPPORTED = -2, FMRI_ERR_CUDA = -3, FMRI_ERR_WORKSPACE = -4 } fmri_status;
 typedef enum { FMRI_F32 = 0, FMRI_BF16 = 1 } fmri_dtype;
@@ -303,6 +303,44 @@ size_t fmri_image_rescale_workspace(int N); /* bytes; 0 for N < 1 */
 int fmri_image_rescale(const unsigned char* src, size_t src_bytes, const fmri_image_src* images, int N, int H, int W,
                        const int* flip, const int* shift_yx, const float* mean3, const float* std3, float* dst, void* ws,
                        size_t ws_bytes, void* stream);
+/* fmri_image_resample: the COCO Stage-I loader's PIL / torchvision resize (Resize, CenterCrop, RandomResizedCrop on PIL
+ *   images: PIL.Image.resize with BILINEAR or BICUBIC; train/train_vgan_stage1.py:161-171, data_preprocessing/data_loader.py
+ *   :346 CocoDataloader) -> RandomHorizontalFlip / shift -> ToTensor -> GreyToColor -> Normalize, on native-resolution
+ *   uint8 sources. Image n is the window described by images[n]: H x W pixels of C (1 or 3) interleaved channels at byte
+ *   offset `offset` of `src` (src_bytes bytes), rows `pitch` bytes apart, so a crop of a larger image is a strided window
+ *   and, as with PIL's crop-then-resize, the filter taps are clamped at the window's edges. The window is resized to
+ *   Hr x Wr exactly as Pillow's 8-bit Image.resize does (fp64 filter weights, 22-bit fixed-point taps, a horizontal
+ *   then a vertical pass, each rounded and clamped to uint8), and the H x W (the call's H, W) part of it at (oy, ox) is
+ *   kept, which is Resize followed by CenterCrop without computing the discarded pixels. Flip, shift, GreyToColor and
+ *   normalisation are those of fmri_image_pipeline: dst [N, 3, H, W] is bit-identical to fmri_image_pipeline applied to
+ *   Pillow's uint8 result, and with Hr = H = window height, Wr = W = window width to fmri_image_pipeline on the source.
+ *   Integer sums, no atomics: two calls give the same bits. `filter` is FMRI_RESAMPLE_BILINEAR or FMRI_RESAMPLE_BICUBIC
+ *   (Pillow's Image.Resampling values). The taps are computed on the device, per CTA.
+ *   `images` is a HOST array; every entry is checked before anything is launched: sides >= 1 and <= 32768, C in {1, 3},
+ *   pitch >= W * C, the window inside src_bytes, oy + H <= Hr and ox + W <= Wr. An image whose one-row band needs more
+ *   than FMRI_RESAMPLE_MAX_SMEM bytes of shared memory is refused with FMRI_ERR_UNSUPPORTED, also before any launch. Per
+ *   axis, with `in` the window side and `out` the resized side, Pillow's support is sup = s max(in / out, 1) (s = 1
+ *   bilinear, 2 bicubic) and its tap count k = 2 ceil(sup) + 1. A band of `ty` output rows needs, each term rounded up to
+ *   16 bytes: 4 W k_x + 8 W (horizontal taps) + 4 ty k_y + 8 ty (vertical taps) + rows W C (the uint8 horizontal-pass
+ *   rows it reads), rows = min(window H, (int)((ty - 1) in_y / out_y + 2 sup_y) + 2); for a window more than 100 times
+ *   taller than wide that shrinks vertically, which Image.resize (and this call) resamples vertically first, the last
+ *   term is ty Wwin C instead. E.g. 480 x 640 -> 64 x 64 BICUBIC takes 17296 B at ty = 1; a window 4096 wide resized
+ *   to 64 columns BICUBIC (k_x = 257) about 65 KB; 32768 -> 64 columns does not fit. The table is then copied into ws
+ *   (fmri_image_resample_workspace(N) bytes, 8-byte aligned) on `stream`. ws must stay untouched until the kernel has
+ *   run; nothing is read back from the device. Not capturable in a CUDA graph. */
+#define FMRI_RESAMPLE_MAX_SMEM 232448 /* 227 KB: the opt-in shared memory of one CTA on sm_100 */
+typedef enum { FMRI_RESAMPLE_BILINEAR = 2, FMRI_RESAMPLE_BICUBIC = 3 } fmri_resample_filter;
+typedef struct {
+    long long offset; /* byte offset of the window's top-left pixel in src */
+    long long pitch;  /* bytes from one window row to the next (>= W * C) */
+    int H, W, C;      /* window height, width, channels (1 or 3) */
+    int Hr, Wr;       /* size of the whole resized image */
+    int oy, ox;       /* top-left corner of the call's H x W output inside the Hr x Wr resized image */
+} fmri_image_window;
+size_t fmri_image_resample_workspace(int N); /* bytes; 0 for N < 1 */
+int fmri_image_resample(const unsigned char* src, size_t src_bytes, const fmri_image_window* images, int N, int H, int W,
+                        int filter, const int* flip, const int* shift_yx, const float* mean3, const float* std3, float* dst,
+                        void* ws, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * All-pairs similarity and n-way identification: the exhaustive, exact-expectation form of the reference's sampled

@@ -16,6 +16,7 @@
 #include "eval_kernels.cuh"
 #include "similarity_kernels.cuh"
 #include "rescale_kernels.cuh"
+#include "resample_kernels.cuh"
 
 using namespace fmri;
 
@@ -2273,6 +2274,69 @@ extern "C" int fmri_image_rescale(const unsigned char* src, size_t src_bytes, co
     image_rescale_kernel<<<N * tiles, RS_THREADS, smem, S(stream)>>>(src, reinterpret_cast<const fmri_image_src*>(ws), H, W,
                                                                        ty, tiles, flip, shift_yx, m[0], m[1], m[2], sd[0],
                                                                        sd[1], sd[2], dst);
+    LAUNCH_OK();
+    return 0;
+}
+// The COCO Stage-I loader's PIL resize (torchvision Resize / CenterCrop / RandomResizedCrop on PIL images, then the
+// transforms of train/train_vgan_stage1.py:161-171; data_preprocessing/data_loader.py:346 CocoDataloader).
+extern "C" size_t fmri_image_resample_workspace(int N) { return N < 1 ? 0 : sizeof(fmri_image_window) * (size_t)N; }
+extern "C" int fmri_image_resample(const unsigned char* src, size_t src_bytes, const fmri_image_window* images, int N,
+                                   int H, int W, int filter, const int* flip, const int* shift_yx, const float* mean3,
+                                   const float* std3, float* dst, void* ws, size_t ws_bytes, void* stream) {
+    const int kMaxSide = 32768;
+    if (!src || !images || !dst || N < 1 || H < 1 || W < 1 || H > kMaxSide || W > kMaxSide ||
+        (filter != FMRI_RESAMPLE_BILINEAR && filter != FMRI_RESAMPLE_BICUBIC))
+        return fail(FMRI_ERR_ARG, "image_resample arguments (N = %d, H = %d, W = %d, filter = %d)", N, H, W, filter);
+    const size_t need = fmri_image_resample_workspace(N);
+    if (!ws || ws_bytes < need) return fail(FMRI_ERR_WORKSPACE, "image_resample workspace %zu < %zu", ws_bytes, need);
+    if (reinterpret_cast<uintptr_t>(ws) % 8) return fail(FMRI_ERR_ARG, "image_resample workspace not 8-byte aligned");
+    for (int i = 0; i < N; ++i) {
+        const fmri_image_window& d = images[i];
+        if (d.H < 1 || d.W < 1 || d.Hr < 1 || d.Wr < 1 || d.H > kMaxSide || d.W > kMaxSide || d.Hr > kMaxSide ||
+            d.Wr > kMaxSide || (d.C != 1 && d.C != 3))
+            return fail(FMRI_ERR_ARG, "image_resample: image %d is %d x %d x %d -> %d x %d (sides 1..%d, 1 or 3 channels)", i,
+                        d.H, d.W, d.C, d.Hr, d.Wr, kMaxSide);
+        if (d.oy < 0 || d.ox < 0 || d.oy > d.Hr - H || d.ox > d.Wr - W)
+            return fail(FMRI_ERR_ARG, "image_resample: image %d's %d x %d output at (%d, %d) leaves its %d x %d resize", i, H,
+                        W, d.oy, d.ox, d.Hr, d.Wr);
+        const long long row = (long long)d.W * d.C;
+        if (d.pitch < row)
+            return fail(FMRI_ERR_ARG, "image_resample: image %d's pitch %lld < %lld bytes per row", i, d.pitch, row);
+        // the window spans (H - 1) pitch + W C bytes from its offset (compared without forming the product)
+        const unsigned long long avail = d.offset < 0 || (unsigned long long)d.offset > src_bytes
+                                             ? 0 : src_bytes - (unsigned long long)d.offset;
+        if (d.offset < 0 || (unsigned long long)row > avail ||
+            (d.H > 1 && (unsigned long long)d.pitch > (avail - row) / (unsigned long long)(d.H - 1)))
+            return fail(FMRI_ERR_ARG, "image_resample: image %d (offset %lld, %d rows of pitch %lld) outside the %zu-byte "
+                        "source", i, d.offset, d.H, d.pitch, src_bytes);
+    }
+    // rows per CTA: the most (up to 8) whose largest band fits one CTA's shared memory
+    int ty = 8;
+    long long smem = 0;
+    for (; ty >= 1; ty /= 2) {
+        smem = 0;
+        for (int i = 0; i < N; ++i) smem = std::max(smem, rp_smem_bytes(images[i], H, W, filter, ty));
+        if (smem <= FMRI_RESAMPLE_MAX_SMEM) break;
+    }
+    if (ty < 1) {
+        for (int i = 0; i < N; ++i) {
+            const long long b = rp_smem_bytes(images[i], H, W, filter, 1);
+            if (b > FMRI_RESAMPLE_MAX_SMEM)
+                return fail(FMRI_ERR_UNSUPPORTED, "image_resample: the one-row band of image %d (%d x %d x %d -> %d x %d, "
+                            "output %d x %d) needs %lld B of shared memory, more than FMRI_RESAMPLE_MAX_SMEM = %d B", i,
+                            images[i].H, images[i].W, images[i].C, images[i].Hr, images[i].Wr, H, W, b,
+                            FMRI_RESAMPLE_MAX_SMEM);
+        }
+    }
+    const int tiles = cdiv(H, ty);
+    if ((long long)N * tiles > 0x7fffffffLL) return fail(FMRI_ERR_UNSUPPORTED, "image_resample: %d images x %d row tiles", N, tiles);
+    const float m[3] = {mean3 ? mean3[0] : 0.f, mean3 ? mean3[1] : 0.f, mean3 ? mean3[2] : 0.f};
+    const float sd[3] = {std3 ? std3[0] : 1.f, std3 ? std3[1] : 1.f, std3 ? std3[2] : 1.f};
+    CUDA_OK(cudaFuncSetAttribute(image_resample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_OK(cudaMemcpyAsync(ws, images, need, cudaMemcpyHostToDevice, S(stream)));
+    image_resample_kernel<<<N * tiles, RP_THREADS, smem, S(stream)>>>(src, reinterpret_cast<const fmri_image_window*>(ws), H,
+                                                                        W, filter, ty, tiles, flip, shift_yx, m[0], m[1],
+                                                                        m[2], sd[0], sd[1], sd[2], dst);
     LAUNCH_OK();
     return 0;
 }

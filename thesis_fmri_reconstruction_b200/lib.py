@@ -46,6 +46,13 @@ class ImageSrc(C.Structure):
     _fields_ = [("offset", C.c_longlong), ("H", C.c_int), ("W", C.c_int), ("C", C.c_int)]
 
 
+class ImageWindow(C.Structure):
+    """fmri_image_window: a uint8 HWC window (offset of its top-left pixel, row pitch in bytes, H, W, C) of a shared
+    buffer, its resized size (Hr, Wr) and the top-left corner (oy, ox) of the output inside that resize."""
+    _fields_ = [("offset", C.c_longlong), ("pitch", C.c_longlong)] + [(n, C.c_int) for n in
+                                                                         ("H", "W", "C", "Hr", "Wr", "oy", "ox")]
+
+
 def header_functions():
     """Names of every function the public header declares (used by the CPU-side export test)."""
     src = open(HEADER_PATH).read()
@@ -69,7 +76,8 @@ class _Proxy:
         f = getattr(self._c, name)
         if PROF is None or name in ("fmri_last_error", "fmri_conv_out_hw", "fmri_conv_wgrad_workspace",
                                     "fmri_edge_workspace", "fmri_launch_count", "fmri_version", "fmri_conv_pack_elems",
-                                    "fmri_pairwise_workspace", "fmri_image_rescale_workspace"):
+                                    "fmri_pairwise_workspace", "fmri_image_rescale_workspace",
+                                    "fmri_image_resample_workspace"):
             return f
 
         def timed(*a):
@@ -136,6 +144,7 @@ def load():
         c.fmri_edge_workspace.restype = C.c_size_t
         c.fmri_pairwise_workspace.restype = C.c_size_t
         c.fmri_image_rescale_workspace.restype = C.c_size_t
+        c.fmri_image_resample_workspace.restype = C.c_size_t
         c.fmri_conv_out_hw.restype = None
         c.fmri_launch_count.restype = C.c_longlong
         _lib = _Proxy(c)
@@ -577,6 +586,38 @@ def image_rescale(src_u8, table, flip, shift_yx, mean3, std3, dst, ws):
     _check(load().fmri_image_rescale(ptr(src_u8), C.c_size_t(src_u8.numel()), table, N, H, W, ptr(flip), ptr(shift_yx), m,
                                      s, ptr(dst), ptr(ws), _wsb(ws) if ws is not None else C.c_size_t(0), stream()))
 
+
+
+RESAMPLE_FILTERS = {"bilinear": 2, "bicubic": 3}   # fmri_resample_filter: PIL.Image.Resampling.BILINEAR / BICUBIC
+
+
+def image_window_table(entries):
+    """Host descriptor table (ctypes array of ImageWindow) from (offset, pitch, H, W, C, Hr, Wr, oy, ox) tuples."""
+    return (ImageWindow * len(entries))(*[ImageWindow(*[int(v) for v in e]) for e in entries])
+
+
+def image_resample_workspace(N):
+    """Bytes of device workspace fmri_image_resample needs for N images (0 for N < 1)."""
+    return int(load().fmri_image_resample_workspace(int(N)))
+
+
+def image_resample(src_u8, table, filter, flip, shift_yx, mean3, std3, dst, ws):
+    """src_u8: flat uint8 device buffer holding every source window; table: image_window_table(...) on the host (one entry
+    per output image); filter: 'bilinear' or 'bicubic'; dst: fp32 [N, 3, H, W]; ws: a device buffer of at least
+    image_resample_workspace(N) bytes."""
+    _require_cuda(src_u8, flip, shift_yx, dst, ws)
+    if src_u8.dtype != torch.uint8 or dst.dtype != torch.float32 or dst.dim() != 4 or dst.shape[1] != 3:
+        raise FmriError("image_resample expects a uint8 source buffer and a float32 [N, 3, H, W] output")
+    if filter not in RESAMPLE_FILTERS:
+        raise FmriError(f"image_resample: filter {filter!r} is not one of {sorted(RESAMPLE_FILTERS)}")
+    N, _, H, W = dst.shape
+    if len(table) != N:
+        raise FmriError(f"image_resample: {len(table)} descriptors for {N} output images")
+    m = (C.c_float * 3)(*[float(v) for v in mean3])
+    s = (C.c_float * 3)(*[float(v) for v in std3])
+    _check(load().fmri_image_resample(ptr(src_u8), C.c_size_t(src_u8.numel()), table, N, H, W, RESAMPLE_FILTERS[filter],
+                                      ptr(flip), ptr(shift_yx), m, s, ptr(dst), ptr(ws),
+                                      _wsb(ws) if ws is not None else C.c_size_t(0), stream()))
 
 # ------------------------------------------------------------------------------------------------ all-pairs similarity
 def pairwise_workspace(N, M, Cc, H, W, metric):
